@@ -9,7 +9,7 @@ e2e = the same rollout driven through agar_step_host (host action buffers in, ho
 inside the timed region).  Weak scaling: every rank runs its own 4096 envs, no collective on the step path
 (one NCCL all-reduce of episode statistics after the timed region).
 
-python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--envs E] [--frames F] [--tile W]
+python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--envs E] [--frames F] [--tile W] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -290,6 +290,39 @@ def device_rollouts(batch, decisions, steps, warmup, flush, dist=None, world=1):
     return total_ms
 
 
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000  # all files together, .npy headers included
+NPY_HEADER_BYTES = 128
+DUMP_GETTERS = ("reward", "done", "valid", "need_action", "mass", "fov", "ncells", "alive", "stats", "overflow")  # lay.GET_<NAME>
+
+
+def dump_outputs(batch, out_dir, limit=DUMP_LIMIT_BYTES):
+    """--dump-outputs: what the last timed rollout hands its caller, written as out_dir/<name>.npy so that two builds run with
+    the same arguments (same seed, env ids and decision indices, hence the same inputs) can be compared output for output.
+    obs is the [E, A, L] observation tensor the rollout returns; the others are the env's getters after it ([E, A], stats
+    [E, A, 4], overflow [E]); event_hash [E, 2] holds the high and low 32-bit halves of the per-env hash of every event.
+    Values are float32, or float64 where float32 would round them.  Above `limit` bytes a fixed, seeded sample of envs is
+    written and env_index.npy lists them."""
+    import numpy as np
+    import aigar_b200.layout as lay
+    out = {"obs": batch.obs.cpu().numpy()}
+    for name in DUMP_GETTERS:
+        out[name] = batch.get(getattr(lay, "GET_" + name.upper())).cpu().numpy()
+    out["overflow"] = out["overflow"].view(np.uint32).astype(np.float64)
+    h = batch.get(lay.GET_EVENT_HASH).cpu().numpy().view(np.uint64)
+    out["event_hash"] = np.stack([h >> np.uint64(32), h & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)
+    out = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in out.items()}
+    E = batch.n_envs
+    per_env = sum(v.nbytes for v in out.values()) / E
+    room = limit - NPY_HEADER_BYTES * (len(out) + 1)  # + env_index.npy
+    if per_env * E > limit - NPY_HEADER_BYTES * len(out):
+        idx = np.sort(np.random.default_rng(0).choice(E, int(room // (per_env + 8)), replace=False))
+        out = {k: v[idx] for k, v in out.items()}
+        out["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def scaling_sweep(cfg, local, rank, world, dist, flush):
     """BASELINE configs[4]: 65 536 / 262 144 / 1 048 576 TOTAL envs sharded evenly over the ranks (shard_envs: contiguous global
     env ids, Philox key = global id), observations handed to a torch DQN (MLP 123-100-100-25) through DLPack, arg-max -> the
@@ -487,7 +520,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm reports throughput only")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -535,6 +572,8 @@ def main():
     launches = batch.launch_count - launches0 - args.warmup
     clocks = sampler.stop()
     value = world * E * frames * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(batch, args.dump_outputs)
 
     # ---- e2e: host buffers through the C ABI's host-buffer step (actions H2D, obs/reward/done D2H every decision)
     e2e = None

@@ -1,4 +1,5 @@
-"""Reader for tests/golden/*.npz (both formats tools/gen_golden.py writes) and the event-coverage floor.
+"""Reader for tests/golden/*.npz (both formats tools/gen_golden.py writes), the event-coverage floor and the replay of
+tests/golden/live/ (tools/gen_golden_live.py).
 
 Format 1 (round 1): float32 actions, a flags table, every observation.  Format 2 ("long_*", round 2): uint8 actions
 (k/256), flag bit masks, strided observations and the tally of the reference's own event log."""
@@ -70,3 +71,50 @@ def tally_events(record, into):
 def assert_event_floor(tally, floor=MIN_EVENTS_EACH, names=RARE, what=""):
     short = {n: tally.get(n, 0) for n in names if tally.get(n, 0) < floor}
     assert not short, "%sevent types exercised fewer than %d times: %r (tally %r)" % (what, floor, short, tally)
+
+
+LIVE_DIR = os.path.join(GOLDEN_DIR, "live")
+
+
+def live(name):
+    """A recording of tools/gen_golden_live.py (tests/golden/live/<name>.npz)."""
+    return np.load(os.path.join(LIVE_DIR, name + ".npz"))
+
+
+def replay_live_rollout(name):
+    """Replay a recorded rollout through the C oracle (libm build) and compare bit for bit what the oracle-vs-reference
+    comparison compares: every frame's turn flags, float32 observations, event hash, event count and event list, and the
+    recorded env records (every field and event)."""
+    from oracle import oracle as orc
+    z = live(name)
+    cfg = lay.derive_config(event_cap=int(z["event_cap"]), **ast.literal_eval(str(z["kw"])))
+    env = orc.OracleEnv(cfg, seed=int(z["seed"]), env_id=int(z["env_id"]))
+    L = env.layout
+    rec_at = {int(f): i for i, f in enumerate(z["record_frames"])}
+    obs_at = {(int(t), int(a)): i for i, (t, a) in enumerate(z["obs_index"])}
+    records, obs, events = z["records"], z["obs"], z["events"]
+
+    def check_record(t):
+        d = lay.compare_records(lay.Record(L, records[rec_at[t]].copy()), env.record, what="%s frame %d " % (name, t),
+                                check_events=True)
+        assert not d, d
+
+    check_record(-1)
+    ev = 0
+    for t in range(z["actions"].shape[0]):
+        turn = env.frame(z["actions"][t])
+        for a in range(L.n_agents):
+            got = (turn[a]["observed"], turn[a]["valid"], turn[a]["done"], turn[a]["need_action"], turn[a]["obs32"] is not None)
+            assert [int(g) for g in got] == [(int(z["flags"][t, a]) >> b) & 1 for b in range(5)], (name, t, a)
+            if turn[a]["obs32"] is not None:
+                ref = obs[obs_at[(t, a)]]
+                assert np.array_equal(ref, turn[a]["obs32"]), (name, t, a, np.argwhere(ref != turn[a]["obs32"])[:4])
+        h = env.record.header
+        assert int(h["event_hash"][0]) == int(z["event_hash"][t]), "%s: event hash differs at frame %d" % (name, t)
+        assert int(h["n_events"][0]) == int(z["n_events"][t]), "%s: event count differs at frame %d" % (name, t)
+        n = min(int(z["n_events"][t]), L.event_cap)
+        assert env.record.event_list() == [tuple(int(v) for v in e) for e in events[ev:ev + n]], (name, t)
+        ev += n
+        if t in rec_at:
+            check_record(t)
+    assert ev == len(events)

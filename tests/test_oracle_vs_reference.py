@@ -1,126 +1,58 @@
-"""Live pin of the oracle: the unmodified reference Python (imported from /root/reference/src through
-oracle/ref_harness.py) and oracle/agar_oracle.c stepped side by side, records / events / observations compared
-BIT FOR BIT every frame.  Skipped where the reference checkout is absent (the GPU box): tests/golden/ carries
-the same evidence there."""
+"""Pin of the oracle against what the unmodified reference computes: oracle/agar_oracle.c replays the recordings of
+tests/golden/live/ (tools/gen_golden_live.py, on the inputs of tools/compare_oracle_ref.py) and must reproduce records, events
+and observations BIT FOR BIT every frame.  Where the reference's sources are at hand, tools/compare_oracle_ref.py and
+tools/fuzz_oracle_ref.py step the two side by side, and tools/gen_golden_live.py --source reference re-records these files."""
+import numpy as np
 import pytest
 
-from oracle import ref_harness as rh
+import aigar_b200.layout as lay
+import gen_golden_live as gl
+from golden_util import live, replay_live_rollout
 
-pytestmark = pytest.mark.skipif(not rh.reference_available(), reason="reference checkout not present")
 
-
-@pytest.mark.parametrize("which,frames,seed", [("1", 400, 11), ("1", 250, 12), ("3", 500, 13), ("r", 300, 14), ("4", 40, 15),
-                                               ("4nv", 30, 16)])
+@pytest.mark.parametrize("which,frames,seed", gl.ORACLE_CASES)
 def test_oracle_equals_reference(which, frames, seed):
-    import compare_oracle_ref as cmp
-    kws = {"1": dict(), "3": dict(num_nn=1, num_greedy=1, virus=True, split=True, eject=True),
-           "4": dict(num_nn=8, num_greedy=8, virus=True, split=True, eject=True),
-           "r": dict(num_nn=1, num_greedy=1, num_random=1, virus=True, split=True, eject=True),
-           "4nv": dict(num_nn=8, num_greedy=8, virus=False, split=True, eject=True)}
-    assert cmp.run(kws[which], frames, seed=seed, verbose=False)
+    assert live("oracle_%s_%d" % (which, seed))["actions"].shape[0] == frames
+    replay_live_rollout("oracle_%s_%d" % (which, seed))
 
 
 def test_reset_matches_reference():
-    import numpy as np
-    import aigar_b200.layout as lay
-    from oracle import oracle as orc
+    z, got = live("reset"), gl.record_reset("oracle")
     cfg = lay.derive_config(num_nn=1, num_greedy=1, virus=True, split=True, eject=True, event_cap=256)
-    ref, ora = rh.RefEnv(cfg, seed=5, env_id=1), orc.OracleEnv(cfg, seed=5, env_id=1)
-    rng = np.random.default_rng(0)
-    for t in range(120):
-        a = rng.random((1, 4)).astype(np.float32)
-        ref.step(a)
-        ora.frame(a)
-    ref.reset(), ref.reset_bots()
-    ora.reset(), ora.reset_bots()
-    d = lay.compare_records(ref.to_record(), ora.record, what="after reset ", check_events=False)
+    L = lay.layout_for_config(cfg)
+    d = lay.compare_records(lay.Record(L, z["after_reset"].copy()), lay.Record(L, got["after_reset"]), what="after reset ",
+                            check_events=False)
     assert not d, d
-    for t in range(60):
-        a = rng.random((1, 4)).astype(np.float32)
-        tr = ref.step(a)
-        ora.frame(a)
-    d = lay.compare_records(ref.to_record(tr), ora.record, what="after reset+60 ")
+    d = lay.compare_records(lay.Record(L, z["after_reset_60"].copy()), lay.Record(L, got["after_reset_60"]),
+                            what="after reset+60 ")
     assert not d, d
 
 
-VARIATIONS = [
-    dict(mass_as_reward=True),
-    dict(frame_skip=3, reward_scale=1.0, reward_term=0.5),
-    dict(grid=7),
-    dict(grid=13, num_nn=1, num_greedy=1),
-    dict(num_nn=2, num_random=1, split=True),                      # two agents, a random bot, split without eject
-    dict(num_nn=1, num_greedy=2, virus=True),                      # viruses without split: explosions only
-    dict(num_nn=1, num_greedy=1, virus=True, split=True, eject=True, death_term=-10.0, death_factor=0.5),
-    dict(num_nn=3, num_greedy=1, split=True, eject=True, obs_mode=1),
-    dict(overrides={"use_second_last_action": 1, "self_grid_slf": 1, "enemy_grid_slf": 1}, num_nn=1, num_greedy=1,
-         virus=True, split=True, eject=True),
-    dict(grid=42, overrides={"use_fovsize": 0, "use_totalmass": 0}),   # the handcraft-CNN grid (bot.py:103-111), §8f rank 3
-    dict(grid=42, num_nn=1, num_greedy=1, virus=True, split=True, eject=True),
-    dict(grid=63),
-    dict(grid=84, overrides={"use_fovsize": 0, "use_totalmass": 0}),   # CNN_INPUT_DIM_2
-    # ALL_PLAYER_GRID (networkParameters.py:88-91): one "biggest cell of any player" channel instead of self / enemy
-    dict(num_nn=1, num_greedy=1, virus=True, split=True, eject=True, overrides={"all_player_grid": 1, "self_grid": 0, "enemy_grid": 0, "self_grid_lf": 0, "enemy_grid_lf": 0}),
-    dict(overrides={"all_player_grid": 1}),
-    # NORMALIZE_GRID_BY_MAX_MASS in the run's parameters (bot.py:365,412,422,430): cell channels relative to the biggest cell in view
-    dict(num_nn=2, num_greedy=1, virus=True, split=True, eject=True, overrides={"normalize_grid_by_max_mass": 1}),
-    dict(num_nn=1, num_greedy=1, split=True, overrides={"normalize_grid_by_max_mass": 1, "all_player_grid": 1, "self_grid": 0, "enemy_grid": 0,
-                                                        "self_grid_lf": 0, "enemy_grid_lf": 0}),
-    # GRID_VIEW_ENABLED = False (networkParameters.py:119): Bot.getSimpleStateRepresentation, bot.py:511-548
-    dict(grid_view=False),
-    dict(num_nn=1, num_greedy=1, virus=True, split=True, eject=True, grid_view=False),
-    dict(num_nn=2, num_greedy=3, split=True, eject=True, grid_view=False, frame_skip=2),
-]
-
-
-@pytest.mark.parametrize("kw", VARIATIONS, ids=[str(i) for i in range(len(VARIATIONS))])
+@pytest.mark.parametrize("kw", gl.VARIATIONS, ids=[str(i) for i in range(len(gl.VARIATIONS))])
 def test_config_variations_equal_reference(kw):
     """Flags of networkParameters.py the default configs do not exercise: reward variants, frame-skip, grid sizes,
     channel subsets, bot mixes."""
-    import compare_oracle_ref as cmp
-    frames = 160 if kw.get("num_nn", 1) + kw.get("num_greedy", 0) + kw.get("num_random", 0) <= 2 else 90
-    if kw.get("grid", 11) >= 42:
-        frames = 48  # the reference's encoder is O(G^2) Python per observation
-    assert cmp.run(kw, frames, seed=31, verbose=False)
+    i = gl.VARIATIONS.index(kw)
+    z = live("variation_%d" % i)
+    assert str(z["kw"]) == repr(kw) and z["actions"].shape[0] == gl.variation_frames(kw)
+    replay_live_rollout("variation_%d" % i)
 
 
 def test_views_show_what_the_reference_objects_show():
-    """a.i.gar_b200/views.py (SURVEY §8f rank 4): the getters the reference's View reads, over an env record, against
-    the live reference objects after 150 frames of the 1-vs-greedy config."""
-    import numpy as np
-    import aigar_b200.layout as lay
-    from aigar_b200.views import FieldView
-    from oracle import oracle as orc
-    cfg = lay.derive_config(num_nn=1, num_greedy=1, virus=True, split=True, eject=True)
-    ref, ora = rh.RefEnv(cfg, seed=9, env_id=2), orc.OracleEnv(cfg, seed=9, env_id=2)
-    rng = np.random.default_rng(1)
-    for t in range(150):
-        a = rng.random((1, 4)).astype(np.float32)
-        ref.step(a)
-        ora.frame(a)
-    fv, f = FieldView(ora.record), ref.field
-    assert fv.getWidth() == f.getWidth() and fv.getHeight() == f.getHeight()
-    key = lambda c: (round(c.getX(), 9), round(c.getY(), 9), round(c.getMass(), 9))
-    for mine, theirs in ((fv.getPellets(), f.getPellets()), (fv.getViruses(), f.getViruses()), (fv.getBlobs(), f.getBlobs()),
-                         (fv.getPlayerCells(), f.getPlayerCells())):
-        assert sorted(map(key, mine)) == sorted(map(key, theirs))
-        assert sorted(round(c.getRadius(), 9) for c in mine) == sorted(round(c.getRadius(), 9) for c in theirs)
-    for pv, p in zip(fv.getPlayers(), f.getPlayers()):
-        assert pv.getIsAlive() == p.getIsAlive() and len(pv.getCells()) == len(p.getCells())
-        assert abs(pv.getTotalMass() - p.getTotalMass()) < 1e-9
-        for cv, c in zip(pv.getCells(), p.getCells()):
-            assert cv.getPos() == list(c.getPos()) and cv.getMass() == c.getMass() and cv.getRadius() == c.getRadius()
-    p0 = f.getPlayers()[0]
-    if p0.getIsAlive():
-        pos, size = p0.getFovPos(), p0.getFovSize()
-        assert sorted(map(key, fv.getPelletsInFov(pos, size))) == sorted(map(key, f.getPelletsInFov(pos, size)))
+    """a.i.gar_b200/views.py (SURVEY §8f rank 4): the getters the reference's View reads, over the oracle's env record after 150
+    frames of the 1-vs-greedy config, against what the reference objects returned."""
+    z, got = live("views"), gl.record_views("oracle")
+    assert sorted(z.files) == sorted(list(got) + ["source"])
+    for k, v in got.items():
+        assert np.array_equal(z[k], v), k
 
 
 def test_random_configs_equal_reference():
-    """tools/fuzz_oracle_ref.py: random flag / bot-mix / grid / frame-skip combinations, oracle vs the executed reference."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, os.path.join(root, "tools", "fuzz_oracle_ref.py"), "6", "23"], capture_output=True,
-                       text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+    """tools/fuzz_oracle_ref.py's random flag / bot-mix / grid / frame-skip combinations (6 cases, seed 23) replayed."""
+    from fuzz_oracle_ref import cases
+    cs = cases(gl.FUZZ_N, gl.FUZZ_SEED)
+    assert len(cs) >= 4
+    for case, kw, frames, seed in cs:
+        z = live("fuzz_%d" % case)
+        assert str(z["kw"]) == repr(kw) and int(z["seed"]) == seed and z["actions"].shape[0] == frames
+        replay_live_rollout("fuzz_%d" % case)

@@ -1,14 +1,9 @@
-"""GPU replay buffer (SURVEY §8f rank 1).  CPU: oracle/replay_oracle.py pinned against the reference's own
-ReplayBuffer / PrioritizedReplayBuffer (imported from /root/reference/src).  GPU: the CUDA buffer against the oracle."""
-import os
-import sys
-
+"""GPU replay buffer (SURVEY §8f rank 1).  CPU: oracle/replay_oracle.py pinned against a recording of the reference's own
+ReplayBuffer / PrioritizedReplayBuffer.  GPU: the CUDA buffer against the oracle."""
 import numpy as np
 import pytest
 
 from oracle.replay_oracle import ReplayOracle
-
-REF_SRC = os.environ.get("AGAR_REF_SRC", "/root/reference/src")
 
 
 def _transitions(n, L, rng):
@@ -16,49 +11,17 @@ def _transitions(n, L, rng):
              rng.random(L).astype(np.float32), bool(rng.random() < 0.1)) for _ in range(n)]
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF_SRC, "model", "replay_buffer.py")), reason="reference absent")
 @pytest.mark.parametrize("prioritized", [False, True])
-def test_oracle_equals_reference_replay_buffer(prioritized, monkeypatch):
-    if REF_SRC not in sys.path:
-        sys.path.insert(0, REF_SRC)
-    import importlib
-    rb = importlib.import_module("model.replay_buffer")
-    rng = np.random.default_rng(3)
-    feed = []
-
-    class _R(object):  # the injected stdlib random
-        @staticmethod
-        def randint(a, b):
-            return min(a + int(feed.pop(0) * (b - a + 1)), b)
-
-        @staticmethod
-        def random():
-            return feed.pop(0)
-
-    monkeypatch.setattr(rb, "random", _R)
-    size, L = 37, 6
-    ref = rb.PrioritizedReplayBuffer(size, 0.6, 0.4) if prioritized else rb.ReplayBuffer(size)
-    ora = ReplayOracle(size, prioritized, 0.6, 0.4)
-    for rnd in range(12):
-        for tr in _transitions(int(rng.integers(3, 15)), L, rng):
-            ref.add(*tr)
-            ora.add(*tr)
-        assert len(ref) == len(ora) and ref._next_idx == ora.next_idx
-        if len(ref) < 4:
-            continue
-        u = [float(x) for x in rng.random(8)]
-        feed[:] = list(u)
-        out_r = ref.sample(8)
-        out_o = ora.sample(u)
-        for a, b in zip(out_r[:5], out_o[:5]):
-            assert np.array_equal(np.asarray(a), np.asarray(b))
-        if prioritized:
-            assert list(out_r[6]) == list(out_o[6]) and np.array_equal(out_r[5], out_o[5])  # idxes, weights bit-exact
-            pr = np.abs(rng.normal(size=8)) + 1e-4
-            ref.update_priorities(out_r[6], pr)
-            ora.update_priorities(out_o[6], pr)
-            assert ref._max_priority == ora.max_priority
-            assert ref._it_sum._value == ora.sum and ref._it_min._value == ora.min
+def test_oracle_equals_reference_replay_buffer(prioritized):
+    """12 rounds of adds, samples from 8 injected uniforms and priority updates: length, next index, every sampled column,
+    index and weight, the max priority and both segment trees bit for bit against the recording of the reference's ReplayBuffer /
+    PrioritizedReplayBuffer on the same sequence (tests/golden/live/replay_*.npz, tools/gen_golden_live.py)."""
+    import gen_golden_live as gl
+    from golden_util import live
+    z = live("replay_prioritized" if prioritized else "replay_uniform")
+    got = gl.record_replay("oracle", prioritized)
+    assert np.array_equal(z["states"], got["states"], equal_nan=True)
+    assert np.array_equal(z["samples"], got["samples"])
 
 
 @pytest.mark.gpu

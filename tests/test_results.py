@@ -2,7 +2,6 @@
 import os
 
 import numpy as np
-import pytest
 
 from aigar_b200 import results as res
 
@@ -35,18 +34,10 @@ def test_file_formats(tmp_path):
 
 
 def test_against_the_reference_functions(tmp_path):
-    """exportResults / the final_results writer of the reference itself, executed on the same numbers (the functions are pure
-    Python; aigar.py imports Keras at module level, so they are extracted from its source)."""
-    src_path = "/root/reference/src/aigar.py"
-    if not os.path.isfile(src_path):
-        pytest.skip("reference checkout not present")
-    src = open(src_path).read()
-    start = src.index("def exportResults(results, path, name):")
-    end = src.index("# Plot test result and export plot to file with given name")
-    ns = {}
-    exec(src[start:end], ns)
-    vals = [123.456, 99.0, 1e-3, 250.12345678901234]
-    a, b = str(tmp_path) + os.sep + "a_", str(tmp_path) + os.sep + "b_"
-    ns["exportResults"](vals, a, "m")
-    res.export_results(vals, b, "m")
-    assert open(a + "m.txt").read() == open(b + "m.txt").read()
+    """The file the reference's own exportResults writes for four fixed values (recorded in tests/golden/live/export_results.npz
+    by tools/gen_golden_live.py; the function is pure Python, extracted from aigar.py, which imports Keras at module level)."""
+    from golden_util import live
+    z = live("export_results")
+    b = str(tmp_path) + os.sep + "b_"
+    res.export_results([float(v) for v in z["values"]], b, "m")
+    assert open(b + "m.txt").read() == str(z["text"])
