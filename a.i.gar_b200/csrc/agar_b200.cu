@@ -220,14 +220,47 @@ struct SimplePlan {
     int frame_sync; /* CTA barrier at every frame: the warps of a CTA fetch the same instructions together */
     int strideB; /* bytes between the staged [pellets .. end of record] regions of consecutive envs */
     int grid_off; /* byte offset of the env's G x G observation accumulator inside its region; 0: accumulate in the caller's row */
+    int obs_warps; /* observer warps at the end of the CTA (0: every warp steps envs and encodes its own observations) */
+    int snap_off; /* byte offset of the two snapshot buffers (observer launches): after the envs' regions */
+    int snap_stride; /* bytes per env in one snapshot buffer: SimpleSnap + the pellet pool */
 };
+
+/* Observer warps (launches that hand decision observations off, see plan_observers): at each decision the physics warps
+ * copy the env's pellet pool and the four values s_encode reads into a snapshot slot and go straight on to the frames;
+ * the observer warps bin the snapshot into the env's row meanwhile.  Nothing the frames read depends on the grid, and the
+ * pool changes only in s_field_update, so the row is the one the inline encoder would have written at that moment.
+ * Two snapshot buffers (decision d uses buffer d & 1), each with a FULL / EMPTY named-barrier pair:
+ *   physics:  [d >= 2: bar.sync EMPTY[b]]  fill b  bar.arrive FULL[b]
+ *   observer: bar.sync FULL[b]  encode b  [d + 2 < n_dec: bar.arrive EMPTY[b]]
+ * so every barrier instance gets exactly (physics + observer threads) arrivals.  ID 0 stays __syncthreads. */
+enum { SB_PHYS = 1, SB_FULL = 2, SB_EMPTY = 4 }; /* named barrier IDs: SB_FULL + b, SB_EMPTY + b for buffer b */
+struct SimpleSnap {
+    double fov_x, fov_y, fov_size, mass;
+    int32_t out; /* a row is stored (the env observes at this decision and is not a spare slot) */
+    int32_t pad;
+};
+/* CTA size bound of k_simple<W, true>: the physics warps plus the observers.  W = 8: 11 warps, one CTA per SM
+ * (ptxas budgets the bound rounded up to 12 warps: 168 registers; CUDA 12.9 allocates 167, no spills — 176 without the
+ * bound).  W = 4 needs 188-192 registers and spills under that budget, so it keeps 8 warps (4 + 4, 255 registers). */
+__host__ __device__ constexpr int simple_max_threads(int W) { return W == 8 ? 352 : 256; }
+constexpr int SIMPLE_OBS_MIN_FRAMES = 4; /* frames per handed-off observation below which the inline encoder stays (measured) */
+constexpr int SIMPLE_OBS_LANES = 4;      /* lanes per env of the observer warps */
+constexpr int SIMPLE_OBS_WARPS = 4;      /* observer warps per CTA */
+
+/* immediate IDs: ptxas then reserves the barriers used, not all 16 */
+template <int ID>
+DEV void named_bar_sync(int n) { asm volatile("bar.sync %0, %1;" ::"n"(ID), "r"(n) : "memory"); }
+template <int ID>
+DEV void named_bar_arrive(int n) { asm volatile("bar.arrive %0, %1;" ::"n"(ID), "r"(n) : "memory"); }
+
 /* one lane per env is throughput-bound: cap registers at 128 for 8 CTAs / SM (measured +10..50 % at >= 64k envs);
  * wider tiles are latency-bound at small env counts and prefer the uncapped allocation (measured) */
-template <int W>
-__global__ void __launch_bounds__(256, W == 1 ? 2 : 1)
+template <int W, bool OBSW> /* OBSW: the observer-warp launch (plan_observers); false: the inline encoder, CTA barrier per frame */
+__global__ void __launch_bounds__(OBSW ? simple_max_threads(W) : 256, W == 1 ? 2 : 1)
 k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __restrict__ state, const float* __restrict__ actions,
          float* __restrict__ obs, int n_frames, int n_dec, int flags, uint32_t dec_base) {
-    const int per = blockDim.x / W; /* envs per CTA */
+    const int phys_threads = blockDim.x - 32 * SP.obs_warps; /* the one place the barrier counts come from */
+    const int per = phys_threads / W; /* envs per CTA */
     const int env0 = blockIdx.x * per;
     const int n_here = min(per, P.n_envs - env0);
     const int rec_words = (int)(P.L.record_bytes / 4), pel_word = (int)(P.L.off_pellets / 4);
@@ -242,58 +275,110 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
         }
     }
     __syncthreads();
-    const int slot = threadIdx.x / W, sub = threadIdx.x % W;
-    const bool valid = slot < n_here;
-    const int env = env0 + (valid ? slot : n_here - 1);
-    const uint32_t env_id = (uint32_t)(P.first_env + (uint64_t)env);
-    uint8_t* rec = state + (size_t)env * P.L.record_bytes;
-    uint8_t* b = g_smem + (size_t)slot * SP.strideB;
-    SPtr q;
-    q.h = (AgarEnvHeader*)(rec + P.L.off_header);
-    q.p = (AgarPlayer*)(rec + P.L.off_players);
-    q.c = (AgarCell*)(rec + P.L.off_cells);
-    q.pel = (uint32_t*)b;
-    q.ev = (AgarEvent*)(b + (P.L.off_events - P.L.off_pellets));
-    q.grid = SP.grid_off ? (uint32_t*)(b + SP.grid_off) : nullptr;
-    SReg r;
-    s_load(r, q);
-    float* row = (obs != nullptr && valid) ? obs + (size_t)env * P.L.state_len : nullptr;
-    for (int d = 0; d < n_dec; ++d) {
-        if (flags & KF_OBS_BEFORE) {
+    auto snap = [&](int buf, int e) { return g_smem + SP.snap_off + (size_t)(buf * per + e) * SP.snap_stride; };
+    if (OBSW && (int)threadIdx.x >= phys_threads) { /* observer warps */
+        constexpr int WO = SIMPLE_OBS_LANES;
+        const int ot = ((int)threadIdx.x - phys_threads) / WO, osub = threadIdx.x % WO, n_ot = 32 * SP.obs_warps / WO;
+        for (int d = 0; d < n_dec; ++d) {
+            const int buf = d & 1;
+            if (buf) named_bar_sync<SB_FULL + 1>(blockDim.x);
+            else named_bar_sync<SB_FULL>(blockDim.x);
+            /* static env -> observer tile map: each env's rows are stored by one tile, in decision order, and its G x G
+             * accumulator has one user */
+            for (int base = 0; base < per; base += n_ot) { /* warp-uniform trip count */
+                const int e = min(base + ot, per - 1);
+                const SimpleSnap* sn = (const SimpleSnap*)snap(buf, e);
+                SReg r;
+                r.fov_x = sn->fov_x, r.fov_y = sn->fov_y, r.fov_size = sn->fov_size, r.mass = sn->mass;
+                SPtr q;
+                q.pel = (uint32_t*)(sn + 1);
+                q.grid = (uint32_t*)(g_smem + (size_t)e * SP.strideB + SP.grid_off);
+                const bool out = base + ot < per && sn->out != 0;
+                s_encode<WO>(r, q, P, out, out ? obs + (size_t)(env0 + e) * P.L.state_len : nullptr, osub);
+            }
+            if (d + 2 < n_dec) {
+                if (buf) named_bar_arrive<SB_EMPTY + 1>(blockDim.x);
+                else named_bar_arrive<SB_EMPTY>(blockDim.x);
+            }
+        }
+        if (flags & KF_OBS_AFTER) __syncthreads(); /* drained: the physics warps' trailing observation may use the grids */
+    } else { /* physics warps */
+        const int slot = threadIdx.x / W, sub = threadIdx.x % W;
+        const bool valid = slot < n_here;
+        const int env = env0 + (valid ? slot : n_here - 1);
+        const uint32_t env_id = (uint32_t)(P.first_env + (uint64_t)env);
+        uint8_t* rec = state + (size_t)env * P.L.record_bytes;
+        uint8_t* b = g_smem + (size_t)slot * SP.strideB;
+        SPtr q;
+        q.h = (AgarEnvHeader*)(rec + P.L.off_header);
+        q.p = (AgarPlayer*)(rec + P.L.off_players);
+        q.c = (AgarCell*)(rec + P.L.off_cells);
+        q.pel = (uint32_t*)b;
+        q.ev = (AgarEvent*)(b + (P.L.off_events - P.L.off_pellets));
+        q.grid = SP.grid_off ? (uint32_t*)(b + SP.grid_off) : nullptr;
+        SReg r;
+        s_load(r, q);
+        float* row = (obs != nullptr && valid) ? obs + (size_t)env * P.L.state_len : nullptr;
+        auto frame_bar = [&]() { /* the physics warps only: observers keep their own pace */
+            if (OBSW) named_bar_sync<SB_PHYS>(phys_threads);
+            else __syncthreads();
+        };
+        for (int d = 0; d < n_dec; ++d) {
+            if (OBSW && SP.obs_warps) { /* hand the observation off (the host sets obs_warps only with KF_OBS_BEFORE and a row buffer) */
+                const int d_o = s_turn_begin(r, P);
+                if (d_o) s_observe_state(r, P);
+                const int buf = d & 1;
+                if (d >= 2) {
+                    if (buf) named_bar_sync<SB_EMPTY + 1>(blockDim.x);
+                    else named_bar_sync<SB_EMPTY>(blockDim.x);
+                }
+                uint8_t* sn = snap(buf, slot);
+                uint32_t* pool = (uint32_t*)(sn + sizeof(SimpleSnap));
+                for (int i = sub; i < P.L.pellet_cap; i += W) pool[i] = q.pel[i];
+                if (sub == 0) {
+                    SimpleSnap* h = (SimpleSnap*)sn;
+                    h->fov_x = r.fov_x, h->fov_y = r.fov_y, h->fov_size = r.fov_size, h->mass = r.mass;
+                    h->out = d_o != 0 && row != nullptr;
+                }
+                if (buf) named_bar_arrive<SB_FULL + 1>(blockDim.x);
+                else named_bar_arrive<SB_FULL>(blockDim.x);
+            } else if (flags & KF_OBS_BEFORE) {
+                int d_o = s_turn_begin(r, P);
+                s_observe<W>(r, q, P, d_o != 0, row, sub);
+            }
+            for (int f = 0; f < n_frames; ++f) {
+                if (SP.frame_sync == 1 || SP.frame_sync == 4) frame_bar();
+                if (SP.frame_sync == 2) __syncwarp();
+                r.n_events = 0;
+                int d_o = s_turn_begin(r, P);
+                s_observe<W>(r, q, P, d_o != 0, nullptr, sub);
+                float act[4] = {0.f, 0.f, 0.f, 0.f};
+                if (r.need_action) {
+                    if (flags & KF_RANDOM_ACTIONS) {
+                        uint32_t w[4];
+                        philox(dec_base + (uint32_t)d, 7u, env_id, 0u, (uint32_t)P.seed, (uint32_t)(P.seed >> 32), w);
+                        for (int i = 0; i < 4; ++i) act[i] = (float)(w[i] >> 8) * (1.0f / 16777216.0f);
+                    } else {
+                        const float* ap = actions + (size_t)env * 4;
+                        for (int i = 0; i < 4; ++i) act[i] = ap[i];
+                    }
+                }
+                double speed_pow;
+                s_turn_end<W>(r, P, act, sub, speed_pow);
+                if (SP.frame_sync == 4) frame_bar();
+                s_field_update<W>(r, q, P, env_id, sub, speed_pow);
+            }
+        }
+        if (flags & KF_OBS_AFTER) {
+            if (OBSW) __syncthreads(); /* the observers have stored every handed-off row and left the grid accumulators */
             int d_o = s_turn_begin(r, P);
             s_observe<W>(r, q, P, d_o != 0, row, sub);
         }
-        for (int f = 0; f < n_frames; ++f) {
-            if (SP.frame_sync == 1 || SP.frame_sync == 4) __syncthreads();
-            if (SP.frame_sync == 2) __syncwarp();
-            r.n_events = 0;
-            int d_o = s_turn_begin(r, P);
-            s_observe<W>(r, q, P, d_o != 0, nullptr, sub);
-            float act[4] = {0.f, 0.f, 0.f, 0.f};
-            if (r.need_action) {
-                if (flags & KF_RANDOM_ACTIONS) {
-                    uint32_t w[4];
-                    philox(dec_base + (uint32_t)d, 7u, env_id, 0u, (uint32_t)P.seed, (uint32_t)(P.seed >> 32), w);
-                    for (int i = 0; i < 4; ++i) act[i] = (float)(w[i] >> 8) * (1.0f / 16777216.0f);
-                } else {
-                    const float* ap = actions + (size_t)env * 4;
-                    for (int i = 0; i < 4; ++i) act[i] = ap[i];
-                }
-            }
-            double speed_pow;
-            s_turn_end<W>(r, P, act, sub, speed_pow);
-            if (SP.frame_sync == 4) __syncthreads();
-            s_field_update<W>(r, q, P, env_id, sub, speed_pow);
+        if (valid && sub == 0) {
+            s_store(r, q);
+            if (P.turn_reward) P.turn_reward[env] = (float)r.last_reward; /* Bot.getLastReward / done of this turn, fused */
+            if (P.turn_done) P.turn_done[env] = (uint8_t)r.exp_done;
         }
-    }
-    if (flags & KF_OBS_AFTER) {
-        int d_o = s_turn_begin(r, P);
-        s_observe<W>(r, q, P, d_o != 0, row, sub);
-    }
-    if (valid && sub == 0) {
-        s_store(r, q);
-        if (P.turn_reward) P.turn_reward[env] = (float)r.last_reward; /* Bot.getLastReward / done of this turn, fused */
-        if (P.turn_done) P.turn_done[env] = (uint8_t)r.exp_done;
     }
     __syncthreads();
     for (int i = threadIdx.x; i < n_here * tail_words; i += blockDim.x) { /* stage the pools out */
@@ -428,7 +513,11 @@ struct AgarEnv {
     SimplePlan sp;
     int simple_W, simple_threads;
     size_t simple_smem;
+    SimplePlan sp_obs; /* observer launches of k_simple (plan_observers); obs_threads == 0: none */
+    int obs_threads;
+    size_t obs_smem;
     int64_t launches;
+    int64_t observer_launches; /* launches of k_simple<W, true> */
     char err[256];
     /* step_host staging */
     float *d_actions, *d_obs, *d_reward;
@@ -555,24 +644,37 @@ static int launch_main(AgarEnv* e, const float* actions, float* obs, int n_frame
     CU(cudaSetDevice(e->device));
     cudaError_t err;
     if (e->simple_W) {
-        int blocks = (e->n_envs * e->simple_W + e->simple_threads - 1) / e->simple_threads;
-#define LAUNCH_SIMPLE(WW)                                                                                                     \
+        /* observer warps encode the observations a launch hands off before its frames (KF_OBS_BEFORE), when enough frames
+         * follow each one to hide the encoder; a trailing observation (KF_OBS_AFTER) stays with the physics warps */
+        const bool handoff = e->obs_threads && (flags & KF_OBS_BEFORE) && obs != nullptr && n_frames >= SIMPLE_OBS_MIN_FRAMES;
+        const SimplePlan& sp = handoff ? e->sp_obs : e->sp;
+        const int threads = handoff ? e->obs_threads : e->simple_threads;
+        const size_t smem = handoff ? e->obs_smem : e->simple_smem;
+        const int per = (threads - 32 * sp.obs_warps) / e->simple_W;
+        if (threads % 32 || threads > (handoff ? simple_max_threads(e->simple_W) : 256) || per < 1 || per * e->simple_W % 32 ||
+            (sp.obs_warps && (!sp.grid_off || 32 * sp.obs_warps % SIMPLE_OBS_LANES)))
+            return fail(e, AGAR_E_INVALID, "inconsistent k_simple launch shape%s", "");
+        int blocks = (e->n_envs + per - 1) / per;
+#define LAUNCH_SIMPLE(WW, OB)                                                                                                 \
     do {                                                                                                                      \
-        static unsigned char done_##WW[64];                                                                                   \
-        err = ensure_max_smem(k_simple<WW>, e->device, done_##WW);                                                            \
+        static unsigned char done_##WW##OB[64];                                                                               \
+        err = ensure_max_smem(k_simple<WW, OB>, e->device, done_##WW##OB);                                                    \
         if (err == cudaSuccess) {                                                                                             \
-            k_simple<WW><<<blocks, e->simple_threads, e->simple_smem, (cudaStream_t)stream>>>(e->P, e->sp, e->state, actions, obs, \
-                                                                                              n_frames, n_dec, flags, dec_base);  \
+            k_simple<WW, OB><<<blocks, threads, smem, (cudaStream_t)stream>>>(e->P, sp, e->state, actions, obs, n_frames,     \
+                                                                              n_dec, flags, dec_base);                        \
             err = cudaGetLastError();                                                                                         \
         }                                                                                                                     \
     } while (0)
-        if (e->simple_W == 1) LAUNCH_SIMPLE(1);
-        else if (e->simple_W == 2) LAUNCH_SIMPLE(2);
-        else if (e->simple_W == 4) LAUNCH_SIMPLE(4);
-        else if (e->simple_W == 8) LAUNCH_SIMPLE(8);
-        else if (e->simple_W == 16) LAUNCH_SIMPLE(16);
-        else LAUNCH_SIMPLE(32);
+        if (handoff && e->simple_W == 4) LAUNCH_SIMPLE(4, true);
+        else if (handoff) LAUNCH_SIMPLE(8, true);
+        else if (e->simple_W == 1) LAUNCH_SIMPLE(1, false);
+        else if (e->simple_W == 2) LAUNCH_SIMPLE(2, false);
+        else if (e->simple_W == 4) LAUNCH_SIMPLE(4, false);
+        else if (e->simple_W == 8) LAUNCH_SIMPLE(8, false);
+        else if (e->simple_W == 16) LAUNCH_SIMPLE(16, false);
+        else LAUNCH_SIMPLE(32, false);
 #undef LAUNCH_SIMPLE
+        if (handoff && err == cudaSuccess) e->observer_launches += 1;
     } else
         err = DISPATCH(launch_main_t, e, actions, obs, n_frames, n_dec, flags, dec_base, (cudaStream_t)stream);
     if (err != cudaSuccess) return fail(e, AGAR_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
@@ -590,6 +692,62 @@ static int launch_init(AgarEnv* e, const uint8_t* mask, int mode, void* stream) 
     return AGAR_OK;
 }
 
+/* resident CTAs per SM of k_simple<W, OBSW> at this CTA size and shared memory (0: cannot run, or the query failed) */
+template <int W, bool OBSW>
+static int simple_ctas_per_sm(int device, int threads, size_t smem) {
+    static unsigned char done[64];
+    int n = 0;
+    if (ensure_max_smem(k_simple<W, OBSW>, device, done) != cudaSuccess ||
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_simple<W, OBSW>, threads, smem) != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
+    return n;
+}
+
+/* Launch shape of k_simple with observer warps: one CTA per SM, ceil(envs / SMs) envs rounded up to whole physics warps
+ * (4096 envs at W = 8: 7 warps, 28 envs, 147 CTAs), plus SIMPLE_OBS_WARPS observers, within the registers of one SM
+ * (simple_max_threads).  Latency-bound tile widths (4 and 8 lanes) only: at 1 and 2 lanes the kernel is throughput-bound
+ * and the encoder's work costs the same wherever it runs.  Wave-aware: past the physics-warp cap one CTA holds at most 28
+ * (W = 8) or 32 (W = 4) envs and an SM holds one such CTA, while the inline shape fits two CTAs of 16 / 32 envs per SM —
+ * the observers are used only where their launch needs no more waves than the inline one (4096 envs at W = 8: one wave
+ * each; 4608: two against one). */
+static void plan_observers(AgarEnv* e) {
+    e->obs_threads = 0;
+    e->sp_obs = e->sp;
+    const int W = e->simple_W;
+    if ((W != 4 && W != 8) || !e->sp.grid_off || e->L.pellet_cap > 64 * SIMPLE_OBS_LANES) return; /* SMask<SIMPLE_OBS_LANES> */
+    if (cudaSetDevice(e->device) != cudaSuccess) {
+        cudaGetLastError();
+        return;
+    }
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->device);
+    const int per_warp = 32 / W;
+    const int K = SIMPLE_OBS_WARPS;
+    int warps = ((e->n_envs + sms - 1) / sms + per_warp - 1) / per_warp;
+    if (warps > simple_max_threads(W) / 32 - K) warps = simple_max_threads(W) / 32 - K;
+    const int per = warps * per_warp;
+    const size_t env_bytes = ((size_t)per * e->sp.strideB + 15) / 16 * 16;
+    const int snap_stride = (int)((sizeof(SimpleSnap) + (size_t)e->L.pellet_cap * 4 + 15) / 16 * 16);
+    const size_t smem = env_bytes + 2 * (size_t)per * snap_stride;
+    if (smem > 200 * 1024) return;
+    const int threads = (warps + K) * 32;
+    const int occ = W == 8 ? simple_ctas_per_sm<8, true>(e->device, threads, smem) : simple_ctas_per_sm<4, true>(e->device, threads, smem);
+    const int occ_in = W == 8 ? simple_ctas_per_sm<8, false>(e->device, e->simple_threads, e->simple_smem)
+                              : simple_ctas_per_sm<4, false>(e->device, e->simple_threads, e->simple_smem);
+    if (occ < 1 || occ_in < 1) return;
+    const long long per_in = e->simple_threads / W;
+    const long long waves = ((e->n_envs + per - 1) / per + (long long)sms * occ - 1) / ((long long)sms * occ);
+    const long long waves_in = ((e->n_envs + per_in - 1) / per_in + (long long)sms * occ_in - 1) / ((long long)sms * occ_in);
+    if (waves > waves_in) return;
+    e->sp_obs.obs_warps = K;
+    e->sp_obs.snap_off = (int)env_bytes;
+    e->sp_obs.snap_stride = snap_stride;
+    e->obs_threads = threads;
+    e->obs_smem = smem;
+}
+
 /* Lanes per env.  Single-cell pellet-collection configs: 1, 2, 4, 8 select the register-resident kernel
  * (agar_simple.cuh), 16 / 32 the general kernel; every other config: 4, 8, 16, 32 (general kernel). */
 extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
@@ -600,6 +758,7 @@ extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
         int tail_words = (int)((e->L.record_bytes - e->L.off_pellets) / 4);
         e->sp.strideB = (tail_words | 1) * 4;
         e->sp.grid_off = 0;
+        e->sp.obs_warps = e->sp.snap_off = e->sp.snap_stride = 0;
         /* the observation's G x G sums are accumulated in shared memory and leave once, as consecutive floats of the row
          * (measured: 4096 envs W=8 +1.2 %, 65536 envs W=2 +8 %).  Not at one lane per env: 484 more bytes per env halve the
          * resident envs per SM there (1M envs: 3.28e9 -> 1.52e9), and a lone lane's stores are strided either way. */
@@ -626,6 +785,7 @@ extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
         e->simple_threads = threads;
         e->simple_smem = per_env * (threads / W);
         e->W = W;
+        plan_observers(e);
         return AGAR_OK;
     }
     bool ok = W == 32 || (e->full && (W == 4 || W == 8 || W == 16));
@@ -763,6 +923,7 @@ extern "C" int agar_get_layout(const AgarEnv* e, AgarLayout* out) {
 }
 extern "C" int agar_num_envs(const AgarEnv* e) { return e ? e->n_envs : AGAR_E_INVALID; }
 extern "C" int64_t agar_launch_count(const AgarEnv* e) { return e ? e->launches : 0; }
+extern "C" int64_t agar_observer_launch_count(const AgarEnv* e) { return e ? e->observer_launches : 0; }
 extern "C" void* agar_state_ptr(const AgarEnv* e) { return e ? e->state : nullptr; }
 
 extern "C" int agar_reset(AgarEnv* e, const uint8_t* env_mask_dev, void* stream) {

@@ -212,18 +212,19 @@ struct SMask<2> {
 DEV int s_ffs(uint32_t m) { return __ffs((int)m); }
 DEV int s_ffs(unsigned long long m) { return __ffsll((long long)m); }
 
-/* bot.py:326-497 for the pellet channel.  Warp-uniform: every lane calls it; `mine` = this tile observes now.
- * row: this env's observation row in the caller's buffer (nullptr: a decision inside a multi-frame step, nobody
- * reads the grid — only the fov caches advance, as in the reference). */
+/* The state change of an observation (player.py:156-167, bot.py:326): the fov caches advance; s_encode reads them. */
+DEV void s_observe_state(SReg& r, const DevParams& P) {
+    s_update_fov(r, P);
+    r.fov_size_feat = P.cfg.use_fovsize ? r.fov_size : r.fov_size_feat;
+}
+
+/* bot.py:326-497 for the pellet channel: bins q.pel into row.  Reads r.fov_x, r.fov_y, r.fov_size and r.mass only, and
+ * writes nothing but q.grid and row — so it can run on a snapshot of the pool and of those four values (observer warps,
+ * k_simple).  Warp-uniform: every lane calls it; out = this tile stores a row. */
 template <int W>
-DEV void s_observe(SReg& r, const SPtr& q, const DevParams& P, bool mine, float* row, int sub) {
+DEV void s_encode(const SReg& r, const SPtr& q, const DevParams& P, bool out, float* row, int sub) {
     const int G = P.L.grid_squares, GG = G * G, SL = P.L.state_len;
     const double S = (double)P.S;
-    if (mine) {
-        s_update_fov(r, P);
-        r.fov_size_feat = P.cfg.use_fovsize ? r.fov_size : r.fov_size_feat;
-    }
-    const bool out = mine && row != nullptr;
     if (!s_any<W>(out)) return;
     const bool staged = q.grid != nullptr;
     if (out) { /* clear the row; extras: [fov size], [total mass] (bot.py:302-323) */
@@ -332,6 +333,15 @@ DEV void s_observe(SReg& r, const SPtr& q, const DevParams& P, bool mine, float*
         if (out)
             for (int i = sub; i < GG; i += W) row[i] = (float)q.grid[i];
     }
+}
+
+/* Warp-uniform: every lane calls it; `mine` = this tile observes now.  row: this env's observation row in the caller's
+ * buffer (nullptr: a decision inside a multi-frame step, nobody reads the grid — only the fov caches advance, as in the
+ * reference). */
+template <int W>
+DEV void s_observe(SReg& r, const SPtr& q, const DevParams& P, bool mine, float* row, int sub) {
+    if (mine) s_observe_state(r, P);
+    s_encode<W>(r, q, P, mine && row != nullptr, row, sub);
 }
 
 /* one frame of Field.update for a single-cell env (field.py:85-92); warp-uniform, state replicated per tile */

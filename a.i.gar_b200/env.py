@@ -133,6 +133,13 @@ class AgarBatch(object):
     def launch_count(self):
         return int(self.lib.agar_launch_count(self.h))
 
+    @property
+    def observer_launch_count(self):
+        """Launches whose decision observations observer warps encoded (not in EXPORTS: older builds load for A/B runs)."""
+        fn = self.lib.agar_observer_launch_count
+        fn.argtypes, fn.restype = [ctypes.c_void_p], ctypes.c_int64
+        return int(fn(self.h))
+
     def _ptr(self, t):
         return ctypes.c_void_p(t.data_ptr()) if t is not None else ctypes.c_void_p()
 

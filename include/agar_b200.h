@@ -301,6 +301,8 @@ int agar_debug_load(AgarEnv* env, int env_index, const void* record_host, size_t
 
 /* number of kernels this handle has launched so far (bench.py's gpu_launches) */
 int64_t agar_launch_count(const AgarEnv* env);
+/* how many of them handed their observations to observer warps (single-cell rollouts at 4 / 8 lanes per env) */
+int64_t agar_observer_launch_count(const AgarEnv* env);
 
 /* ---- host-buffer convenience path (the e2e call: host arrays in, host arrays out) ----
  * actions_host float[E][A][4] -> H2D, n_frames frames, observe, D2H of obs/reward/done.
