@@ -550,6 +550,7 @@ extern "C" int agar_layout_for_config(const AgarConfig* cfg, AgarLayout* out) {
 
 static bool config_is_simple(const AgarConfig& c, const AgarLayout& L) {
     return c.n_players == 1 && c.bot_type[0] == AGAR_BOT_NN && !c.virus_enabled && !c.enable_split && !c.enable_eject &&
+           c.pellet_grid && /* s_encode always writes the G x G pellet grid in front of the extras */
            L.cell_cap == 1 && !c.self_grid && !c.wall_grid && !c.enemy_grid && !c.virus_grid && !c.self_grid_lf &&
            !c.self_grid_slf && !c.enemy_grid_lf && !c.enemy_grid_slf && !c.use_last_action && !c.use_second_last_action &&
            !c.use_last_fovsize && L.n_hist == 0 && !c.all_player_grid && !c.simple_state && /* the 12-value representation lives in the general kernel */
@@ -748,8 +749,9 @@ static void plan_observers(AgarEnv* e) {
     e->obs_smem = smem;
 }
 
-/* Lanes per env.  Single-cell pellet-collection configs: 1, 2, 4, 8 select the register-resident kernel
- * (agar_simple.cuh), 16 / 32 the general kernel; every other config: 4, 8, 16, 32 (general kernel). */
+/* Lanes per env.  Single-cell pellet-collection configs (config_is_simple) with G <= 16: 1, 2, 4, 8, 16, 32 select the
+ * register-resident kernel (agar_simple.cuh, k_simple<W>); they run the general kernel (k_main<32, false>, 32 lanes only)
+ * with G > 16 or under AGAR_GENERAL_KERNEL=1.  Every other config: 4, 8, 16, 32 (general kernel). */
 extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
     if (!e) return AGAR_E_INVALID;
     /* the register-resident kernel bins a pellet into at most two squares per axis: 2 * radius < fov / G needs G <= 16 */

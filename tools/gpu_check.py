@@ -21,8 +21,10 @@ def records(batch):
     return [lay.Record(batch.layout, st[i].copy()) for i in range(batch.n_envs)]
 
 
-def check(which="1", n_envs=32, frames=200, seed=3, first_env=5, tile_width=None, every=1, event_cap=64, verbose=True, tally=None):
-    """tally: dict that receives the event-type counts of the ORACLE's per-frame event logs (all envs, all frames)."""
+def check(which="1", n_envs=32, frames=200, seed=3, first_env=5, tile_width=None, every=1, event_cap=64, verbose=True, tally=None,
+          setup=None):
+    """tally: dict that receives the event-type counts of the ORACLE's per-frame event logs (all envs, all frames).
+    setup: setup(batch, oracles) runs once before the first comparison, e.g. to load the same records into both."""
     cfg = lay.derive_config(event_cap=event_cap, **(which if isinstance(which, dict) else KWS[which]))
     batch = AgarBatch(cfg, n_envs, seed=seed, first_env_id=first_env, tile_width=tile_width)
     L = batch.layout
@@ -30,6 +32,8 @@ def check(which="1", n_envs=32, frames=200, seed=3, first_env=5, tile_width=None
     A = max(L.n_agents, 1)
     rng = np.random.default_rng(seed)
     bad = []
+    if setup is not None:
+        setup(batch, oras)
 
     def cmp(tag):
         recs = records(batch)
