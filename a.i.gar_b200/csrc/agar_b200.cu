@@ -39,7 +39,7 @@ __device__ __forceinline__ void stage_out(const DevParams& P, uint8_t* state, in
         dst[i] = ((const uint2*)(g_smem + (size_t)e * P.rec_stride))[w];
     }
 }
-/* stage >= 2 ("hot sections"): big records stay in HBM / L2; what every scan and every lane-0 step reads is cached in
+/* FULL kernels ("hot sections"): big records stay in HBM / L2; what every scan and every lane-0 step reads is cached in
  * shared memory — the pellet pool, and with hot_a > 0 also bytes [0, hot_a) = header, players, cells, viruses */
 __device__ __forceinline__ int hot_a_bytes(const DevParams& P) { return (P.hot_a + 15) / 16 * 16; }
 __device__ __forceinline__ int pel_cache_bytes(const DevParams& P) { return hot_a_bytes(P) + (P.L.pellet_cap * 4 + 15) / 16 * 16; }
@@ -55,11 +55,13 @@ __device__ __forceinline__ void pel_cache_copy(const DevParams& P, uint8_t* stat
     }
     __syncthreads();
 }
-template <int W>
+/* where a record lives during a launch: !FULL (the single-cell general kernel) stages the whole record in shared memory
+ * (stage_in / stage_out); FULL keeps it in HBM / L2 and caches the hot sections (pel_cache_copy) */
+template <int W, bool FULL>
 __device__ __forceinline__ void bind_ctx(Ctx<W>& c, const DevParams& P, int tile_id, int tiles, int env, uint8_t* state) {
     c.lane = c.t.thread_rank();
     c.env_id = (uint32_t)(P.first_env + (uint64_t)env);
-    c.rec = P.stage == 1 ? g_smem + (size_t)tile_id * P.rec_stride : state + (size_t)env * P.L.record_bytes;
+    c.rec = FULL ? state + (size_t)env * P.L.record_bytes : g_smem + (size_t)tile_id * P.rec_stride;
     c.h = (AgarEnvHeader*)(c.rec + P.L.off_header);
     c.pl = (AgarPlayer*)(c.rec + P.L.off_players);
     c.cells = (AgarCell*)(c.rec + P.L.off_cells);
@@ -69,19 +71,16 @@ __device__ __forceinline__ void bind_ctx(Ctx<W>& c, const DevParams& P, int tile
     c.pel = (uint32_t*)(c.rec + P.L.off_pellets);
     c.hist = (float*)(c.rec + P.L.off_hist);
     c.ev = (AgarEvent*)(c.rec + P.L.off_events);
-    c.scratch = g_smem + (P.stage == 1 ? (size_t)tiles * P.rec_stride : 0) + (size_t)tile_id * P.scratch_bytes;
-    if (P.stage >= 2) {
+    c.scratch = g_smem + (FULL ? 0 : (size_t)tiles * P.rec_stride) + (size_t)tile_id * P.scratch_bytes;
+    if (FULL) {
         uint8_t* hot = g_smem + (size_t)tiles * P.scratch_bytes + (size_t)tile_id * pel_cache_bytes(P);
         c.pel = (uint32_t*)(hot + hot_a_bytes(P));
-        /* header, players, cells, viruses are contiguous from byte 0 of the record: whichever of them end inside the cached
-         * prefix [0, hot_a) are served from shared memory (stage 4 caches header + players only: the bot bookkeeping and the
-         * command / fov fields every lane-0 bot turn walks through) */
-        if (P.hot_a >= (int)P.L.off_cells) {
+        if (P.hot_a) { /* hot_a = off_blobs: header, players, cells, viruses are contiguous from byte 0 of the record */
             c.h = (AgarEnvHeader*)(hot + P.L.off_header);
             c.pl = (AgarPlayer*)(hot + P.L.off_players);
+            c.cells = (AgarCell*)(hot + P.L.off_cells);
+            c.vir = (AgarMote*)(hot + P.L.off_viruses);
         }
-        if (P.hot_a >= (int)P.L.off_viruses) c.cells = (AgarCell*)(hot + P.L.off_cells);
-        if (P.hot_a >= (int)P.L.off_blobs) c.vir = (AgarMote*)(hot + P.L.off_viruses);
     }
 }
 
@@ -119,24 +118,22 @@ k_main(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const f
     const int tiles = blockDim.x / W;
     const int env0 = blockIdx.x * tiles;
     const int n_here = min(tiles, P.n_envs - env0);
-    if (P.stage == 1) stage_in(P, state, env0, n_here, false);
-    if (P.stage >= 2) pel_cache_copy(P, state, env0, n_here, tiles, true);
+    if (FULL) pel_cache_copy(P, state, env0, n_here, tiles, true);
+    else stage_in(P, state, env0, n_here, false);
     const int tile_id = threadIdx.x / W;
     const bool active = tile_id < n_here;
     {
         Ctx<W> c(cg::tiled_partition<W>(cg::this_thread_block()));
         const int env = env0 + (active ? tile_id : 0);
-        bind_ctx(c, P, active ? tile_id : 0, tiles, env, state);
+        bind_ctx<W, FULL>(c, P, active ? tile_id : 0, tiles, env, state);
         const int A = P.L.n_agents, K = P.L.n_players, SL = P.L.state_len;
         float* obs_env = obs ? obs + (size_t)env * A * SL : nullptr;
-        const bool psync = P.phase_sync != 0;             /* barriers at frame start and before the field update */
-        const bool psync_field = P.phase_sync == 2 || P.phase_sync >= 4; /* ... between the field phases */
-        const bool psync_bots = P.phase_sync >= 3;        /* ... between bot turns */
         /* One loop with ONE call site per helper: the multi-agent frame is ~22 k SASS instructions and instruction
          * fetch is its top stall (profiles/r01_k_main_cfg3_*), so nothing big may be inlined twice.  Iteration `it` is
          * frame f of decision d; the trailing observation (KF_OBS_AFTER) is one extra iteration without a frame.
-         * With phase_sync, CTA barriers between the phases keep all warps of the CTA in the same code region, so the
-         * instruction cache serves them together (idle tiles of a partly filled CTA only hit the barriers). */
+         * FULL: CTA barriers at frame start and before the field update keep all warps of the CTA in the same code
+         * region, so the instruction cache serves them together (idle tiles of a partly filled CTA only hit the
+         * barriers; measured 2.5x, DESIGN §4). */
         const int total = n_dec * n_frames;
         for (int it = 0; it <= total; ++it) {
             const bool last = it == total;
@@ -144,7 +141,7 @@ k_main(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const f
 #ifdef AGAR_PHASE_CLOCKS
             c.clk_t = clock64(), c.clk_env = env;
 #endif
-            if (psync) __syncthreads();
+            if (FULL) __syncthreads();
             CLK_MARK(0); /* (ptxas hoists this clock read above the barrier: the wait lands in the NEXT slot, the fov pass) */
             const int f = n_frames > 0 ? it % n_frames : 0, d = n_frames > 0 ? it / n_frames : 0;
             const bool emit = last || (f == 0 && (flags & KF_OBS_BEFORE)); /* observations leave the kernel here */
@@ -157,7 +154,6 @@ k_main(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const f
                 CLK_MARK(11); /* live-cell list */
             }
             for (int k = 0; k < K; ++k) {
-                if (psync_bots && k > 0) __syncthreads(); /* one bot turn per barrier interval */
                 if (active) {
                     if (!FULL || P.cfg.bot_type[k] == AGAR_BOT_NN) {
                         nn_turn_begin<W, FULL>(c, P, k, (emit && obs_env) ? obs_env + (size_t)k * SL : nullptr);
@@ -189,7 +185,7 @@ k_main(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const f
             CLK_MARK(1); /* bot turns */
             c.fov_done = false, c.n_live = -1;
             for (int ph = 0; ph < AGAR_FIELD_PHASES; ++ph) {
-                if (ph == 0 ? psync : psync_field) __syncthreads();
+                if (FULL && ph == 0) __syncthreads();
                 if (ph == 0) CLK_MARK(2); /* wait at the field barrier */
                 if (active) field_update_phase<W, FULL>(c, P, ph);
                 CLK_MARK(3 + ph); /* 3: viruses / blobs / players  4: merge, virus overlaps  5: pellets  6: blobs, player-player, spawn */
@@ -206,18 +202,17 @@ k_main(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const f
                 if (P.turn_done) P.turn_done[(size_t)env * A + a] = (uint8_t)c.pl[a].bot.exp_done;
             }
     }
-    if (P.stage == 1) stage_out(P, state, env0, n_here);
-    if (P.stage >= 2) {
+    if (FULL) {
         __syncthreads();
         pel_cache_copy(P, state, env0, n_here, tiles, false);
-    }
+    } else
+        stage_out(P, state, env0, n_here);
     export_tail(P, obs, env0, n_here);
 }
 
 
 /* ------------------------------------------------------------------ register-resident kernel (agar_simple.cuh) */
 struct SimplePlan {
-    int frame_sync; /* CTA barrier at every frame: the warps of a CTA fetch the same instructions together */
     int strideB; /* bytes between the staged [pellets .. end of record] regions of consecutive envs */
     int grid_off; /* byte offset of the env's G x G observation accumulator inside its region; 0: accumulate in the caller's row */
     int obs_warps; /* observer warps at the end of the CTA (0: every warp steps envs and encodes its own observations) */
@@ -319,7 +314,9 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
         SReg r;
         s_load(r, q);
         float* row = (obs != nullptr && valid) ? obs + (size_t)env * P.L.state_len : nullptr;
-        auto frame_bar = [&]() { /* the physics warps only: observers keep their own pace */
+        /* one barrier per frame: the warps of a CTA walk the ~5000-instruction frame body together (measured 1.9x at 1M envs
+         * and 2.3x at 4096); the physics warps only, observers keep their own pace */
+        auto frame_bar = [&]() {
             if (OBSW) named_bar_sync<SB_PHYS>(phys_threads);
             else __syncthreads();
         };
@@ -347,8 +344,7 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
                 s_observe<W>(r, q, P, d_o != 0, row, sub);
             }
             for (int f = 0; f < n_frames; ++f) {
-                if (SP.frame_sync == 1 || SP.frame_sync == 4) frame_bar();
-                if (SP.frame_sync == 2) __syncwarp();
+                frame_bar();
                 r.n_events = 0;
                 int d_o = s_turn_begin(r, P);
                 s_observe<W>(r, q, P, d_o != 0, nullptr, sub);
@@ -365,7 +361,6 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
                 }
                 double speed_pow;
                 s_turn_end<W>(r, P, act, sub, speed_pow);
-                if (SP.frame_sync == 4) frame_bar();
                 s_field_update<W>(r, q, P, env_id, sub, speed_pow);
             }
         }
@@ -397,19 +392,20 @@ k_init(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const u
     const int tiles = blockDim.x / W;
     const int env0 = blockIdx.x * tiles;
     const int n_here = min(tiles, P.n_envs - env0);
-    if (P.stage == 1)
+    if (FULL) {
+        if (mode == 0) { /* records stay in HBM: clear them in place */
+            const int chunks = (int)(P.L.record_bytes / 8);
+            uint2* dst = (uint2*)(state + (size_t)env0 * P.L.record_bytes);
+            for (int i = threadIdx.x; i < n_here * chunks; i += blockDim.x) dst[i] = make_uint2(0u, 0u);
+            __syncthreads();
+        }
+        pel_cache_copy(P, state, env0, n_here, tiles, true);
+    } else
         stage_in(P, state, env0, n_here, mode == 0);
-    else if (mode == 0) { /* records stay in HBM: clear them in place */
-        const int chunks = (int)(P.L.record_bytes / 8);
-        uint2* dst = (uint2*)(state + (size_t)env0 * P.L.record_bytes);
-        for (int i = threadIdx.x; i < n_here * chunks; i += blockDim.x) dst[i] = make_uint2(0u, 0u);
-        __syncthreads();
-    }
-    if (P.stage >= 2) pel_cache_copy(P, state, env0, n_here, tiles, true);
     const int tile_id = threadIdx.x / W;
     if (tile_id < n_here && (mask == nullptr || mode == 0 || mask[env0 + tile_id])) {
         Ctx<W> c(cg::tiled_partition<W>(cg::this_thread_block()));
-        bind_ctx(c, P, tile_id, tiles, env0 + tile_id, state);
+        bind_ctx<W, FULL>(c, P, tile_id, tiles, env0 + tile_id, state);
         const int K = P.L.n_players;
         if (mode == 0 || mode == 1) {
             if (mode == 1) { /* clear pools cooperatively: fresh lists and hash tables */
@@ -457,11 +453,11 @@ k_init(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const u
             c.t.sync();
         }
     }
-    if (P.stage == 1) stage_out(P, state, env0, n_here);
-    if (P.stage >= 2) {
+    if (FULL) {
         __syncthreads();
         pel_cache_copy(P, state, env0, n_here, tiles, false);
-    }
+    } else
+        stage_out(P, state, env0, n_here);
 }
 
 /* agar_get: one thread per (env, agent) or per env, straight from HBM */
@@ -500,22 +496,25 @@ __global__ void k_get(const __grid_constant__ DevParams P, const uint8_t* __rest
 }
 
 /* ------------------------------------------------------------------ host side */
+struct LaunchShape {
+    int W;       /* lanes per env */
+    int tiles;   /* envs per CTA (0: the shape does not fit) */
+    int threads; /* CTA size; k_simple with observer warps: tiles * W physics threads + the observers */
+    size_t smem; /* dynamic shared memory */
+};
 struct AgarEnv {
     AgarConfig cfg;
     AgarLayout L;
     DevParams P;
     uint8_t* state;
     double* deg_tab;
-    int n_envs, device, W, full, threads, tiles;
-    size_t smem_bytes;
-    int init_W, init_threads, init_tiles;
-    size_t init_smem;
+    int n_envs, device, full;
+    LaunchShape init; /* k_init<32, FULL> */
+    LaunchShape step; /* k_simple<W, false> if `simple`, else k_main<W, FULL> */
+    int simple;
     SimplePlan sp;
-    int simple_W, simple_threads;
-    size_t simple_smem;
-    SimplePlan sp_obs; /* observer launches of k_simple (plan_observers); obs_threads == 0: none */
-    int obs_threads;
-    size_t obs_smem;
+    SimplePlan sp_obs; /* observer launches of k_simple (plan_observers); obs.threads == 0: none */
+    LaunchShape obs;
     int64_t launches;
     int64_t observer_launches; /* launches of k_simple<W, true> */
     char err[256];
@@ -528,7 +527,6 @@ struct AgarEnv {
     uint32_t flag_seq;
     int host_polling; /* the pending step raises h_flag (zero-copy path) */
     int host_pending; /* agar_step_host_begin issued, _end not yet */
-    int host_zerocopy; /* pinned caller buffers are read / written in place (AGAR_HOST_ZEROCOPY=0 disables) */
 };
 static char g_create_err[256] = "";
 
@@ -557,19 +555,18 @@ static bool config_is_simple(const AgarConfig& c, const AgarLayout& L) {
            L.field_size < 128; /* the float32 candidate filter of k_simple's eat chain is analysed for coordinates below 128 (one player: 75) */
 }
 
-/* pick the launch shape for tile width W; returns false if one record does not fit in shared memory */
-static bool plan_launch(AgarEnv* e, int W) {
+/* launch shape of k_init / k_main for tile width W (bind_ctx's shared-memory layout); tiles == 0: one record does not fit */
+static LaunchShape plan_launch(const AgarEnv* e, int W) {
     const size_t budget = 200 * 1024;
-    size_t per_tile = (e->P.stage == 1 ? (size_t)e->P.rec_stride : 0) + (size_t)e->P.scratch_bytes +
-                      (e->P.stage >= 2 ? (size_t)((e->P.hot_a + 15) / 16 * 16) + (size_t)((e->L.pellet_cap * 4 + 15) / 16 * 16) : 0);
+    const size_t per_tile = (size_t)e->P.scratch_bytes +
+                            (e->full ? (size_t)((e->P.hot_a + 15) / 16 * 16) + (size_t)((e->L.pellet_cap * 4 + 15) / 16 * 16)
+                                     : (size_t)e->P.rec_stride);
     const int max_threads = (e->full && W == 32) ? 1024 : 512; /* k_main<32, true, 1024> exists for 32-lane tiles only */
     int tiles = e->full ? max_threads / W : 128 / W; /* as many envs per CTA as fit: the barriers then align more warps */
-    if (getenv("AGAR_MAX_TILES")) tiles = atoi(getenv("AGAR_MAX_TILES"));
-    if (tiles * W > max_threads) tiles = max_threads / W;
     while (tiles > 1 && per_tile * tiles > budget) tiles -= 1;
     if (W == 32 && tiles > 4) tiles -= tiles % 4; /* warps spread evenly over the four schedulers of an SM */
-    if (per_tile * tiles > budget) return false;
-    if (e->full && W == 32 && tiles > 8 && !getenv("AGAR_MAX_TILES")) {
+    if (per_tile * tiles > budget) return LaunchShape{W, 0, 0, 0};
+    if (e->full && W == 32 && tiles > 8) {
         /* one CTA per SM and all CTAs take about as long: fewer envs per CTA can fill the last wave better.  Cost model
          * waves x envs-per-CTA (measured, config 3 at 16384 envs: 32 -> 1.01e8, 28 -> 1.05e8, 24 -> 0.97e8, 20 -> 0.89e8) */
         int sms = 148;
@@ -583,11 +580,7 @@ static bool plan_launch(AgarEnv* e, int W) {
         }
         tiles = best;
     }
-    e->W = W;
-    e->tiles = tiles;
-    e->threads = tiles * W;
-    e->smem_bytes = per_tile * tiles;
-    return true;
+    return LaunchShape{W, tiles, tiles * W, per_tile * tiles};
 }
 
 /* cudaFuncSetAttribute is per kernel FUNCTION and process-wide, not per handle: two handles with different shared-memory
@@ -611,49 +604,41 @@ static cudaError_t launch_main_k(AgarEnv* e, const float* actions, float* obs, i
     static unsigned char done[64];
     cudaError_t err = ensure_max_smem(k_main<W, FULL, MAXT>, e->device, done);
     if (err != cudaSuccess) return err;
-    int blocks = (e->n_envs + e->tiles - 1) / e->tiles;
-    k_main<W, FULL, MAXT><<<blocks, e->threads, e->smem_bytes, s>>>(e->P, e->state, actions, obs, n_frames, n_dec, flags, dec_base);
+    int blocks = (e->n_envs + e->step.tiles - 1) / e->step.tiles;
+    k_main<W, FULL, MAXT><<<blocks, e->step.threads, e->step.smem, s>>>(e->P, e->state, actions, obs, n_frames, n_dec, flags, dec_base);
     return cudaGetLastError();
 }
 template <int W, bool FULL>
 static cudaError_t launch_main_t(AgarEnv* e, const float* actions, float* obs, int n_frames, int n_dec, int flags,
                                  uint32_t dec_base, cudaStream_t s) {
-    if (W == 32 && FULL && e->threads > 768) return launch_main_k<32, true, 1024>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
-    if (W == 32 && FULL && e->threads > 512) return launch_main_k<32, true, 768>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
+    if (W == 32 && FULL && e->step.threads > 768) return launch_main_k<32, true, 1024>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
+    if (W == 32 && FULL && e->step.threads > 512) return launch_main_k<32, true, 768>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
     return launch_main_k<W, FULL, 512>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
 }
-template <int W, bool FULL>
+template <bool FULL>
 static cudaError_t launch_init_t(AgarEnv* e, const uint8_t* mask, int mode, cudaStream_t s) {
     static unsigned char done[64];
-    cudaError_t err = ensure_max_smem(k_init<W, FULL>, e->device, done);
+    cudaError_t err = ensure_max_smem(k_init<32, FULL>, e->device, done);
     if (err != cudaSuccess) return err;
-    int blocks = (e->n_envs + e->init_tiles - 1) / e->init_tiles;
-    k_init<W, FULL><<<blocks, e->init_threads, e->init_smem, s>>>(e->P, e->state, mask, mode);
+    int blocks = (e->n_envs + e->init.tiles - 1) / e->init.tiles;
+    k_init<32, FULL><<<blocks, e->init.threads, e->init.smem, s>>>(e->P, e->state, mask, mode);
     return cudaGetLastError();
 }
-#define DISPATCH(fn, ...)                                                 \
-    (e->full ? (e->W == 32  ? fn<32, true>(__VA_ARGS__)                   \
-                : e->W == 16 ? fn<16, true>(__VA_ARGS__)                  \
-                : e->W == 8  ? fn<8, true>(__VA_ARGS__)                   \
-                             : fn<4, true>(__VA_ARGS__))                  \
-             : (e->W == 32  ? fn<32, false>(__VA_ARGS__)                  \
-                             : fn<32, false>(__VA_ARGS__)))
 
 static int launch_main(AgarEnv* e, const float* actions, float* obs, int n_frames, int n_dec, int flags, uint32_t dec_base,
                        void* stream) {
     AgarEnv* env = e;
     CU(cudaSetDevice(e->device));
     cudaError_t err;
-    if (e->simple_W) {
+    if (e->simple) {
         /* observer warps encode the observations a launch hands off before its frames (KF_OBS_BEFORE), when enough frames
          * follow each one to hide the encoder; a trailing observation (KF_OBS_AFTER) stays with the physics warps */
-        const bool handoff = e->obs_threads && (flags & KF_OBS_BEFORE) && obs != nullptr && n_frames >= SIMPLE_OBS_MIN_FRAMES;
+        const bool handoff = e->obs.threads && (flags & KF_OBS_BEFORE) && obs != nullptr && n_frames >= SIMPLE_OBS_MIN_FRAMES;
         const SimplePlan& sp = handoff ? e->sp_obs : e->sp;
-        const int threads = handoff ? e->obs_threads : e->simple_threads;
-        const size_t smem = handoff ? e->obs_smem : e->simple_smem;
-        const int per = (threads - 32 * sp.obs_warps) / e->simple_W;
-        if (threads % 32 || threads > (handoff ? simple_max_threads(e->simple_W) : 256) || per < 1 || per * e->simple_W % 32 ||
-            (sp.obs_warps && (!sp.grid_off || 32 * sp.obs_warps % SIMPLE_OBS_LANES)))
+        const LaunchShape& sh = handoff ? e->obs : e->step;
+        const int per = (sh.threads - 32 * sp.obs_warps) / sh.W; /* what k_simple derives from blockDim */
+        if (sh.threads % 32 || sh.threads > (handoff ? simple_max_threads(sh.W) : 256) || per < 1 || per != sh.tiles ||
+            per * sh.W % 32 || (sp.obs_warps && (!sp.grid_off || 32 * sp.obs_warps % SIMPLE_OBS_LANES)))
             return fail(e, AGAR_E_INVALID, "inconsistent k_simple launch shape%s", "");
         int blocks = (e->n_envs + per - 1) / per;
 #define LAUNCH_SIMPLE(WW, OB)                                                                                                 \
@@ -661,23 +646,30 @@ static int launch_main(AgarEnv* e, const float* actions, float* obs, int n_frame
         static unsigned char done_##WW##OB[64];                                                                               \
         err = ensure_max_smem(k_simple<WW, OB>, e->device, done_##WW##OB);                                                    \
         if (err == cudaSuccess) {                                                                                             \
-            k_simple<WW, OB><<<blocks, threads, smem, (cudaStream_t)stream>>>(e->P, sp, e->state, actions, obs, n_frames,     \
-                                                                              n_dec, flags, dec_base);                        \
+            k_simple<WW, OB><<<blocks, sh.threads, sh.smem, (cudaStream_t)stream>>>(e->P, sp, e->state, actions, obs,         \
+                                                                                    n_frames, n_dec, flags, dec_base);        \
             err = cudaGetLastError();                                                                                         \
         }                                                                                                                     \
     } while (0)
-        if (handoff && e->simple_W == 4) LAUNCH_SIMPLE(4, true);
+        if (handoff && sh.W == 4) LAUNCH_SIMPLE(4, true);
         else if (handoff) LAUNCH_SIMPLE(8, true);
-        else if (e->simple_W == 1) LAUNCH_SIMPLE(1, false);
-        else if (e->simple_W == 2) LAUNCH_SIMPLE(2, false);
-        else if (e->simple_W == 4) LAUNCH_SIMPLE(4, false);
-        else if (e->simple_W == 8) LAUNCH_SIMPLE(8, false);
-        else if (e->simple_W == 16) LAUNCH_SIMPLE(16, false);
+        else if (sh.W == 1) LAUNCH_SIMPLE(1, false);
+        else if (sh.W == 2) LAUNCH_SIMPLE(2, false);
+        else if (sh.W == 4) LAUNCH_SIMPLE(4, false);
+        else if (sh.W == 8) LAUNCH_SIMPLE(8, false);
+        else if (sh.W == 16) LAUNCH_SIMPLE(16, false);
         else LAUNCH_SIMPLE(32, false);
 #undef LAUNCH_SIMPLE
         if (handoff && err == cudaSuccess) e->observer_launches += 1;
-    } else
-        err = DISPATCH(launch_main_t, e, actions, obs, n_frames, n_dec, flags, dec_base, (cudaStream_t)stream);
+    } else {
+        const int W = e->step.W;
+        cudaStream_t s = (cudaStream_t)stream;
+        err = !e->full ? launch_main_t<32, false>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
+              : W == 32 ? launch_main_t<32, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
+              : W == 16 ? launch_main_t<16, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
+              : W == 8  ? launch_main_t<8, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
+                        : launch_main_t<4, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
+    }
     if (err != cudaSuccess) return fail(e, AGAR_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     e->launches += 1;
     return AGAR_OK;
@@ -685,9 +677,8 @@ static int launch_main(AgarEnv* e, const float* actions, float* obs, int n_frame
 static int launch_init(AgarEnv* e, const uint8_t* mask, int mode, void* stream) {
     AgarEnv* env = e;
     CU(cudaSetDevice(e->device));
-    cudaError_t err = e->full ? (e->init_W == 32 ? launch_init_t<32, true>(e, mask, mode, (cudaStream_t)stream)
-                                                  : launch_init_t<8, true>(e, mask, mode, (cudaStream_t)stream))
-                              : launch_init_t<32, false>(e, mask, mode, (cudaStream_t)stream);
+    cudaError_t err = e->full ? launch_init_t<true>(e, mask, mode, (cudaStream_t)stream)
+                              : launch_init_t<false>(e, mask, mode, (cudaStream_t)stream);
     if (err != cudaSuccess) return fail(e, AGAR_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     e->launches += 1;
     return AGAR_OK;
@@ -714,9 +705,9 @@ static int simple_ctas_per_sm(int device, int threads, size_t smem) {
  * the observers are used only where their launch needs no more waves than the inline one (4096 envs at W = 8: one wave
  * each; 4608: two against one). */
 static void plan_observers(AgarEnv* e) {
-    e->obs_threads = 0;
+    e->obs = LaunchShape{};
     e->sp_obs = e->sp;
-    const int W = e->simple_W;
+    const int W = e->step.W;
     if ((W != 4 && W != 8) || !e->sp.grid_off || e->L.pellet_cap > 64 * SIMPLE_OBS_LANES) return; /* SMask<SIMPLE_OBS_LANES> */
     if (cudaSetDevice(e->device) != cudaSuccess) {
         cudaGetLastError();
@@ -735,18 +726,17 @@ static void plan_observers(AgarEnv* e) {
     if (smem > 200 * 1024) return;
     const int threads = (warps + K) * 32;
     const int occ = W == 8 ? simple_ctas_per_sm<8, true>(e->device, threads, smem) : simple_ctas_per_sm<4, true>(e->device, threads, smem);
-    const int occ_in = W == 8 ? simple_ctas_per_sm<8, false>(e->device, e->simple_threads, e->simple_smem)
-                              : simple_ctas_per_sm<4, false>(e->device, e->simple_threads, e->simple_smem);
+    const int occ_in = W == 8 ? simple_ctas_per_sm<8, false>(e->device, e->step.threads, e->step.smem)
+                              : simple_ctas_per_sm<4, false>(e->device, e->step.threads, e->step.smem);
     if (occ < 1 || occ_in < 1) return;
-    const long long per_in = e->simple_threads / W;
+    const long long per_in = e->step.tiles;
     const long long waves = ((e->n_envs + per - 1) / per + (long long)sms * occ - 1) / ((long long)sms * occ);
     const long long waves_in = ((e->n_envs + per_in - 1) / per_in + (long long)sms * occ_in - 1) / ((long long)sms * occ_in);
     if (waves > waves_in) return;
     e->sp_obs.obs_warps = K;
     e->sp_obs.snap_off = (int)env_bytes;
     e->sp_obs.snap_stride = snap_stride;
-    e->obs_threads = threads;
-    e->obs_smem = smem;
+    e->obs = LaunchShape{W, per, threads, smem};
 }
 
 /* Lanes per env.  Single-cell pellet-collection configs (config_is_simple) with G <= 16: 1, 2, 4, 8, 16, 32 select the
@@ -757,46 +747,39 @@ extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
     /* the register-resident kernel bins a pellet into at most two squares per axis: 2 * radius < fov / G needs G <= 16 */
     if (!e->full && e->L.grid_squares <= 16 && (W == 1 || W == 2 || W == 4 || W == 8 || W == 16 || W == 32) &&
         !getenv("AGAR_GENERAL_KERNEL")) {
-        int tail_words = (int)((e->L.record_bytes - e->L.off_pellets) / 4);
-        e->sp.strideB = (tail_words | 1) * 4;
-        e->sp.grid_off = 0;
-        e->sp.obs_warps = e->sp.snap_off = e->sp.snap_stride = 0;
+        const int tail_words = (int)((e->L.record_bytes - e->L.off_pellets) / 4);
+        SimplePlan sp = {};
+        sp.strideB = (tail_words | 1) * 4;
         /* the observation's G x G sums are accumulated in shared memory and leave once, as consecutive floats of the row
          * (measured: 4096 envs W=8 +1.2 %, 65536 envs W=2 +8 %).  Not at one lane per env: 484 more bytes per env halve the
          * resident envs per SM there (1M envs: 3.28e9 -> 1.52e9), and a lone lane's stores are strided either way. */
-        const char* genv = getenv("AGAR_SIMPLE_OBS_SMEM");
-        if (genv ? atoi(genv) != 0 : W >= 2) {
+        if (W >= 2) {
             const int gg = e->L.grid_squares * e->L.grid_squares;
-            e->sp.grid_off = tail_words * 4;
-            e->sp.strideB = ((tail_words + gg) | 1) * 4;
+            sp.grid_off = tail_words * 4;
+            sp.strideB = ((tail_words + gg) | 1) * 4;
         }
         if (e->L.pellet_cap > (W >= 4 ? 64 : 128) * W) /* two mask words per lane: SMask<W>, agar_simple.cuh */
             return fail(e, AGAR_E_UNSUPPORTED, "pellet pool too large for this tile width%s", "");
         int threads = 128; /* measured (round 2, exact libm arithmetic): four warps per CTA beat two at every batch size (4096 envs: 7.7e8 vs 7.0e8) */
-        const char* tenv = getenv("AGAR_SIMPLE_THREADS");
-        if (tenv && atoi(tenv) >= 32) threads = atoi(tenv) / 32 * 32;
-        if (threads > 256) threads = 256; /* __launch_bounds__(256, ...) */
-        /* measured: one CTA barrier per frame is worth 1.9x at 1M envs and 2.3x at 4096 (a warp-level barrier is
-         * worth nothing): the warps of a CTA then walk the ~5000-instruction frame body together */
-        e->sp.frame_sync = getenv("AGAR_SIMPLE_SYNC") ? atoi(getenv("AGAR_SIMPLE_SYNC")) : 1;
-        size_t per_env = (size_t)e->sp.strideB;
+        const size_t per_env = (size_t)sp.strideB;
         while (threads > 32 && per_env * (threads / W) > 200 * 1024) threads -= 32;
         if (per_env * (threads / W) > 200 * 1024)
             return fail(e, AGAR_E_NOMEM, "pellet pool + event ring of %s do not fit in shared memory at this tile width", "the envs of one CTA");
-        e->simple_W = W;
-        e->simple_threads = threads;
-        e->simple_smem = per_env * (threads / W);
-        e->W = W;
+        e->simple = 1;
+        e->sp = sp;
+        e->step = LaunchShape{W, threads / W, threads, per_env * (threads / W)};
         plan_observers(e);
         return AGAR_OK;
     }
     bool ok = W == 32 || (e->full && (W == 4 || W == 8 || W == 16));
     if (!ok) return fail(e, AGAR_E_INVALID, "unsupported tile width%s", "");
-    if (!plan_launch(e, W)) return fail(e, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
-    e->simple_W = 0;
+    const LaunchShape s = plan_launch(e, W);
+    if (!s.tiles) return fail(e, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
+    e->simple = 0;
+    e->step = s;
     return AGAR_OK;
 }
-extern "C" int agar_get_tile_width(const AgarEnv* e) { return e ? e->W : 0; }
+extern "C" int agar_get_tile_width(const AgarEnv* e) { return e ? e->step.W : 0; }
 
 extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64_t seed, uint64_t first_env_id, void* stream,
                            AgarEnv** out) {
@@ -832,29 +815,24 @@ extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64
     int obs_bytes = obs_scratch_bytes(L.grid_squares, e->full != 0);
     /* the pellet index (agar_dev.cuh) lives in the same scratch: it is built after the players have moved (velocities dead)
      * and before the next bot phase (observation tables dead); pools of <= 8 chunks are scanned directly */
-    P.pel_index = e->full && L.pellet_cap > (getenv("AGAR_PEL_INDEX_MIN") ? atoi(getenv("AGAR_PEL_INDEX_MIN")) : 256) && !(getenv("AGAR_PEL_INDEX") && atoi(getenv("AGAR_PEL_INDEX")) == 0);
+    P.pel_index = e->full && L.pellet_cap > 256;
     const int gb_idx = (P.S + 9) / 10; /* AG_IDX_CELL */
     int idx_bytes = P.pel_index ? ((gb_idx * gb_idx + 3) & ~1) * 2 + L.pellet_cap * 2 + 128 + 64 + 16 : 0; /* counters, entries, sort list, ex-blob list */
     if (idx_bytes > vel_bytes) vel_bytes = idx_bytes;
     P.scratch_bytes = ((vel_bytes > obs_bytes ? vel_bytes : obs_bytes) + 15) / 16 * 16 + 8;
     P.live_off = P.scratch_bytes; /* live-cell list: uint16 per cell slot, after the observation / velocity scratch */
     if (e->full) P.scratch_bytes += (L.n_players * L.cell_cap * 2 + 15) / 16 * 16;
-    /* Where a record lives during a launch.  1: whole record staged in shared memory (single-cell general kernel).
-     * Multi-agent configs keep the record in HBM / L2 and cache on chip what every scan and lane-0 step reads:
-     * 3 = header + players + cells + viruses + pellet pool if at least 12 envs per CTA still fit, else 2 = the pellet
-     * pool only (the 16-player arena: 23 KB of cells).  Measured when the policy was chosen (16 envs per CTA): config 3
-     * 6.3e7 / 7.3e7 / 7.7e7 env-steps/s for 1 / 2 / 3; config 4 0.75e6 (1, 3 warps per SM) / 3.3e6 (2) / 1.6e6 (3);
-     * with 32 envs per CTA (profiles/r01_sweep.txt) config 3 does 9.1e7 (2) / 9.6e7 (3). */
-    if (!e->full)
-        P.stage = 1;
-    else {
-        size_t hot3 = (size_t)((L.off_blobs + 15) / 16 * 16) + (size_t)((L.pellet_cap * 4 + 15) / 16 * 16) + P.scratch_bytes;
-        P.stage = hot3 * 12 <= 200 * 1024 ? 3 : 2;
+    /* Where a record lives during a launch (bind_ctx).  The single-cell general kernel stages the whole record in shared
+     * memory.  Multi-agent configs keep the record in HBM / L2 and cache on chip what every scan and lane-0 step reads:
+     * header + players + cells + viruses (hot_a = off_blobs) + pellet pool if at least 12 envs per CTA still fit, else the
+     * pellet pool only (the 16-player arena: 23 KB of cells).  Measured when the policy was chosen (16 envs per CTA):
+     * config 3 6.3e7 / 7.3e7 / 7.7e7 env-steps/s for whole record / pool / hot sections; config 4 0.75e6 (whole record, 3
+     * warps per SM) / 3.3e6 (pool) / 1.6e6 (hot sections); with 32 envs per CTA (profiles/r01_sweep.txt) config 3 does
+     * 9.1e7 (pool) / 9.6e7 (hot sections). */
+    if (e->full) {
+        size_t hot = (size_t)((L.off_blobs + 15) / 16 * 16) + (size_t)((L.pellet_cap * 4 + 15) / 16 * 16) + P.scratch_bytes;
+        P.hot_a = hot * 12 <= 200 * 1024 ? (int)L.off_blobs : 0;
     }
-    if (getenv("AGAR_STAGE")) P.stage = atoi(getenv("AGAR_STAGE"));
-    P.hot_a = P.stage == 3 ? (int)L.off_blobs : (P.stage == 4 ? (int)L.off_cells : 0);
-    /* multi-agent kernels are instruction-fetch bound: lock-step the CTA's warps phase by phase (measured 2x) */
-    P.phase_sync = getenv("AGAR_PHASE_SYNC") ? atoi(getenv("AGAR_PHASE_SYNC")) : e->full;
     double speed_modifier = 1.0 / 30;
     P.move_speed = 90 * speed_modifier;
     P.decay_rate = 1 - (0.01 * speed_modifier);
@@ -880,16 +858,12 @@ extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64
     CU(cudaMemcpyAsync(e->deg_tab, tab, sizeof tab, cudaMemcpyHostToDevice, (cudaStream_t)stream));
     CU(cudaStreamSynchronize((cudaStream_t)stream)); /* tab is a stack buffer */
     P.deg_tab = e->deg_tab;
-    {   /* k_init always runs with 32-lane tiles (8 if a record is too big for four tiles... it is not hot) */
-        if (!plan_launch(e, 32)) {
-            cudaFree(e->state), cudaFree(e->deg_tab), free(e);
-            return fail(nullptr, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
-        }
-        e->init_W = 32, e->init_threads = e->threads, e->init_tiles = e->tiles, e->init_smem = e->smem_bytes;
+    e->init = plan_launch(e, 32); /* k_init always runs with 32-lane tiles */
+    if (!e->init.tiles) {
+        cudaFree(e->state), cudaFree(e->deg_tab), free(e);
+        return fail(nullptr, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
     }
     int W = e->full ? 32 : (n_envs <= 8192 ? 8 : (n_envs <= 32768 ? 2 : 1)); /* tools/sweep.py, profiles/r01_sweep.txt */
-    const char* wenv = getenv("AGAR_TILE_W");
-    if (wenv && atoi(wenv) > 0) W = atoi(wenv);
     if (agar_set_tile_width(e, W) != AGAR_OK && agar_set_tile_width(e, 8) != AGAR_OK && agar_set_tile_width(e, 32) != AGAR_OK) {
         snprintf(g_create_err, sizeof g_create_err, "%s", e->err);
         cudaFree(e->state), cudaFree(e->deg_tab), free(e);
@@ -1019,14 +993,12 @@ extern "C" int agar_step_host_begin(AgarEnv* e, const float* actions_host, int n
         e->d_done = (uint8_t*)e->d_reward + EA * 4;
         CU(cudaMemsetAsync(e->d_obs, 0, EA * e->L.state_len * sizeof(float), s));
         CU(cudaMemsetAsync(e->d_reward, 0, turn_words * 4, s));
-        const char* zc = getenv("AGAR_HOST_ZEROCOPY");
-        e->host_zerocopy = zc ? atoi(zc) : 1;
     }
     /* Pinned caller buffers (cudaHostAlloc / cudaHostRegister / torch pin_memory) are visible to the device: the step
      * kernel reads the actions in place and its CTAs store the results straight into them (export_tail).  Pageable buffers take the
      * copy-engine path. */
-    const float* act_dev = e->host_zerocopy ? (const float*)pinned_dev_ptr(actions_host) : nullptr;
-    float* obs_dev_host = (e->host_zerocopy && obs_host) ? (float*)pinned_dev_ptr(obs_host) : nullptr;
+    const float* act_dev = (const float*)pinned_dev_ptr(actions_host);
+    float* obs_dev_host = (float*)pinned_dev_ptr(obs_host);
     const bool zero_copy = act_dev && (!obs_host || (obs_dev_host && ((uintptr_t)obs_dev_host & 15) == 0));
     if (!zero_copy) CU(cudaMemcpyAsync(e->d_actions, actions_host, EA * 4 * sizeof(float), cudaMemcpyHostToDevice, s));
     e->P.turn_reward = e->d_reward, e->P.turn_done = e->d_done; /* reward / done written by the step kernel itself */

@@ -39,14 +39,14 @@ struct DevParams {
     AgarConfig cfg;
     AgarLayout L;
     int S, nb, n_envs, rec_stride; /* rec_stride: bytes between staged records in shared memory */
-    int scratch_bytes, full, stage, phase_sync; /* phase_sync: CTA barriers between frame phases keep the warps' instruction streams aligned */ /* stage: 1 = records live in shared memory during a launch, 0 = in HBM/L2 */
+    int scratch_bytes, full;
     double move_speed, decay_rate, blob_mass, virus_split_mass, start_radius, virus_radius;
     double pellet_r[4];
     double pow_n[17];
     const double* deg_tab; /* cos(d*pi/180)[360], sin(...)[360] — host libm, exactly the oracle's table */
     uint64_t seed, first_env;
     int pel_index; /* 1: multi-agent configs with a large pellet pool build the per-env bucket index every frame (agar_dev.cuh) */
-    int hot_a, live_off; /* live_off: offset of the live-cell list in a tile's scratch (multi-agent configs) */ /* stage >= 2: bytes [0, hot_a) of a record (header, players, cells, viruses) are cached in shared memory too */
+    int hot_a, live_off; /* live_off: offset of the live-cell list in a tile's scratch (multi-agent configs) */ /* hot_a: 0 or off_blobs; FULL kernels cache bytes [0, hot_a) of a record (header, players, cells, viruses) in shared memory too */
     /* optional per-launch outputs of the last bot turn ([E][A]); NULL = use agar_get */
     float* turn_reward;
     uint8_t* turn_done;

@@ -18,5 +18,5 @@ for i in range(steps):
     s.record(); b.rollout_random(125, 8, (i + 1) * 125); e.record(); torch.cuda.synchronize()
     ts.append(s.elapsed_time(e))
 ms = sum(ts) / len(ts)
-print("config %s, %d envs: %.3e env-steps/s (%.1f ms per 1000-frame rollout, tile %d, PHASE_SYNC=%s)" % (
-    which, E, E * 1000 / (ms * 1e-3), ms, b.tile_width, os.environ.get("AGAR_PHASE_SYNC", "default")))
+print("config %s, %d envs: %.3e env-steps/s (%.1f ms per 1000-frame rollout, tile %d)" % (
+    which, E, E * 1000 / (ms * 1e-3), ms, b.tile_width))

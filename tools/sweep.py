@@ -30,4 +30,4 @@ if __name__ == "__main__":
         for W in Ws:
             dec = (125 if E <= 16384 else 25) if which == "1" else 12
             v, ms = measure(E, W, decisions=dec, which=which)
-            print(json.dumps({"config": which, "envs": E, "tile": W, "env_steps_per_s": v, "ms": ms, "frames": dec * 8, "threads": os.environ.get("AGAR_SIMPLE_THREADS", "64")}), flush=True)
+            print(json.dumps({"config": which, "envs": E, "tile": W, "env_steps_per_s": v, "ms": ms, "frames": dec * 8}), flush=True)
