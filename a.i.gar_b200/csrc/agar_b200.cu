@@ -495,6 +495,112 @@ __global__ void k_get(const __grid_constant__ DevParams P, const uint8_t* __rest
     }
 }
 
+/* A record may only be installed if no kernel can index out of bounds with it.  The record fields the kernels use as a
+ * loop bound or an index, and where:
+ *   header n_viruses  <= virus_cap  loops over c.vir (agar_dev.cuh update_viruses_blobs, virus_remove, any_player_mote_hit;
+ *                                   agar_bots.cuh observation and greedy scans), slot of the next virus (spawn_viruses)
+ *   header n_blobs    <= blob_cap   loops over c.blob (update_viruses_blobs, blob_remove, any_player_mote_hit), slot of the
+ *                                   next ejected blob (player_ejections)
+ *   header n_fat      <= fat_cap    counter of the live ex-blob slots: spawn_pellets' refill target
+ *   header n_pellets  <= pellet_cap counter of the live pellet slots: the refill target of spawn_pellets and of
+ *                                   agar_simple.cuh's field update, which also reads n_pellets == pellet_cap as a full pool
+ *   header n_dead     <= n_players  spawn_players copies dead_order[..n_dead] into a 16-entry array
+ *   dead_order[..n_dead]            player indices (spawn_players -> c.pl[k]): in [0, n_players), each at most once, so
+ *                                   that later deaths (delete_player_cell: dead_order[n_dead++]) stay inside the array
+ *   player n_cells    <= cell_cap   loops over a player's cells everywhere, CELLP(.., n_cells) of a new cell, P.pow_n[n_cells]
+ *   pellet words      x, y < S      build_pellet_index's bucket (y / 10) * gb + x / 10 indexes shared memory
+ * Counts must also be >= 0.  header n_events is not checked: it counts past event_cap by design, and every frame sets it to
+ * 0 before its first log_ev.  record_counts_bad checks everything but the pellet words (warp-cooperative, lane `lane` of a
+ * warp, the answer is this lane's share); k_records scans the pellet words over the whole CTA. */
+__device__ bool record_counts_bad(const AgarLayout& L, const uint8_t* rec, int lane) {
+    const AgarEnvHeader* h = (const AgarEnvHeader*)(rec + L.off_header);
+    const AgarPlayer* pl = (const AgarPlayer*)(rec + L.off_players);
+    const int K = L.n_players, nd = h->n_dead;
+    bool bad = h->n_viruses < 0 || h->n_viruses > L.virus_cap || h->n_blobs < 0 || h->n_blobs > L.blob_cap || h->n_fat < 0 ||
+               h->n_fat > L.fat_cap || h->n_pellets < 0 || h->n_pellets > L.pellet_cap || nd < 0 || nd > K;
+    if (!bad && lane < nd) {
+        const int k = h->dead_order[lane];
+        bad = k < 0 || k >= K;
+        for (int j = 0; j < lane; ++j) bad |= h->dead_order[j] == k;
+    }
+    if (lane < K) bad |= pl[lane].n_cells < 0 || pl[lane].n_cells > L.cell_cap;
+    return bad;
+}
+
+/* agar_save_records / agar_load_records: destination row r takes source row map[r] (map NULL: row r), -1 skips the row on
+ * load.  A CTA owns `rows` consecutive destination rows.  It first resolves each row's source (index in range) and, on load,
+ * validates the source records: one warp per row for the counts, then every thread of the CTA over the flattened
+ * (row, 16-byte pellet word) range, so that the check costs a few load latencies per CTA rather than one pool scan per warp.
+ * Then all threads copy the CTA's rows as one flattened (row, 16-byte word) range, four independent loads in flight per
+ * thread.  A skipped or refused row is left untouched. */
+constexpr int REC_ROWS_MAX = 64;
+__global__ void __launch_bounds__(256)
+k_records(const __grid_constant__ DevParams P, const uint4* __restrict__ src, int n_src, uint4* __restrict__ dst, int n_dst,
+          const int32_t* __restrict__ map, int load, int rows, unsigned int* err) {
+    __shared__ int row_src[REC_ROWS_MAX];
+    __shared__ int row_bad[REC_ROWS_MAX];
+    const AgarLayout& L = P.L;
+    const int r0 = blockIdx.x * rows, n_here = min(rows, n_dst - r0);
+    const int words = (int)(L.record_bytes / 16);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int r = threadIdx.x; r < n_here; r += blockDim.x) {
+        const int s = map ? map[r0 + r] : r0 + r;
+        const bool ok = s >= 0 && s < n_src;
+        if (!ok && !(load && s == -1)) atomicOr(err, (unsigned)AGAR_REC_ERR_INDEX);
+        row_src[r] = ok ? s : -1;
+        row_bad[r] = 0;
+    }
+    __syncthreads();
+    if (load) {
+        for (int r = warp; r < n_here; r += blockDim.x >> 5) {
+            const int s = row_src[r];
+            if (s >= 0 && __any_sync(0xffffffffu, record_counts_bad(L, (const uint8_t*)(src + (size_t)s * words), lane)) &&
+                lane == 0)
+                row_bad[r] = 1;
+        }
+        /* the pellet pool starts 16-byte aligned and is padded to 16 bytes (agar_layout.h); slots >= pellet_cap are padding */
+        const int pw = (L.pellet_cap + 3) / 4, pel_word = (int)(L.off_pellets / 16);
+        for (int i = threadIdx.x; i < n_here * pw; i += blockDim.x) {
+            const int r = i / pw, w = i - r * pw;
+            const int s = row_src[r];
+            if (s < 0) continue;
+            const uint4 v = src[(size_t)s * words + pel_word + w];
+            const uint32_t pk[4] = {v.x, v.y, v.z, v.w};
+            bool bad = false;
+#pragma unroll
+            for (int c = 0; c < 4; ++c)
+                bad |= 4 * w + c < L.pellet_cap && pk[c] != 0 && (AGAR_PELLET_X(pk[c]) >= P.S || AGAR_PELLET_Y(pk[c]) >= P.S);
+            if (bad) row_bad[r] = 1;
+        }
+        __syncthreads();
+        for (int r = threadIdx.x; r < n_here; r += blockDim.x)
+            if (row_src[r] >= 0 && row_bad[r]) {
+                row_src[r] = -1;
+                atomicOr(err, (unsigned)AGAR_REC_ERR_RECORD);
+            }
+    }
+    __syncthreads();
+    const int total = n_here * words;
+    constexpr int U = 4;
+    for (int base = threadIdx.x; base < total; base += U * blockDim.x) {
+        uint4 v[U];
+        int at[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int i = base + u * blockDim.x;
+            const int r = i / words, w = i - r * words;
+            const int s = i < total ? row_src[r] : -1;
+            at[u] = s < 0 ? -1 : r;
+            if (s >= 0) v[u] = src[(size_t)s * words + w];
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int i = base + u * blockDim.x;
+            if (at[u] >= 0) dst[(size_t)(r0 + at[u]) * words + (i - at[u] * words)] = v[u];
+        }
+    }
+}
+
 /* ------------------------------------------------------------------ host side */
 struct LaunchShape {
     int W;       /* lanes per env */
@@ -524,6 +630,7 @@ struct AgarEnv {
     void* h_turn; /* pinned: float reward[EA] | uint8 done[EA], then (64-byte aligned) the completion flag word */
     volatile uint32_t* h_flag; /* inside h_turn's allocation; the last CTA of a zero-copy step launch writes flag_seq there */
     unsigned int* d_export_count;
+    unsigned int* d_rec_err; /* sticky AGAR_REC_ERR_* bits of k_records */
     uint32_t flag_seq;
     int host_polling; /* the pending step raises h_flag (zero-copy path) */
     int host_pending; /* agar_step_host_begin issued, _end not yet */
@@ -849,30 +956,33 @@ extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64
         double a = d * (M_PI / 180.0);
         tab[d] = cos(a), tab[360 + d] = sin(a);
     }
-    if (cudaMalloc(&e->deg_tab, sizeof tab) != cudaSuccess || cudaMalloc(&e->state, (size_t)n_envs * L.record_bytes) != cudaSuccess) {
+    if (cudaMalloc(&e->deg_tab, sizeof tab) != cudaSuccess || cudaMalloc(&e->state, (size_t)n_envs * L.record_bytes) != cudaSuccess ||
+        cudaMalloc(&e->d_rec_err, sizeof(unsigned int)) != cudaSuccess) {
         cudaGetLastError();
         if (e->deg_tab) cudaFree(e->deg_tab);
+        if (e->state) cudaFree(e->state);
         free(e);
         return fail(nullptr, AGAR_E_NOMEM, "cudaMalloc of the env state failed%s", "");
     }
     CU(cudaMemcpyAsync(e->deg_tab, tab, sizeof tab, cudaMemcpyHostToDevice, (cudaStream_t)stream));
+    CU(cudaMemsetAsync(e->d_rec_err, 0, sizeof(unsigned int), (cudaStream_t)stream));
     CU(cudaStreamSynchronize((cudaStream_t)stream)); /* tab is a stack buffer */
     P.deg_tab = e->deg_tab;
     e->init = plan_launch(e, 32); /* k_init always runs with 32-lane tiles */
     if (!e->init.tiles) {
-        cudaFree(e->state), cudaFree(e->deg_tab), free(e);
+        cudaFree(e->state), cudaFree(e->deg_tab), cudaFree(e->d_rec_err), free(e);
         return fail(nullptr, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
     }
     int W = e->full ? 32 : (n_envs <= 8192 ? 8 : (n_envs <= 32768 ? 2 : 1)); /* tools/sweep.py, profiles/r01_sweep.txt */
     if (agar_set_tile_width(e, W) != AGAR_OK && agar_set_tile_width(e, 8) != AGAR_OK && agar_set_tile_width(e, 32) != AGAR_OK) {
         snprintf(g_create_err, sizeof g_create_err, "%s", e->err);
-        cudaFree(e->state), cudaFree(e->deg_tab), free(e);
+        cudaFree(e->state), cudaFree(e->deg_tab), cudaFree(e->d_rec_err), free(e);
         return AGAR_E_NOMEM;
     }
     rc = launch_init(e, nullptr, 0, stream);
     if (rc != AGAR_OK) {
         snprintf(g_create_err, sizeof g_create_err, "%s", e->err);
-        cudaFree(e->state), cudaFree(e->deg_tab), free(e);
+        cudaFree(e->state), cudaFree(e->deg_tab), cudaFree(e->d_rec_err), free(e);
         return rc;
     }
     *out = e;
@@ -888,6 +998,7 @@ extern "C" int agar_destroy(AgarEnv* e) {
     if (e->d_reward) cudaFree(e->d_reward);
     if (e->h_turn) cudaFreeHost(e->h_turn);
     if (e->d_export_count) cudaFree(e->d_export_count);
+    cudaFree(e->d_rec_err);
     free(e);
     return AGAR_OK;
 }
@@ -961,6 +1072,47 @@ extern "C" int agar_debug_load(AgarEnv* e, int env_index, const void* record_hos
     CU(cudaStreamSynchronize((cudaStream_t)stream));
     return AGAR_OK;
 }
+/* save (load = 0): bank rows <- env records; load: env records <- bank rows.  Enqueued on `stream`, no allocation. */
+static int launch_records(AgarEnv* e, const void* bank, int n_bank, const int32_t* index, int load, void* stream) {
+    AgarEnv* env = e;
+    const size_t rb = e->L.record_bytes;
+    const char* what = load ? "agar_load_records" : "agar_save_records";
+    if (!bank) return fail(e, AGAR_E_INVALID, "%s: bank is NULL", what);
+    if (n_bank < 1) return fail(e, AGAR_E_INVALID, "%s: the bank needs at least one row", what);
+    if (!index && n_bank != e->n_envs) return fail(e, AGAR_E_INVALID, "%s: without an index the bank has one row per env", what);
+    if ((uintptr_t)bank % 16) return fail(e, AGAR_E_INVALID, "%s: bank is not 16-byte aligned", what);
+    const uintptr_t b0 = (uintptr_t)bank, b1 = b0 + (uintptr_t)n_bank * rb;
+    const uintptr_t s0 = (uintptr_t)e->state, s1 = s0 + (uintptr_t)e->n_envs * rb;
+    if (b0 < s1 && s0 < b1) return fail(e, AGAR_E_INVALID, "%s: bank overlaps the env records", what);
+    CU(cudaSetDevice(e->device));
+    const int n_dst = load ? e->n_envs : n_bank;
+    const int words = (int)(rb / 16);
+    int rows = 4096 / words; /* about 64 KB per CTA */
+    rows = rows < 1 ? 1 : rows > REC_ROWS_MAX ? REC_ROWS_MAX : rows;
+    const uint4* src = (const uint4*)(load ? bank : e->state);
+    uint4* dst = (uint4*)(load ? e->state : (uint8_t*)bank);
+    k_records<<<(n_dst + rows - 1) / rows, 256, 0, (cudaStream_t)stream>>>(e->P, src, load ? n_bank : e->n_envs, dst, n_dst,
+                                                                           index, load, rows, e->d_rec_err);
+    CU(cudaGetLastError());
+    e->launches += 1;
+    return AGAR_OK;
+}
+extern "C" int agar_save_records(AgarEnv* e, void* bank_dev, const int32_t* env_index_dev, int n, void* stream) {
+    return e ? launch_records(e, bank_dev, n, env_index_dev, 0, stream) : AGAR_E_INVALID;
+}
+extern "C" int agar_load_records(AgarEnv* e, const void* bank_dev, int n_bank, const int32_t* bank_index_dev, void* stream) {
+    return e ? launch_records(e, bank_dev, n_bank, bank_index_dev, 1, stream) : AGAR_E_INVALID;
+}
+extern "C" int agar_record_error_flags(AgarEnv* e, void* stream) {
+    AgarEnv* env = e;
+    if (!e) return AGAR_E_INVALID;
+    CU(cudaSetDevice(e->device));
+    unsigned int flags = 0;
+    CU(cudaMemcpyAsync(&flags, e->d_rec_err, sizeof flags, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    CU(cudaStreamSynchronize((cudaStream_t)stream));
+    return (int)flags;
+}
+
 /* device-visible address of a pinned host buffer, or nullptr for pageable memory */
 static void* pinned_dev_ptr(const void* p) {
     if (!p) return nullptr;

@@ -4,6 +4,7 @@ reference's Model / Bot surface (src/model/model.py:90-120, src/model/bot.py:252
 PyTorch is used for device memory, streams and DLPack only.  There is NO CPU fallback: if libagar_b200.so is
 missing or no CUDA device is present every constructor raises."""
 import ctypes
+import hashlib
 import os
 
 import numpy as np
@@ -66,6 +67,63 @@ class AgarError(RuntimeError):
     pass
 
 
+class CheckpointError(AgarError):
+    """A checkpoint file that does not match the handle it is loaded into (the message names the field)."""
+
+
+CHECKPOINT_FORMAT = "agar_b200.records.v1"
+_CHECKPOINT_KEYS = ("format", "abi_version", "config", "layout", "n_envs", "seed", "first_env_id", "records", "sha256")
+
+
+def _struct_bytes(s):
+    return np.frombuffer(bytes(s), dtype=np.uint8).copy()
+
+
+def write_checkpoint(path, cfg, layout, n_envs, seed, first_env_id, records):
+    """Write a batch checkpoint (.npz, no pickled objects).  records: uint8 [n_envs, record_bytes] host array."""
+    records = np.ascontiguousarray(records, dtype=np.uint8)
+    with open(path, "wb") as f:  # a file object: numpy would otherwise append ".npz" to the name
+        np.savez(f, format=np.array(CHECKPOINT_FORMAT), abi_version=np.int64(lay.ABI_VERSION),
+                 config=_struct_bytes(cfg), layout=_struct_bytes(layout), n_envs=np.int64(n_envs),
+                 seed=np.uint64(seed), first_env_id=np.uint64(first_env_id), records=records,
+                 sha256=np.array(hashlib.sha256(records.tobytes()).hexdigest()))
+
+
+def read_checkpoint(path):
+    """Parse a checkpoint file without a device: a dict of its fields.  Raises CheckpointError for a file that is not a
+    checkpoint of this format and ABI version, whose records are not [n_envs, record_bytes] uint8, or whose digest differs."""
+    with np.load(path, allow_pickle=False) as z:
+        missing = [k for k in _CHECKPOINT_KEYS if k not in z.files]
+        if missing:
+            raise CheckpointError("%s: not a records checkpoint (missing %s)" % (path, ", ".join(missing)))
+        ck = {k: z[k] for k in _CHECKPOINT_KEYS}
+    if str(ck["format"]) != CHECKPOINT_FORMAT:
+        raise CheckpointError("%s: format %r, expected %r" % (path, str(ck["format"]), CHECKPOINT_FORMAT))
+    if int(ck["abi_version"]) != lay.ABI_VERSION:
+        raise CheckpointError("%s: abi_version %d, this library has %d" % (path, int(ck["abi_version"]), lay.ABI_VERSION))
+    for name, struct in (("config", lay.AgarConfig), ("layout", lay.AgarLayout)):
+        if ck[name].dtype != np.uint8 or ck[name].nbytes != ctypes.sizeof(struct):
+            raise CheckpointError("%s: %s is not the bytes of an %s" % (path, name, struct.__name__))
+    rec, rb = ck["records"], int(lay.AgarLayout.from_buffer_copy(ck["layout"].tobytes()).record_bytes)
+    if rec.dtype != np.uint8 or rec.ndim != 2 or rec.shape != (int(ck["n_envs"]), rb):
+        raise CheckpointError("%s: records of shape %s / %s do not match n_envs and the layout's record_bytes"
+                              % (path, rec.shape, rec.dtype))
+    if hashlib.sha256(np.ascontiguousarray(rec).tobytes()).hexdigest() != str(ck["sha256"]):
+        raise CheckpointError("%s: sha256 of the records does not match the stored digest" % path)
+    return ck
+
+
+def check_checkpoint(ck, cfg, layout, n_envs, seed, first_env_id):
+    """Raise CheckpointError naming the first field of a parsed checkpoint that differs from a handle's."""
+    want = (("config", _struct_bytes(cfg)), ("layout", _struct_bytes(layout)))
+    for name, mine in want:
+        if not np.array_equal(ck[name], mine):
+            raise CheckpointError("checkpoint %s bytes differ from the handle's" % name)
+    for name, mine in (("n_envs", n_envs), ("seed", seed), ("first_env_id", first_env_id)):
+        if int(ck[name]) != int(mine):
+            raise CheckpointError("checkpoint %s is %d, the handle's is %d" % (name, int(ck[name]), int(mine)))
+
+
 _GET_DTYPES = {lay.GET_REWARD: "float32", lay.GET_DONE: "uint8", lay.GET_VALID: "uint8", lay.GET_NEED_ACTION: "uint8",
                lay.GET_MASS: "float32", lay.GET_FOV: "float32", lay.GET_NCELLS: "int32", lay.GET_ALIVE: "uint8",
                lay.GET_STATS: "float64", lay.GET_OVERFLOW: "uint32", lay.GET_EVENT_HASH: "uint64"}
@@ -84,6 +142,7 @@ class AgarBatch(object):
         self.lib = load_library()
         self.cfg = cfg
         self.n_envs = int(n_envs)
+        self.seed, self.first_env_id = int(seed), int(first_env_id)  # the Philox key of slot e: (seed, first_env_id + e)
         self.device = torch.device("cuda", device)
         self.stream = stream
         self.h = ctypes.c_void_p()
@@ -139,6 +198,12 @@ class AgarBatch(object):
         fn = self.lib.agar_observer_launch_count
         fn.argtypes, fn.restype = [ctypes.c_void_p], ctypes.c_int64
         return int(fn(self.h))
+
+    def _lazy(self, name, argtypes, restype=ctypes.c_int):
+        """A C function bound on first use (not in EXPORTS: older builds load for A/B runs)."""
+        fn = getattr(self.lib, name)
+        fn.argtypes, fn.restype = argtypes, restype
+        return fn
 
     def _ptr(self, t):
         return ctypes.c_void_p(t.data_ptr()) if t is not None else ctypes.c_void_p()
@@ -229,6 +294,93 @@ class AgarBatch(object):
                                          self.stream.cuda_stream if self.stream is not None else self._stream())
         if rc != 0:
             self._check(rc)
+
+    # ---- state snapshots (agar_save_records / agar_load_records)
+    def _index(self, idx, n):
+        """a device tensor must already be int32 on this device (no copy, graph-capturable); anything else is converted"""
+        if self.torch.is_tensor(idx):
+            t = idx
+        else:
+            t = self.torch.as_tensor(np.asarray(idx, dtype=np.int32), device=self.device)
+        if t.dtype != self.torch.int32 or t.device != self.device or t.dim() != 1 or (n is not None and t.numel() != n):
+            raise ValueError("index must be a 1-D int32 tensor on %s%s" % (self.device, "" if n is None else " of %d entries" % n))
+        return t.contiguous()
+
+    def _bank(self, bank):
+        rb = int(self.layout.record_bytes)
+        if not (self.torch.is_tensor(bank) and bank.dtype == self.torch.uint8 and bank.device == self.device and
+                bank.dim() == 2 and bank.shape[1] == rb and bank.is_contiguous()):
+            raise ValueError("a bank is a contiguous uint8 tensor [n, %d] on %s" % (rb, self.device))
+        return bank
+
+    def snapshot(self, envs=None, out=None):
+        """Records of all envs, or of envs[i] for row i (any order, repeats allowed), as a uint8 device tensor
+        [n, record_bytes].  out: a bank to write into instead of a new tensor."""
+        idx = None if envs is None else self._index(envs, None)
+        n = self.n_envs if idx is None else idx.numel()
+        if out is None:
+            out = self.torch.empty((n, int(self.layout.record_bytes)), dtype=self.torch.uint8, device=self.device)
+        out = self._bank(out)
+        if out.shape[0] != n:
+            raise ValueError("out has %d rows, %d are saved" % (out.shape[0], n))
+        fn = self._lazy("agar_save_records", [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p])
+        self._check(fn(self.h, self._ptr(out), self._ptr(idx), int(n), self._stream()))
+        return out
+
+    def restore(self, bank, index=None):
+        """Overwrite env records from a bank: env e takes row index[e] (int32 [n_envs], -1 keeps env e); without an index
+        row e.  A record restored into the slot it came from continues bit for bit; one restored into another slot (a
+        clone: b.restore(b.snapshot(), index)) continues under that slot's Philox key.  Observation buffers are not
+        part of a record.  Rows that fail the device-side checks are not installed (record_error_flags())."""
+        bank = self._bank(bank)
+        idx = None if index is None else self._index(index, self.n_envs)
+        fn = self._lazy("agar_load_records", [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p])
+        self._check(fn(self.h, self._ptr(bank), int(bank.shape[0]), self._ptr(idx), self._stream()))
+
+    def record_error_flags(self):
+        """Sticky AGAR_REC_ERR_* bits (1: an index out of range, 2: a record refused on load); synchronises the stream."""
+        rc = self._lazy("agar_record_error_flags", [ctypes.c_void_p, ctypes.c_void_p])(self.h, self._stream())
+        if rc < 0:
+            self._check(rc)
+        return int(rc)
+
+    def _on_stream(self):
+        """torch's copies in stream order with this handle's calls"""
+        import contextlib
+        return self.torch.cuda.stream(self.stream) if self.stream is not None else contextlib.nullcontext()
+
+    def save_checkpoint(self, path):
+        """Write every env record with what a later load must match (config, layout, n_envs, seed, first_env_id)."""
+        with self._on_stream():
+            records = self.snapshot().cpu().numpy()
+        write_checkpoint(path, self.cfg, self.layout, self.n_envs, self.seed, self.first_env_id, records)
+
+    def load_checkpoint(self, path):
+        """Restore every env from a checkpoint of a handle with the same config, layout, n_envs, seed and first_env_id.
+        A file that differs in any of them, whose digest is wrong, or one of whose records the device-side checks refuse is
+        refused (CheckpointError) and the handle's state is left as it was."""
+        ck = read_checkpoint(path)
+        check_checkpoint(ck, self.cfg, self.layout, self.n_envs, self.seed, self.first_env_id)
+        with self._on_stream():
+            bank = self.torch.from_numpy(ck["records"]).to(self.device)
+            backup = self.snapshot()
+            self.restore(bank)
+            # an identity load installs every row unless the checks refuse it: compare instead of reading the sticky flags,
+            # which an earlier call may have set already
+            if not self.torch.equal(self.state_tensor(), bank):
+                self.restore(backup)
+                raise CheckpointError("%s: records that fail the device-side checks (counts or indices out of range); "
+                                      "nothing was loaded" % path)
+
+    @classmethod
+    def from_checkpoint(cls, path, device=0, tile_width=None, stream=None):
+        """A new handle matching a checkpoint (config, n_envs, seed, first_env_id), loaded from it."""
+        ck = read_checkpoint(path)
+        cfg = lay.AgarConfig.from_buffer_copy(ck["config"].tobytes())
+        b = cls(cfg, int(ck["n_envs"]), device=device, seed=int(ck["seed"]), first_env_id=int(ck["first_env_id"]),
+                tile_width=tile_width, stream=stream)
+        b.load_checkpoint(path)
+        return b
 
     # ---- parity / debugging
     def dump(self, env_index):

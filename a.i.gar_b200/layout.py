@@ -8,6 +8,7 @@ import math
 
 import numpy as np
 
+ABI_VERSION = 1  # AGAR_ABI_VERSION
 MAX_PLAYERS = 16
 MAX_CELLS = 16
 ACTION_DIM = 4
@@ -16,6 +17,7 @@ BOT_NN, BOT_GREEDY, BOT_RANDOM = 0, 1, 2
 OBS_REFERENCE, OBS_CANONICAL = 0, 1
 SIMPLE_STATE_LEN = 12  # Bot.getSimpleStateRepresentation, bot.py:511-548 (AGAR_SIMPLE_STATE_LEN)
 CF_EJECT, CF_INHASH = 1, 2
+REC_ERR_INDEX, REC_ERR_RECORD = 1, 2  # AGAR_REC_ERR_*
 
 (GET_REWARD, GET_DONE, GET_VALID, GET_NEED_ACTION, GET_MASS, GET_FOV, GET_NCELLS, GET_ALIVE, GET_STATS,
  GET_OVERFLOW, GET_EVENT_HASH) = range(11)

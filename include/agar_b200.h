@@ -299,6 +299,34 @@ void* agar_state_ptr(const AgarEnv* env);
 int agar_debug_dump(AgarEnv* env, int env_index, void* record_host, size_t bytes, void* stream);
 int agar_debug_load(AgarEnv* env, int env_index, const void* record_host, size_t bytes, void* stream);
 
+/* ---- state snapshots: whole env records moved on the device ----
+ * An env's record is its whole state (DESIGN.md §3); the Philox key (seed, first_env_id + slot) is not part of it.  Both
+ * calls are enqueued on `stream`, never synchronise the host and allocate nothing, so they can be captured in a CUDA graph;
+ * each is one kernel launch (agar_launch_count).  A bank is caller-owned device memory on the handle's device, rows of
+ * record_bytes bytes, 16-byte aligned, and must not overlap the handle's own records.
+ *   - A record restored into the slot it was saved from (same seed and first_env_id) continues bit for bit as the original
+ *     would have, at any tile width, kernel and launch shape.
+ *   - A record loaded into another slot (a clone: save, then load with an index) continues from the same state under that
+ *     slot's Philox key: its spawns, random bots and agar_rollout_random actions differ from the source's, deterministically.
+ *   - Observation and action buffers are caller memory and are not part of a record.  agar_observe leaves the rows of
+ *     skipping or dead agents untouched, so a caller comparing observations across a restore restores its observation
+ *     buffer too.  agar_rollout_random's decision_base is the caller's counter and is not stored either.
+ * Host-side refusals (AGAR_E_INVALID): a NULL bank, fewer than one row, a NULL index with a row count other than n_envs, a
+ * misaligned bank, a bank overlapping the records.  Device-side, an index out of range (other than -1 on load) leaves its
+ * row untouched and sets AGAR_REC_ERR_INDEX; the other rows of the call are still copied. */
+
+/* Gather env records into a bank: bank row i = record of env env_index_dev[i], for i < n.
+ * env_index_dev NULL: row i = env i, n must equal n_envs.  bank_dev: n * record_bytes bytes. */
+int agar_save_records(AgarEnv* env, void* bank_dev, const int32_t* env_index_dev, int n, void* stream);
+/* Overwrite env records from a bank of n_bank rows: env e takes bank row bank_index_dev[e]; -1 leaves env e unchanged.
+ * bank_index_dev NULL: env e takes row e (n_bank must equal n_envs).  To clone within a batch, save first, then load.
+ * A bank may come from a file: a row whose counts or indices could make a later kernel index out of bounds (the list is
+ * at k_records' validation in csrc/agar_b200.cu) is not installed, and AGAR_REC_ERR_RECORD is set. */
+int agar_load_records(AgarEnv* env, const void* bank_dev, int n_bank, const int32_t* bank_index_dev, void* stream);
+/* Sticky AGAR_REC_ERR_* bits that save / load raised on the device since create (synchronises `stream`). */
+enum { AGAR_REC_ERR_INDEX = 1, AGAR_REC_ERR_RECORD = 2 };
+int agar_record_error_flags(AgarEnv* env, void* stream);
+
 /* number of kernels this handle has launched so far (bench.py's gpu_launches) */
 int64_t agar_launch_count(const AgarEnv* env);
 /* how many of them handed their observations to observer warps (single-cell rollouts at 4 / 8 lanes per env) */
