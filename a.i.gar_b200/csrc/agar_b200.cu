@@ -40,17 +40,18 @@ __device__ __forceinline__ void stage_out(const DevParams& P, uint8_t* state, in
     }
 }
 /* FULL kernels ("hot sections"): big records stay in HBM / L2; what every scan and every lane-0 step reads is cached in
- * shared memory — the pellet pool, and with hot_a > 0 also bytes [0, hot_a) = header, players, cells, viruses */
-__device__ __forceinline__ int hot_a_bytes(const DevParams& P) { return (P.hot_a + 15) / 16 * 16; }
-__device__ __forceinline__ int pel_cache_bytes(const DevParams& P) { return hot_a_bytes(P) + (P.L.pellet_cap * 4 + 15) / 16 * 16; }
+ * shared memory — the pellet pool, and with hot_a > 0 also bytes [0, hot_a) = header, players, cells, viruses.  A tile's
+ * cache holds bytes [0, hot_a), then the pool, each padded to 16 bytes; the launch planner sizes CTAs with the same helpers. */
+__host__ __device__ __forceinline__ int hot_a_bytes(int hot_a) { return (hot_a + 15) / 16 * 16; }
+__host__ __device__ __forceinline__ int pel_cache_bytes(int hot_a, int pellet_cap) { return hot_a_bytes(hot_a) + (pellet_cap * 4 + 15) / 16 * 16; }
 __device__ __forceinline__ void pel_cache_copy(const DevParams& P, uint8_t* state, int env0, int n_here, int tiles, bool in) {
     const int wa = P.hot_a / 4, words = wa + P.L.pellet_cap;
     for (int i = threadIdx.x; i < n_here * words; i += blockDim.x) {
         int e = i / words, w = i - e * words;
         uint8_t* rec = state + (size_t)(env0 + e) * P.L.record_bytes;
-        uint8_t* hot = g_smem + (size_t)tiles * P.scratch_bytes + (size_t)e * pel_cache_bytes(P);
+        uint8_t* hot = g_smem + (size_t)tiles * P.scratch_bytes + (size_t)e * pel_cache_bytes(P.hot_a, P.L.pellet_cap);
         uint32_t* g = w < wa ? (uint32_t*)rec + w : (uint32_t*)(rec + P.L.off_pellets) + (w - wa);
-        uint32_t* s = w < wa ? (uint32_t*)hot + w : (uint32_t*)(hot + hot_a_bytes(P)) + (w - wa);
+        uint32_t* s = w < wa ? (uint32_t*)hot + w : (uint32_t*)(hot + hot_a_bytes(P.hot_a)) + (w - wa);
         if (in) *s = *g; else *g = *s;
     }
     __syncthreads();
@@ -73,8 +74,8 @@ __device__ __forceinline__ void bind_ctx(Ctx<W>& c, const DevParams& P, int tile
     c.ev = (AgarEvent*)(c.rec + P.L.off_events);
     c.scratch = g_smem + (FULL ? 0 : (size_t)tiles * P.rec_stride) + (size_t)tile_id * P.scratch_bytes;
     if (FULL) {
-        uint8_t* hot = g_smem + (size_t)tiles * P.scratch_bytes + (size_t)tile_id * pel_cache_bytes(P);
-        c.pel = (uint32_t*)(hot + hot_a_bytes(P));
+        uint8_t* hot = g_smem + (size_t)tiles * P.scratch_bytes + (size_t)tile_id * pel_cache_bytes(P.hot_a, P.L.pellet_cap);
+        c.pel = (uint32_t*)(hot + hot_a_bytes(P.hot_a));
         if (P.hot_a) { /* hot_a = off_blobs: header, players, cells, viruses are contiguous from byte 0 of the record */
             c.h = (AgarEnvHeader*)(hot + P.L.off_header);
             c.pl = (AgarPlayer*)(hot + P.L.off_players);
@@ -602,11 +603,32 @@ k_records(const __grid_constant__ DevParams P, const uint4* __restrict__ src, in
 }
 
 /* ------------------------------------------------------------------ host side */
+constexpr size_t SMEM_BUDGET = 200 * 1024; /* dynamic shared memory of one planned CTA, every kernel */
+
 struct LaunchShape {
     int W;       /* lanes per env */
     int tiles;   /* envs per CTA (0: the shape does not fit) */
     int threads; /* CTA size; k_simple with observer warps: tiles * W physics threads + the observers */
     size_t smem; /* dynamic shared memory */
+};
+typedef void (*InitFn)(DevParams, uint8_t*, const uint8_t*, int);
+typedef void (*MainFn)(DevParams, uint8_t*, const float*, float*, int, int, int, uint32_t);
+typedef void (*SimpleFn)(DevParams, SimplePlan, uint8_t*, const float*, float*, int, int, int, uint32_t);
+/* What a launch runs, resolved once by plan_launches: the instantiation, its shape and, for k_simple, its plan */
+struct InitLaunch {
+    InitFn fn; /* k_init<32, FULL> */
+    LaunchShape sh;
+};
+struct StepLaunch {
+    MainFn main;     /* k_main<W, FULL, MAXT>, or */
+    SimpleFn simple; /* k_simple<W, OBSW>; neither: no such launch */
+    LaunchShape sh;
+    SimplePlan sp;
+};
+struct LaunchPlan {
+    InitLaunch init;
+    StepLaunch step; /* every step launch that hands no observation off */
+    StepLaunch obs;  /* k_simple<W, true>: the launches that hand decision observations off to observer warps */
 };
 struct AgarEnv {
     AgarConfig cfg;
@@ -614,13 +636,9 @@ struct AgarEnv {
     DevParams P;
     uint8_t* state;
     double* deg_tab;
-    int n_envs, device, full;
-    LaunchShape init; /* k_init<32, FULL> */
-    LaunchShape step; /* k_simple<W, false> if `simple`, else k_main<W, FULL> */
-    int simple;
-    SimplePlan sp;
-    SimplePlan sp_obs; /* observer launches of k_simple (plan_observers); obs.threads == 0: none */
-    LaunchShape obs;
+    int n_envs, device;
+    int sms; /* multiprocessors of the device, for the planner's wave counts */
+    LaunchPlan plan;
     int64_t launches;
     int64_t observer_launches; /* launches of k_simple<W, true> */
     char err[256];
@@ -662,26 +680,55 @@ static bool config_is_simple(const AgarConfig& c, const AgarLayout& L) {
            L.field_size < 128; /* the float32 candidate filter of k_simple's eat chain is analysed for coordinates below 128 (one player: 75) */
 }
 
+/* Every instantiation a plan can select.  A shape none of them serves is refused when it is planned. */
+static const struct { int W; bool full; int maxt; MainFn fn; } MAIN_KERNELS[] = {
+    {32, false, 512, k_main<32, false, 512>}, {32, true, 512, k_main<32, true, 512>},
+    {32, true, 768, k_main<32, true, 768>},   {32, true, 1024, k_main<32, true, 1024>},
+    {16, true, 512, k_main<16, true, 512>},   {8, true, 512, k_main<8, true, 512>},
+    {4, true, 512, k_main<4, true, 512>}};
+static const struct { int W; bool obsw; SimpleFn fn; } SIMPLE_KERNELS[] = {
+    {1, false, k_simple<1, false>}, {2, false, k_simple<2, false>},   {4, false, k_simple<4, false>},
+    {8, false, k_simple<8, false>}, {16, false, k_simple<16, false>}, {32, false, k_simple<32, false>},
+    {4, true, k_simple<4, true>},   {8, true, k_simple<8, true>}};
+static MainFn main_kernel(int W, bool full, int maxt) {
+    for (const auto& k : MAIN_KERNELS)
+        if (k.W == W && k.full == full && k.maxt == maxt) return k.fn;
+    return nullptr;
+}
+static SimpleFn simple_kernel(int W, bool obsw) {
+    for (const auto& k : SIMPLE_KERNELS)
+        if (k.W == W && k.obsw == obsw) return k.fn;
+    return nullptr;
+}
+
+/* cudaFuncSetAttribute is per kernel FUNCTION and process-wide, not per handle: two handles with different shared-memory
+ * needs (a training batch and an evaluation batch of the same config) must not lower each other's limit.  Every kernel a
+ * plan selects is therefore raised to the device's opt-in maximum (the launch itself still requests only what it needs, so
+ * occupancy is unaffected).  The planner calls this for each kernel it selects, off the launch path; setting twice is
+ * harmless. */
+template <typename Fn>
+static cudaError_t ensure_max_smem(Fn kernel, int device) {
+    int optin = 0;
+    cudaError_t err = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+    return err != cudaSuccess ? err : cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin);
+}
+
 /* launch shape of k_init / k_main for tile width W (bind_ctx's shared-memory layout); tiles == 0: one record does not fit */
-static LaunchShape plan_launch(const AgarEnv* e, int W) {
-    const size_t budget = 200 * 1024;
+static LaunchShape main_shape(const AgarEnv* e, bool full, int W) {
     const size_t per_tile = (size_t)e->P.scratch_bytes +
-                            (e->full ? (size_t)((e->P.hot_a + 15) / 16 * 16) + (size_t)((e->L.pellet_cap * 4 + 15) / 16 * 16)
-                                     : (size_t)e->P.rec_stride);
-    const int max_threads = (e->full && W == 32) ? 1024 : 512; /* k_main<32, true, 1024> exists for 32-lane tiles only */
-    int tiles = e->full ? max_threads / W : 128 / W; /* as many envs per CTA as fit: the barriers then align more warps */
-    while (tiles > 1 && per_tile * tiles > budget) tiles -= 1;
+                            (full ? (size_t)pel_cache_bytes(e->P.hot_a, e->L.pellet_cap) : (size_t)e->P.rec_stride);
+    const int max_threads = (full && W == 32) ? 1024 : 512; /* k_main<32, true, 1024> exists for 32-lane tiles only */
+    int tiles = full ? max_threads / W : 128 / W; /* as many envs per CTA as fit: the barriers then align more warps */
+    while (tiles > 1 && per_tile * tiles > SMEM_BUDGET) tiles -= 1;
     if (W == 32 && tiles > 4) tiles -= tiles % 4; /* warps spread evenly over the four schedulers of an SM */
-    if (per_tile * tiles > budget) return LaunchShape{W, 0, 0, 0};
-    if (e->full && W == 32 && tiles > 8) {
+    if (per_tile * tiles > SMEM_BUDGET) return LaunchShape{W, 0, 0, 0};
+    if (full && W == 32 && tiles > 8) {
         /* one CTA per SM and all CTAs take about as long: fewer envs per CTA can fill the last wave better.  Cost model
          * waves x envs-per-CTA (measured, config 3 at 16384 envs: 32 -> 1.01e8, 28 -> 1.05e8, 24 -> 0.97e8, 20 -> 0.89e8) */
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->device);
         long long best_cost = -1;
         int best = tiles;
         for (int t = tiles; t >= 8 && t >= tiles - 4; t -= 4) { /* one step: smaller CTAs lose lock-step efficiency */
-            long long ctas = (e->n_envs + t - 1) / t, waves = (ctas + sms - 1) / sms;
+            long long ctas = (e->n_envs + t - 1) / t, waves = (ctas + e->sms - 1) / e->sms;
             long long cost = waves * t;
             if (best_cost < 0 || cost < best_cost) best_cost = cost, best = t;
         }
@@ -690,118 +737,13 @@ static LaunchShape plan_launch(const AgarEnv* e, int W) {
     return LaunchShape{W, tiles, tiles * W, per_tile * tiles};
 }
 
-/* cudaFuncSetAttribute is per kernel FUNCTION and process-wide, not per handle: two handles with different shared-memory
- * needs (a training batch and an evaluation batch of the same config) must not lower each other's limit.  Every
- * instantiation is therefore raised ONCE per device to the device's opt-in maximum (the launch itself still requests only
- * what it needs, so occupancy is unaffected).  `done` is a per-instantiation static; setting twice is harmless. */
-template <typename K>
-static cudaError_t ensure_max_smem(K kernel, int device, unsigned char* done) {
-    if (device >= 0 && device < 64 && done[device]) return cudaSuccess;
-    int optin = 0;
-    cudaError_t err = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
-    if (err != cudaSuccess) return err;
-    err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin);
-    if (err == cudaSuccess && device >= 0 && device < 64) done[device] = 1;
-    return err;
-}
-
-template <int W, bool FULL, int MAXT>
-static cudaError_t launch_main_k(AgarEnv* e, const float* actions, float* obs, int n_frames, int n_dec, int flags,
-                                 uint32_t dec_base, cudaStream_t s) {
-    static unsigned char done[64];
-    cudaError_t err = ensure_max_smem(k_main<W, FULL, MAXT>, e->device, done);
-    if (err != cudaSuccess) return err;
-    int blocks = (e->n_envs + e->step.tiles - 1) / e->step.tiles;
-    k_main<W, FULL, MAXT><<<blocks, e->step.threads, e->step.smem, s>>>(e->P, e->state, actions, obs, n_frames, n_dec, flags, dec_base);
-    return cudaGetLastError();
-}
-template <int W, bool FULL>
-static cudaError_t launch_main_t(AgarEnv* e, const float* actions, float* obs, int n_frames, int n_dec, int flags,
-                                 uint32_t dec_base, cudaStream_t s) {
-    if (W == 32 && FULL && e->step.threads > 768) return launch_main_k<32, true, 1024>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
-    if (W == 32 && FULL && e->step.threads > 512) return launch_main_k<32, true, 768>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
-    return launch_main_k<W, FULL, 512>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
-}
-template <bool FULL>
-static cudaError_t launch_init_t(AgarEnv* e, const uint8_t* mask, int mode, cudaStream_t s) {
-    static unsigned char done[64];
-    cudaError_t err = ensure_max_smem(k_init<32, FULL>, e->device, done);
-    if (err != cudaSuccess) return err;
-    int blocks = (e->n_envs + e->init.tiles - 1) / e->init.tiles;
-    k_init<32, FULL><<<blocks, e->init.threads, e->init.smem, s>>>(e->P, e->state, mask, mode);
-    return cudaGetLastError();
-}
-
-static int launch_main(AgarEnv* e, const float* actions, float* obs, int n_frames, int n_dec, int flags, uint32_t dec_base,
-                       void* stream) {
-    AgarEnv* env = e;
-    CU(cudaSetDevice(e->device));
-    cudaError_t err;
-    if (e->simple) {
-        /* observer warps encode the observations a launch hands off before its frames (KF_OBS_BEFORE), when enough frames
-         * follow each one to hide the encoder; a trailing observation (KF_OBS_AFTER) stays with the physics warps */
-        const bool handoff = e->obs.threads && (flags & KF_OBS_BEFORE) && obs != nullptr && n_frames >= SIMPLE_OBS_MIN_FRAMES;
-        const SimplePlan& sp = handoff ? e->sp_obs : e->sp;
-        const LaunchShape& sh = handoff ? e->obs : e->step;
-        const int per = (sh.threads - 32 * sp.obs_warps) / sh.W; /* what k_simple derives from blockDim */
-        if (sh.threads % 32 || sh.threads > (handoff ? simple_max_threads(sh.W) : 256) || per < 1 || per != sh.tiles ||
-            per * sh.W % 32 || (sp.obs_warps && (!sp.grid_off || 32 * sp.obs_warps % SIMPLE_OBS_LANES)))
-            return fail(e, AGAR_E_INVALID, "inconsistent k_simple launch shape%s", "");
-        int blocks = (e->n_envs + per - 1) / per;
-#define LAUNCH_SIMPLE(WW, OB)                                                                                                 \
-    do {                                                                                                                      \
-        static unsigned char done_##WW##OB[64];                                                                               \
-        err = ensure_max_smem(k_simple<WW, OB>, e->device, done_##WW##OB);                                                    \
-        if (err == cudaSuccess) {                                                                                             \
-            k_simple<WW, OB><<<blocks, sh.threads, sh.smem, (cudaStream_t)stream>>>(e->P, sp, e->state, actions, obs,         \
-                                                                                    n_frames, n_dec, flags, dec_base);        \
-            err = cudaGetLastError();                                                                                         \
-        }                                                                                                                     \
-    } while (0)
-        if (handoff && sh.W == 4) LAUNCH_SIMPLE(4, true);
-        else if (handoff) LAUNCH_SIMPLE(8, true);
-        else if (sh.W == 1) LAUNCH_SIMPLE(1, false);
-        else if (sh.W == 2) LAUNCH_SIMPLE(2, false);
-        else if (sh.W == 4) LAUNCH_SIMPLE(4, false);
-        else if (sh.W == 8) LAUNCH_SIMPLE(8, false);
-        else if (sh.W == 16) LAUNCH_SIMPLE(16, false);
-        else LAUNCH_SIMPLE(32, false);
-#undef LAUNCH_SIMPLE
-        if (handoff && err == cudaSuccess) e->observer_launches += 1;
-    } else {
-        const int W = e->step.W;
-        cudaStream_t s = (cudaStream_t)stream;
-        err = !e->full ? launch_main_t<32, false>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
-              : W == 32 ? launch_main_t<32, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
-              : W == 16 ? launch_main_t<16, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
-              : W == 8  ? launch_main_t<8, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s)
-                        : launch_main_t<4, true>(e, actions, obs, n_frames, n_dec, flags, dec_base, s);
-    }
-    if (err != cudaSuccess) return fail(e, AGAR_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    e->launches += 1;
-    return AGAR_OK;
-}
-static int launch_init(AgarEnv* e, const uint8_t* mask, int mode, void* stream) {
-    AgarEnv* env = e;
-    CU(cudaSetDevice(e->device));
-    cudaError_t err = e->full ? launch_init_t<true>(e, mask, mode, (cudaStream_t)stream)
-                              : launch_init_t<false>(e, mask, mode, (cudaStream_t)stream);
-    if (err != cudaSuccess) return fail(e, AGAR_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    e->launches += 1;
-    return AGAR_OK;
-}
-
-/* resident CTAs per SM of k_simple<W, OBSW> at this CTA size and shared memory (0: cannot run, or the query failed) */
-template <int W, bool OBSW>
-static int simple_ctas_per_sm(int device, int threads, size_t smem) {
-    static unsigned char done[64];
-    int n = 0;
-    if (ensure_max_smem(k_simple<W, OBSW>, device, done) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_simple<W, OBSW>, threads, smem) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    return n;
+/* what k_simple derives from blockDim and its plan: whole warps, at most `max_threads` (its launch bound), `tiles` envs of
+ * whole warps, and observer warps only with a grid accumulator and whole observer tiles */
+static bool simple_shape_ok(const StepLaunch& r, int max_threads) {
+    const LaunchShape& sh = r.sh;
+    const int per = (sh.threads - 32 * r.sp.obs_warps) / sh.W;
+    return sh.threads % 32 == 0 && sh.threads <= max_threads && per >= 1 && per == sh.tiles && per * sh.W % 32 == 0 &&
+           (!r.sp.obs_warps || (r.sp.grid_off && 32 * r.sp.obs_warps % SIMPLE_OBS_LANES == 0));
 }
 
 /* Launch shape of k_simple with observer warps: one CTA per SM, ceil(envs / SMs) envs rounded up to whole physics warps
@@ -810,50 +752,53 @@ static int simple_ctas_per_sm(int device, int threads, size_t smem) {
  * and the encoder's work costs the same wherever it runs.  Wave-aware: past the physics-warp cap one CTA holds at most 28
  * (W = 8) or 32 (W = 4) envs and an SM holds one such CTA, while the inline shape fits two CTAs of 16 / 32 envs per SM —
  * the observers are used only where their launch needs no more waves than the inline one (4096 envs at W = 8: one wave
- * each; 4608: two against one). */
-static void plan_observers(AgarEnv* e) {
-    e->obs = LaunchShape{};
-    e->sp_obs = e->sp;
-    const int W = e->step.W;
-    if ((W != 4 && W != 8) || !e->sp.grid_off || e->L.pellet_cap > 64 * SIMPLE_OBS_LANES) return; /* SMask<SIMPLE_OBS_LANES> */
-    if (cudaSetDevice(e->device) != cudaSuccess) {
-        cudaGetLastError();
-        return;
-    }
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->device);
+ * each; 4608: two against one).  Leaves p->obs empty where they are not used. */
+static int plan_observers(AgarEnv* e, LaunchPlan* p) {
+    AgarEnv* env = e;
+    const StepLaunch& in = p->step;
+    const int W = in.sh.W, sms = e->sms;
+    const SimpleFn fn = simple_kernel(W, true);
+    if (!fn || !in.sp.grid_off || e->L.pellet_cap > 64 * SIMPLE_OBS_LANES) return AGAR_OK; /* SMask<SIMPLE_OBS_LANES> */
     const int per_warp = 32 / W;
     const int K = SIMPLE_OBS_WARPS;
     int warps = ((e->n_envs + sms - 1) / sms + per_warp - 1) / per_warp;
     if (warps > simple_max_threads(W) / 32 - K) warps = simple_max_threads(W) / 32 - K;
     const int per = warps * per_warp;
-    const size_t env_bytes = ((size_t)per * e->sp.strideB + 15) / 16 * 16;
+    const size_t env_bytes = ((size_t)per * in.sp.strideB + 15) / 16 * 16;
     const int snap_stride = (int)((sizeof(SimpleSnap) + (size_t)e->L.pellet_cap * 4 + 15) / 16 * 16);
     const size_t smem = env_bytes + 2 * (size_t)per * snap_stride;
-    if (smem > 200 * 1024) return;
+    if (smem > SMEM_BUDGET) return AGAR_OK;
     const int threads = (warps + K) * 32;
-    const int occ = W == 8 ? simple_ctas_per_sm<8, true>(e->device, threads, smem) : simple_ctas_per_sm<4, true>(e->device, threads, smem);
-    const int occ_in = W == 8 ? simple_ctas_per_sm<8, false>(e->device, e->step.threads, e->step.smem)
-                              : simple_ctas_per_sm<4, false>(e->device, e->step.threads, e->step.smem);
-    if (occ < 1 || occ_in < 1) return;
-    const long long per_in = e->step.tiles;
+    int occ = 0, occ_in = 0; /* resident CTAs per SM of each launch */
+    CU(ensure_max_smem(fn, e->device));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, threads, smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_in, in.simple, in.sh.threads, in.sh.smem));
+    if (occ < 1 || occ_in < 1) return AGAR_OK;
+    const long long per_in = in.sh.tiles;
     const long long waves = ((e->n_envs + per - 1) / per + (long long)sms * occ - 1) / ((long long)sms * occ);
     const long long waves_in = ((e->n_envs + per_in - 1) / per_in + (long long)sms * occ_in - 1) / ((long long)sms * occ_in);
-    if (waves > waves_in) return;
-    e->sp_obs.obs_warps = K;
-    e->sp_obs.snap_off = (int)env_bytes;
-    e->sp_obs.snap_stride = snap_stride;
-    e->obs = LaunchShape{W, per, threads, smem};
+    if (waves > waves_in) return AGAR_OK;
+    SimplePlan sp = in.sp;
+    sp.obs_warps = K;
+    sp.snap_off = (int)env_bytes;
+    sp.snap_stride = snap_stride;
+    p->obs = StepLaunch{nullptr, fn, LaunchShape{W, per, threads, smem}, sp};
+    return AGAR_OK;
 }
 
-/* Lanes per env.  Single-cell pellet-collection configs (config_is_simple) with G <= 16: 1, 2, 4, 8, 16, 32 select the
- * register-resident kernel (agar_simple.cuh, k_simple<W>); they run the general kernel (k_main<32, false>, 32 lanes only)
- * with G > 16 or under AGAR_GENERAL_KERNEL=1.  Every other config: 4, 8, 16, 32 (general kernel). */
-extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
-    if (!e) return AGAR_E_INVALID;
+/* The launch planner: every launch record of tile width W.  k_init runs 32-lane tiles; the step launch is k_simple<W, false>
+ * or k_main<W, FULL, MAXT>; k_simple at W = 4 / 8 may add the observer launch.  Raises each selected kernel's shared-memory
+ * limit, so that launches only read the records. */
+static int plan_launches(AgarEnv* e, int W, LaunchPlan* out) {
+    AgarEnv* env = e;
+    CU(cudaSetDevice(e->device));
+    const bool full = !config_is_simple(e->cfg, e->L);
+    LaunchPlan p = {};
+    p.init = InitLaunch{full ? k_init<32, true> : k_init<32, false>, main_shape(e, full, 32)};
+    if (!p.init.sh.tiles) return fail(e, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
+    CU(ensure_max_smem(p.init.fn, e->device));
     /* the register-resident kernel bins a pellet into at most two squares per axis: 2 * radius < fov / G needs G <= 16 */
-    if (!e->full && e->L.grid_squares <= 16 && (W == 1 || W == 2 || W == 4 || W == 8 || W == 16 || W == 32) &&
-        !getenv("AGAR_GENERAL_KERNEL")) {
+    if (!full && e->L.grid_squares <= 16 && simple_kernel(W, false) && !getenv("AGAR_GENERAL_KERNEL")) {
         const int tail_words = (int)((e->L.record_bytes - e->L.off_pellets) / 4);
         SimplePlan sp = {};
         sp.strideB = (tail_words | 1) * 4;
@@ -869,24 +814,69 @@ extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
             return fail(e, AGAR_E_UNSUPPORTED, "pellet pool too large for this tile width%s", "");
         int threads = 128; /* measured (round 2, exact libm arithmetic): four warps per CTA beat two at every batch size (4096 envs: 7.7e8 vs 7.0e8) */
         const size_t per_env = (size_t)sp.strideB;
-        while (threads > 32 && per_env * (threads / W) > 200 * 1024) threads -= 32;
-        if (per_env * (threads / W) > 200 * 1024)
+        while (threads > 32 && per_env * (threads / W) > SMEM_BUDGET) threads -= 32;
+        if (per_env * (threads / W) > SMEM_BUDGET)
             return fail(e, AGAR_E_NOMEM, "pellet pool + event ring of %s do not fit in shared memory at this tile width", "the envs of one CTA");
-        e->simple = 1;
-        e->sp = sp;
-        e->step = LaunchShape{W, threads / W, threads, per_env * (threads / W)};
-        plan_observers(e);
-        return AGAR_OK;
+        p.step = StepLaunch{nullptr, simple_kernel(W, false), LaunchShape{W, threads / W, threads, per_env * (threads / W)}, sp};
+        CU(ensure_max_smem(p.step.simple, e->device));
+        const int rc = plan_observers(e, &p);
+        if (rc != AGAR_OK) return rc;
+        if (!simple_shape_ok(p.step, 256) || (p.obs.simple && !simple_shape_ok(p.obs, simple_max_threads(W))))
+            return fail(e, AGAR_E_INVALID, "inconsistent k_simple launch shape%s", "");
+    } else {
+        if (!main_kernel(W, full, 512)) /* every (W, FULL) that exists has MAXT = 512 */
+            return fail(e, AGAR_E_INVALID, "unsupported tile width%s", "");
+        const LaunchShape s = main_shape(e, full, W);
+        if (!s.tiles) return fail(e, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
+        const int maxt = s.threads > 768 ? 1024 : s.threads > 512 ? 768 : 512; /* the smallest bound that admits the CTA */
+        p.step = StepLaunch{main_kernel(W, full, maxt), nullptr, s, SimplePlan{}};
+        if (!p.step.main) return fail(e, AGAR_E_INVALID, "no k_main instantiation for this launch shape%s", "");
+        CU(ensure_max_smem(p.step.main, e->device));
     }
-    bool ok = W == 32 || (e->full && (W == 4 || W == 8 || W == 16));
-    if (!ok) return fail(e, AGAR_E_INVALID, "unsupported tile width%s", "");
-    const LaunchShape s = plan_launch(e, W);
-    if (!s.tiles) return fail(e, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
-    e->simple = 0;
-    e->step = s;
+    *out = p;
     return AGAR_OK;
 }
-extern "C" int agar_get_tile_width(const AgarEnv* e) { return e ? e->step.W : 0; }
+
+/* Lanes per env.  Single-cell pellet-collection configs (config_is_simple) with G <= 16: 1, 2, 4, 8, 16, 32 select the
+ * register-resident kernel (agar_simple.cuh, k_simple<W>); they run the general kernel (k_main<32, false>, 32 lanes only)
+ * with G > 16 or under AGAR_GENERAL_KERNEL=1.  Every other config: 4, 8, 16, 32 (general kernel).  A refused tile width
+ * leaves the handle's plan as it was. */
+extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
+    if (!e) return AGAR_E_INVALID;
+    return plan_launches(e, W, &e->plan);
+}
+extern "C" int agar_get_tile_width(const AgarEnv* e) { return e ? e->plan.step.sh.W : 0; }
+
+static int launch_main(AgarEnv* e, const float* actions, float* obs, int n_frames, int n_dec, int flags, uint32_t dec_base,
+                       void* stream) {
+    AgarEnv* env = e;
+    CU(cudaSetDevice(e->device));
+    /* observer warps encode the observations a launch hands off before its frames (KF_OBS_BEFORE), when enough frames
+     * follow each one to hide the encoder; a trailing observation (KF_OBS_AFTER) stays with the physics warps */
+    const bool handoff = e->plan.obs.simple && (flags & KF_OBS_BEFORE) && obs != nullptr && n_frames >= SIMPLE_OBS_MIN_FRAMES;
+    const StepLaunch& r = handoff ? e->plan.obs : e->plan.step;
+    const int blocks = (e->n_envs + r.sh.tiles - 1) / r.sh.tiles;
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (r.simple)
+        r.simple<<<blocks, r.sh.threads, r.sh.smem, s>>>(e->P, r.sp, e->state, actions, obs, n_frames, n_dec, flags, dec_base);
+    else
+        r.main<<<blocks, r.sh.threads, r.sh.smem, s>>>(e->P, e->state, actions, obs, n_frames, n_dec, flags, dec_base);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(e, AGAR_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
+    e->launches += 1;
+    e->observer_launches += handoff;
+    return AGAR_OK;
+}
+static int launch_init(AgarEnv* e, const uint8_t* mask, int mode, void* stream) {
+    AgarEnv* env = e;
+    CU(cudaSetDevice(e->device));
+    const InitLaunch& r = e->plan.init;
+    r.fn<<<(e->n_envs + r.sh.tiles - 1) / r.sh.tiles, r.sh.threads, r.sh.smem, (cudaStream_t)stream>>>(e->P, e->state, mask, mode);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(e, AGAR_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
+    e->launches += 1;
+    return AGAR_OK;
+}
 
 extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64_t seed, uint64_t first_env_id, void* stream,
                            AgarEnv** out) {
@@ -899,13 +889,16 @@ extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev)
         return fail(nullptr, AGAR_E_CUDA, "no such CUDA device%s", "");
     CU(cudaSetDevice(device));
+    int sms = 0;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
     AgarEnv* e = (AgarEnv*)calloc(1, sizeof(AgarEnv));
     env = e;
     e->cfg = *cfg;
     e->L = L;
     e->n_envs = n_envs;
     e->device = device;
-    e->full = config_is_simple(*cfg, L) ? 0 : 1;
+    e->sms = sms;
+    const bool full = !config_is_simple(*cfg, L);
     DevParams& P = e->P;
     memset(&P, 0, sizeof P);
     P.cfg = *cfg;
@@ -914,21 +907,21 @@ extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64
     P.nb = (int)ceil((double)P.S / AG_BUCKET);
     P.n_envs = n_envs;
     P.rec_stride = (int)L.record_bytes + 8;
-    P.full = e->full;
+    P.full = full;
     static_assert(AGAR_MAX_CELLS == 16, "cap_shift assumes cell_cap in {1, 16} (agar_layout.h)");
     P.cap_shift = L.cell_cap == AGAR_MAX_CELLS ? 4 : 0;
     P.g_magic = L.grid_squares > 1 ? (uint32_t)((1ull << 32) / (unsigned)L.grid_squares) + 1u : 0u;
-    int vel_bytes = e->full ? L.n_players * L.cell_cap * 2 * 8 : 0;
-    int obs_bytes = obs_scratch_bytes(L.grid_squares, e->full != 0);
+    int vel_bytes = full ? L.n_players * L.cell_cap * 2 * 8 : 0;
+    int obs_bytes = obs_scratch_bytes(L.grid_squares, full);
     /* the pellet index (agar_dev.cuh) lives in the same scratch: it is built after the players have moved (velocities dead)
      * and before the next bot phase (observation tables dead); pools of <= 8 chunks are scanned directly */
-    P.pel_index = e->full && L.pellet_cap > 256;
+    P.pel_index = full && L.pellet_cap > 256;
     const int gb_idx = (P.S + 9) / 10; /* AG_IDX_CELL */
     int idx_bytes = P.pel_index ? ((gb_idx * gb_idx + 3) & ~1) * 2 + L.pellet_cap * 2 + 128 + 64 + 16 : 0; /* counters, entries, sort list, ex-blob list */
     if (idx_bytes > vel_bytes) vel_bytes = idx_bytes;
     P.scratch_bytes = ((vel_bytes > obs_bytes ? vel_bytes : obs_bytes) + 15) / 16 * 16 + 8;
     P.live_off = P.scratch_bytes; /* live-cell list: uint16 per cell slot, after the observation / velocity scratch */
-    if (e->full) P.scratch_bytes += (L.n_players * L.cell_cap * 2 + 15) / 16 * 16;
+    if (full) P.scratch_bytes += (L.n_players * L.cell_cap * 2 + 15) / 16 * 16;
     /* Where a record lives during a launch (bind_ctx).  The single-cell general kernel stages the whole record in shared
      * memory.  Multi-agent configs keep the record in HBM / L2 and cache on chip what every scan and lane-0 step reads:
      * header + players + cells + viruses (hot_a = off_blobs) + pellet pool if at least 12 envs per CTA still fit, else the
@@ -936,9 +929,9 @@ extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64
      * config 3 6.3e7 / 7.3e7 / 7.7e7 env-steps/s for whole record / pool / hot sections; config 4 0.75e6 (whole record, 3
      * warps per SM) / 3.3e6 (pool) / 1.6e6 (hot sections); with 32 envs per CTA (profiles/r01_sweep.txt) config 3 does
      * 9.1e7 (pool) / 9.6e7 (hot sections). */
-    if (e->full) {
-        size_t hot = (size_t)((L.off_blobs + 15) / 16 * 16) + (size_t)((L.pellet_cap * 4 + 15) / 16 * 16) + P.scratch_bytes;
-        P.hot_a = hot * 12 <= 200 * 1024 ? (int)L.off_blobs : 0;
+    if (full) {
+        const size_t hot = (size_t)pel_cache_bytes((int)L.off_blobs, L.pellet_cap) + P.scratch_bytes;
+        P.hot_a = hot * 12 <= SMEM_BUDGET ? (int)L.off_blobs : 0;
     }
     double speed_modifier = 1.0 / 30;
     P.move_speed = 90 * speed_modifier;
@@ -968,12 +961,7 @@ extern "C" int agar_create(const AgarConfig* cfg, int n_envs, int device, uint64
     CU(cudaMemsetAsync(e->d_rec_err, 0, sizeof(unsigned int), (cudaStream_t)stream));
     CU(cudaStreamSynchronize((cudaStream_t)stream)); /* tab is a stack buffer */
     P.deg_tab = e->deg_tab;
-    e->init = plan_launch(e, 32); /* k_init always runs with 32-lane tiles */
-    if (!e->init.tiles) {
-        cudaFree(e->state), cudaFree(e->deg_tab), cudaFree(e->d_rec_err), free(e);
-        return fail(nullptr, AGAR_E_NOMEM, "env record does not fit in shared memory%s", "");
-    }
-    int W = e->full ? 32 : (n_envs <= 8192 ? 8 : (n_envs <= 32768 ? 2 : 1)); /* tools/sweep.py, profiles/r01_sweep.txt */
+    int W = full ? 32 : (n_envs <= 8192 ? 8 : (n_envs <= 32768 ? 2 : 1)); /* tools/sweep.py, profiles/r01_sweep.txt */
     if (agar_set_tile_width(e, W) != AGAR_OK && agar_set_tile_width(e, 8) != AGAR_OK && agar_set_tile_width(e, 32) != AGAR_OK) {
         snprintf(g_create_err, sizeof g_create_err, "%s", e->err);
         cudaFree(e->state), cudaFree(e->deg_tab), cudaFree(e->d_rec_err), free(e);

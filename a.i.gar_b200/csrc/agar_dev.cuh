@@ -1064,6 +1064,7 @@ DEVN void player_virus_overlap_seq(Ctx<W>& c, const DevParams& P) {
 #define AG_IDX_CELL 10
 DEV int pel_index_gb(const DevParams& P) { return (P.S + AG_IDX_CELL - 1) / AG_IDX_CELL; }
 DEV int pel_index_cnt_len(const DevParams& P) { return (pel_index_gb(P) * pel_index_gb(P) + 2 + 1) & ~1; }
+/* pel_index is only ever set with full; without the redundant read ptxas gives k_main<32, true, 512> two more registers */
 DEV bool pel_index_enabled(const DevParams& P) { return P.full && P.pel_index; }
 template <int W>
 DEV void build_pellet_index(Ctx<W>& c, const DevParams& P) {
