@@ -212,6 +212,116 @@ k_main(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const f
 }
 
 
+/* agar_rollout's launch: k_main's loop, with obs and actions holding one slice per decision and each decision's turn values
+ * and random actions stored into P.traj; a launch without frames still observes n_dec times.  A separate kernel rather than
+ * a recording flag on a body shared with k_main: compiled through a shared inline body, k_main's code changed (same
+ * registers, different schedule) and configs[3] measured 1.2 % slower on a B200. */
+template <int W, bool FULL, int MAXT>
+__global__ void __launch_bounds__(MAXT, (FULL || MAXT > 512) ? 1 : 2)
+k_main_rec(const __grid_constant__ DevParams P, uint8_t* __restrict__ state, const float* __restrict__ actions,
+           float* __restrict__ obs, int n_frames, int n_dec, int flags, uint32_t dec_base) {
+    const int tiles = blockDim.x / W;
+    const int env0 = blockIdx.x * tiles;
+    const int n_here = min(tiles, P.n_envs - env0);
+    if (FULL) pel_cache_copy(P, state, env0, n_here, tiles, true);
+    else stage_in(P, state, env0, n_here, false);
+    const int tile_id = threadIdx.x / W;
+    const bool active = tile_id < n_here;
+    {
+        Ctx<W> c(cg::tiled_partition<W>(cg::this_thread_block()));
+        const int env = env0 + (active ? tile_id : 0);
+        bind_ctx<W, FULL>(c, P, active ? tile_id : 0, tiles, env, state);
+        const int A = P.L.n_agents, K = P.L.n_players, SL = P.L.state_len;
+        float* obs_env = obs ? obs + (size_t)env * A * SL : nullptr;
+        /* One loop with ONE call site per helper: the multi-agent frame is ~22 k SASS instructions and instruction
+         * fetch is its top stall (profiles/r01_k_main_cfg3_*), so nothing big may be inlined twice.  Iteration `it` is
+         * frame f of decision d; the trailing observation (KF_OBS_AFTER) is one extra iteration without a frame.
+         * FULL: CTA barriers at frame start and before the field update keep all warps of the CTA in the same code
+         * region, so the instruction cache serves them together (idle tiles of a partly filled CTA only hit the
+         * barriers; measured 2.5x, DESIGN §4). */
+        const int fpd = n_frames > 0 ? n_frames : 1;         /* iterations per decision: without frames, n_dec observations */
+        const size_t dec_obs = (size_t)P.n_envs * A * SL;    /* floats between two decisions' observation slices */
+        const size_t dec_act = (size_t)P.n_envs * A * 4;     /* ... and action slices */
+        const int total = n_dec * fpd;
+        for (int it = 0; it <= total; ++it) {
+            const bool last = it == total;
+            if (last && !(flags & KF_OBS_AFTER)) break;
+#ifdef AGAR_PHASE_CLOCKS
+            c.clk_t = clock64(), c.clk_env = env;
+#endif
+            if (FULL) __syncthreads();
+            CLK_MARK(0); /* (ptxas hoists this clock read above the barrier: the wait lands in the NEXT slot, the fov pass) */
+            const int f = it % fpd, d = it / fpd;
+            const bool idle = last || n_frames == 0; /* turns only, no frame: an agar_observe */
+            const bool emit = last || (f == 0 && (flags & KF_OBS_BEFORE)); /* observations leave the kernel here */
+            if (active && !idle && c.lane == 0) c.h->n_events = 0;
+            if (FULL && K > 1 && active && !idle) { /* every alive player's turn below would compute its own, on lane 0 */
+                update_all_fovs(c, P);
+                c.fov_done = true;
+                CLK_MARK(8); /* fov pass */
+                if (K * P.L.cell_cap > W) build_live_cells(c, P); /* one iteration covers all slots otherwise */
+                CLK_MARK(11); /* live-cell list */
+            }
+            for (int k = 0; k < K; ++k) {
+                if (active) {
+                    if (!FULL || P.cfg.bot_type[k] == AGAR_BOT_NN) {
+                        nn_turn_begin<W, FULL>(c, P, k, (emit && obs_env) ? obs_env + (size_t)k * SL + d * dec_obs : nullptr);
+                        if (emit && c.lane == 0) { /* NN bots are the first A player slots */
+                            const AgarBot& B = c.pl[k].bot;
+                            const size_t i = ((size_t)d * P.n_envs + env) * A + k;
+                            record_turn(P, i, B.last_reward, B.exp_done, B.exp_valid, B.need_action);
+                            if (!last && (flags & KF_RANDOM_ACTIONS)) record_action(P, i, dec_base + (uint32_t)d, c.env_id, k);
+                        }
+                        if (idle) continue;
+                        if (c.lane == 0) {
+                            float act[4] = {0.f, 0.f, 0.f, 0.f};
+                            if (c.pl[k].bot.need_action) {
+                                if (flags & KF_RANDOM_ACTIONS) /* random-action driver (SURVEY §8d config 2) */
+                                    random_action(P, dec_base + (uint32_t)d, c.env_id, (uint32_t)k, act);
+                                else {
+                                    const float* ap = actions + ((size_t)env * A + k) * 4 + d * dec_act;
+                                    for (int i = 0; i < 4; ++i) act[i] = ap[i];
+                                }
+                            }
+                            nn_turn_end(c, P, k, act);
+                        }
+                        c.t.sync();
+                    } else if (FULL && !idle) {
+                        CLK_MARK(1); /* NN turns so far */
+                        scripted_turn(c, P, k);
+                        CLK_MARK(7); /* scripted (greedy / random) turns */
+                    }
+                }
+            }
+            if (last) break;
+            if (idle) continue; /* no frames: the next decision observes again */
+            CLK_MARK(1); /* bot turns */
+            c.fov_done = false, c.n_live = -1;
+            for (int ph = 0; ph < AGAR_FIELD_PHASES; ++ph) {
+                if (FULL && ph == 0) __syncthreads();
+                if (ph == 0) CLK_MARK(2); /* wait at the field barrier */
+                if (active) field_update_phase<W, FULL>(c, P, ph);
+                CLK_MARK(3 + ph); /* 3: viruses / blobs / players  4: merge, virus overlaps  5: pellets  6: blobs, player-player, spawn */
+            }
+            if (active) {
+                if (c.lane == 0) c.h->frame += 1;
+                c.t.sync();
+            }
+            CLK_MARK(12); /* frame tail */
+        }
+        if (active && c.lane == 0 && (P.turn_reward || P.turn_done))
+            for (int a = 0; a < A; ++a) {
+                if (P.turn_reward) P.turn_reward[(size_t)env * A + a] = (float)c.pl[a].bot.last_reward;
+                if (P.turn_done) P.turn_done[(size_t)env * A + a] = (uint8_t)c.pl[a].bot.exp_done;
+            }
+    }
+    if (FULL) {
+        __syncthreads();
+        pel_cache_copy(P, state, env0, n_here, tiles, false);
+    } else
+        stage_out(P, state, env0, n_here);
+    export_tail(P, obs, env0, n_here);
+}
 /* ------------------------------------------------------------------ register-resident kernel (agar_simple.cuh) */
 struct SimplePlan {
     int strideB; /* bytes between the staged [pellets .. end of record] regions of consecutive envs */
@@ -249,12 +359,13 @@ DEV void named_bar_sync(int n) { asm volatile("bar.sync %0, %1;" ::"n"(ID), "r"(
 template <int ID>
 DEV void named_bar_arrive(int n) { asm volatile("bar.arrive %0, %1;" ::"n"(ID), "r"(n) : "memory"); }
 
-/* one lane per env is throughput-bound: cap registers at 128 for 8 CTAs / SM (measured +10..50 % at >= 64k envs);
- * wider tiles are latency-bound at small env counts and prefer the uncapped allocation (measured) */
-template <int W, bool OBSW> /* OBSW: the observer-warp launch (plan_observers); false: the inline encoder, CTA barrier per frame */
-__global__ void __launch_bounds__(OBSW ? simple_max_threads(W) : 256, W == 1 ? 2 : 1)
-k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __restrict__ state, const float* __restrict__ actions,
-         float* __restrict__ obs, int n_frames, int n_dec, int flags, uint32_t dec_base) {
+/* The body of k_simple and k_simple_rec.  OBSW: the observer-warp launch (plan_observers); false: the inline encoder, CTA
+ * barrier per frame.  REC (agar_rollout): obs and actions hold one slice per decision, and each decision's turn values and
+ * random action are stored into P.traj. */
+template <int W, bool OBSW, bool REC>
+__device__ __forceinline__ void simple_body(const DevParams& P, const SimplePlan& SP, uint8_t* __restrict__ state,
+                                            const float* __restrict__ actions, float* __restrict__ obs, int n_frames, int n_dec,
+                                            int flags, uint32_t dec_base) {
     const int phys_threads = blockDim.x - 32 * SP.obs_warps; /* the one place the barrier counts come from */
     const int per = phys_threads / W; /* envs per CTA */
     const int env0 = blockIdx.x * per;
@@ -272,6 +383,8 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
     }
     __syncthreads();
     auto snap = [&](int buf, int e) { return g_smem + SP.snap_off + (size_t)(buf * per + e) * SP.snap_stride; };
+    const size_t dec_obs = REC ? (size_t)P.n_envs * P.L.state_len : 0; /* floats between two decisions' rows (one agent) */
+    const size_t dec_act = REC ? (size_t)P.n_envs * 4 : 0;             /* ... and action rows */
     if (OBSW && (int)threadIdx.x >= phys_threads) { /* observer warps */
         constexpr int WO = SIMPLE_OBS_LANES;
         const int ot = ((int)threadIdx.x - phys_threads) / WO, osub = threadIdx.x % WO, n_ot = 32 * SP.obs_warps / WO;
@@ -290,7 +403,7 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
                 q.pel = (uint32_t*)(sn + 1);
                 q.grid = (uint32_t*)(g_smem + (size_t)e * SP.strideB + SP.grid_off);
                 const bool out = base + ot < per && sn->out != 0;
-                s_encode<WO>(r, q, P, out, out ? obs + (size_t)(env0 + e) * P.L.state_len : nullptr, osub);
+                s_encode<WO>(r, q, P, out, out ? obs + (size_t)(env0 + e) * P.L.state_len + d * dec_obs : nullptr, osub);
             }
             if (d + 2 < n_dec) {
                 if (buf) named_bar_arrive<SB_EMPTY + 1>(blockDim.x);
@@ -315,6 +428,14 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
         SReg r;
         s_load(r, q);
         float* row = (obs != nullptr && valid) ? obs + (size_t)env * P.L.state_len : nullptr;
+        auto row_of = [&](int d) { return REC && row ? row + d * dec_obs : row; };
+        auto record = [&](int d, bool action) { /* agar_rollout: decision d's turn values (and random action) */
+            if (REC && valid && sub == 0) {
+                const size_t i = (size_t)d * P.n_envs + env;
+                record_turn(P, i, r.last_reward, r.exp_done, r.exp_valid, r.need_action);
+                if (action && (flags & KF_RANDOM_ACTIONS)) record_action(P, i, dec_base + (uint32_t)d, env_id, 0u);
+            }
+        };
         /* one barrier per frame: the warps of a CTA walk the ~5000-instruction frame body together (measured 1.9x at 1M envs
          * and 2.3x at 4096); the physics warps only, observers keep their own pace */
         auto frame_bar = [&]() {
@@ -338,11 +459,13 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
                     h->fov_x = r.fov_x, h->fov_y = r.fov_y, h->fov_size = r.fov_size, h->mass = r.mass;
                     h->out = d_o != 0 && row != nullptr;
                 }
+                record(d, true);
                 if (buf) named_bar_arrive<SB_FULL + 1>(blockDim.x);
                 else named_bar_arrive<SB_FULL>(blockDim.x);
             } else if (flags & KF_OBS_BEFORE) {
                 int d_o = s_turn_begin(r, P);
-                s_observe<W>(r, q, P, d_o != 0, row, sub);
+                record(d, true);
+                s_observe<W>(r, q, P, d_o != 0, row_of(d), sub);
             }
             for (int f = 0; f < n_frames; ++f) {
                 frame_bar();
@@ -351,12 +474,10 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
                 s_observe<W>(r, q, P, d_o != 0, nullptr, sub);
                 float act[4] = {0.f, 0.f, 0.f, 0.f};
                 if (r.need_action) {
-                    if (flags & KF_RANDOM_ACTIONS) {
-                        uint32_t w[4];
-                        philox(dec_base + (uint32_t)d, 7u, env_id, 0u, (uint32_t)P.seed, (uint32_t)(P.seed >> 32), w);
-                        for (int i = 0; i < 4; ++i) act[i] = (float)(w[i] >> 8) * (1.0f / 16777216.0f);
-                    } else {
-                        const float* ap = actions + (size_t)env * 4;
+                    if (flags & KF_RANDOM_ACTIONS)
+                        random_action(P, dec_base + (uint32_t)d, env_id, 0u, act);
+                    else {
+                        const float* ap = actions + (size_t)env * 4 + d * dec_act;
                         for (int i = 0; i < 4; ++i) act[i] = ap[i];
                     }
                 }
@@ -368,7 +489,8 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
         if (flags & KF_OBS_AFTER) {
             if (OBSW) __syncthreads(); /* the observers have stored every handed-off row and left the grid accumulators */
             int d_o = s_turn_begin(r, P);
-            s_observe<W>(r, q, P, d_o != 0, row, sub);
+            record(n_dec, false);
+            s_observe<W>(r, q, P, d_o != 0, row_of(n_dec), sub);
         }
         if (valid && sub == 0) {
             s_store(r, q);
@@ -383,6 +505,21 @@ k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __re
         dst[w] = *(const uint32_t*)(g_smem + (size_t)e * SP.strideB + w * 4);
     }
     export_tail(P, obs, env0, n_here);
+}
+/* one lane per env is throughput-bound: cap registers at 128 for 8 CTAs / SM (measured +10..50 % at >= 64k envs);
+ * wider tiles are latency-bound at small env counts and prefer the uncapped allocation (measured) */
+template <int W, bool OBSW>
+__global__ void __launch_bounds__(OBSW ? simple_max_threads(W) : 256, W == 1 ? 2 : 1)
+k_simple(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __restrict__ state, const float* __restrict__ actions,
+         float* __restrict__ obs, int n_frames, int n_dec, int flags, uint32_t dec_base) {
+    simple_body<W, OBSW, false>(P, SP, state, actions, obs, n_frames, n_dec, flags, dec_base);
+}
+/* agar_rollout's launch: k_simple plus the per-decision slices, as separate instantiations so that k_simple keeps its code */
+template <int W, bool OBSW>
+__global__ void __launch_bounds__(OBSW ? simple_max_threads(W) : 256, W == 1 ? 2 : 1)
+k_simple_rec(const __grid_constant__ DevParams P, const SimplePlan SP, uint8_t* __restrict__ state,
+             const float* __restrict__ actions, float* __restrict__ obs, int n_frames, int n_dec, int flags, uint32_t dec_base) {
+    simple_body<W, OBSW, true>(P, SP, state, actions, obs, n_frames, n_dec, flags, dec_base);
 }
 
 /* mode 0: Model(...) + createBot*K + Model.initialize (model.py:51,154-162,90-94; field.py:57-67)
@@ -629,6 +766,7 @@ struct LaunchPlan {
     InitLaunch init;
     StepLaunch step; /* every step launch that hands no observation off */
     StepLaunch obs;  /* k_simple<W, true>: the launches that hand decision observations off to observer warps */
+    StepLaunch step_rec, obs_rec; /* agar_rollout: the same shapes with the recording instantiations (k_*_rec) */
 };
 struct AgarEnv {
     AgarConfig cfg;
@@ -680,24 +818,29 @@ static bool config_is_simple(const AgarConfig& c, const AgarLayout& L) {
            L.field_size < 128; /* the float32 candidate filter of k_simple's eat chain is analysed for coordinates below 128 (one player: 75) */
 }
 
-/* Every instantiation a plan can select.  A shape none of them serves is refused when it is planned. */
-static const struct { int W; bool full; int maxt; MainFn fn; } MAIN_KERNELS[] = {
-    {32, false, 512, k_main<32, false, 512>}, {32, true, 512, k_main<32, true, 512>},
-    {32, true, 768, k_main<32, true, 768>},   {32, true, 1024, k_main<32, true, 1024>},
-    {16, true, 512, k_main<16, true, 512>},   {8, true, 512, k_main<8, true, 512>},
-    {4, true, 512, k_main<4, true, 512>}};
-static const struct { int W; bool obsw; SimpleFn fn; } SIMPLE_KERNELS[] = {
-    {1, false, k_simple<1, false>}, {2, false, k_simple<2, false>},   {4, false, k_simple<4, false>},
-    {8, false, k_simple<8, false>}, {16, false, k_simple<16, false>}, {32, false, k_simple<32, false>},
-    {4, true, k_simple<4, true>},   {8, true, k_simple<8, true>}};
-static MainFn main_kernel(int W, bool full, int maxt) {
+/* Every instantiation a plan can select; rec: the agar_rollout instantiation of the same shape.  A shape none of them serves
+ * is refused when it is planned. */
+static const struct { int W; bool full; int maxt; MainFn fn, rec; } MAIN_KERNELS[] = {
+    {32, false, 512, k_main<32, false, 512>, k_main_rec<32, false, 512>},
+    {32, true, 512, k_main<32, true, 512>, k_main_rec<32, true, 512>},
+    {32, true, 768, k_main<32, true, 768>, k_main_rec<32, true, 768>},
+    {32, true, 1024, k_main<32, true, 1024>, k_main_rec<32, true, 1024>},
+    {16, true, 512, k_main<16, true, 512>, k_main_rec<16, true, 512>},
+    {8, true, 512, k_main<8, true, 512>, k_main_rec<8, true, 512>},
+    {4, true, 512, k_main<4, true, 512>, k_main_rec<4, true, 512>}};
+static const struct { int W; bool obsw; SimpleFn fn, rec; } SIMPLE_KERNELS[] = {
+    {1, false, k_simple<1, false>, k_simple_rec<1, false>},    {2, false, k_simple<2, false>, k_simple_rec<2, false>},
+    {4, false, k_simple<4, false>, k_simple_rec<4, false>},    {8, false, k_simple<8, false>, k_simple_rec<8, false>},
+    {16, false, k_simple<16, false>, k_simple_rec<16, false>}, {32, false, k_simple<32, false>, k_simple_rec<32, false>},
+    {4, true, k_simple<4, true>, k_simple_rec<4, true>},       {8, true, k_simple<8, true>, k_simple_rec<8, true>}};
+static MainFn main_kernel(int W, bool full, int maxt, bool rec = false) {
     for (const auto& k : MAIN_KERNELS)
-        if (k.W == W && k.full == full && k.maxt == maxt) return k.fn;
+        if (k.W == W && k.full == full && k.maxt == maxt) return rec ? k.rec : k.fn;
     return nullptr;
 }
-static SimpleFn simple_kernel(int W, bool obsw) {
+static SimpleFn simple_kernel(int W, bool obsw, bool rec = false) {
     for (const auto& k : SIMPLE_KERNELS)
-        if (k.W == W && k.obsw == obsw) return k.fn;
+        if (k.W == W && k.obsw == obsw) return rec ? k.rec : k.fn;
     return nullptr;
 }
 
@@ -823,6 +966,15 @@ static int plan_launches(AgarEnv* e, int W, LaunchPlan* out) {
         if (rc != AGAR_OK) return rc;
         if (!simple_shape_ok(p.step, 256) || (p.obs.simple && !simple_shape_ok(p.obs, simple_max_threads(W))))
             return fail(e, AGAR_E_INVALID, "inconsistent k_simple launch shape%s", "");
+        /* agar_rollout launches the recording instantiations at the same shapes, under the same hand-off rule */
+        p.step_rec = p.step;
+        p.step_rec.simple = simple_kernel(W, false, true);
+        CU(ensure_max_smem(p.step_rec.simple, e->device));
+        if (p.obs.simple) {
+            p.obs_rec = p.obs;
+            p.obs_rec.simple = simple_kernel(W, true, true);
+            CU(ensure_max_smem(p.obs_rec.simple, e->device));
+        }
     } else {
         if (!main_kernel(W, full, 512)) /* every (W, FULL) that exists has MAXT = 512 */
             return fail(e, AGAR_E_INVALID, "unsupported tile width%s", "");
@@ -832,6 +984,9 @@ static int plan_launches(AgarEnv* e, int W, LaunchPlan* out) {
         p.step = StepLaunch{main_kernel(W, full, maxt), nullptr, s, SimplePlan{}};
         if (!p.step.main) return fail(e, AGAR_E_INVALID, "no k_main instantiation for this launch shape%s", "");
         CU(ensure_max_smem(p.step.main, e->device));
+        p.step_rec = p.step;
+        p.step_rec.main = main_kernel(W, full, maxt, true);
+        CU(ensure_max_smem(p.step_rec.main, e->device));
     }
     *out = p;
     return AGAR_OK;
@@ -848,13 +1003,13 @@ extern "C" int agar_set_tile_width(AgarEnv* e, int W) {
 extern "C" int agar_get_tile_width(const AgarEnv* e) { return e ? e->plan.step.sh.W : 0; }
 
 static int launch_main(AgarEnv* e, const float* actions, float* obs, int n_frames, int n_dec, int flags, uint32_t dec_base,
-                       void* stream) {
+                       void* stream, bool rec = false) {
     AgarEnv* env = e;
     CU(cudaSetDevice(e->device));
     /* observer warps encode the observations a launch hands off before its frames (KF_OBS_BEFORE), when enough frames
      * follow each one to hide the encoder; a trailing observation (KF_OBS_AFTER) stays with the physics warps */
     const bool handoff = e->plan.obs.simple && (flags & KF_OBS_BEFORE) && obs != nullptr && n_frames >= SIMPLE_OBS_MIN_FRAMES;
-    const StepLaunch& r = handoff ? e->plan.obs : e->plan.step;
+    const StepLaunch& r = handoff ? (rec ? e->plan.obs_rec : e->plan.obs) : (rec ? e->plan.step_rec : e->plan.step);
     const int blocks = (e->n_envs + r.sh.tiles - 1) / r.sh.tiles;
     const cudaStream_t s = (cudaStream_t)stream;
     if (r.simple)
@@ -1029,6 +1184,22 @@ extern "C" int agar_rollout_random(AgarEnv* e, int n_decisions, int n_frames, ui
                                    void* stream) {
     if (!e || n_decisions < 0 || n_frames < 0) return AGAR_E_INVALID;
     return launch_main(e, nullptr, obs_dev, n_frames, n_decisions, KF_OBS_BEFORE | KF_RANDOM_ACTIONS, decision_base, stream);
+}
+/* n_decisions x (observe -> act -> n_frames frames) + a trailing observation, each decision recorded into `out` (agar_b200.h) */
+extern "C" int agar_rollout(AgarEnv* e, int n_decisions, int n_frames, uint32_t decision_base, const float* actions_dev,
+                            const AgarTrajectory* out, void* stream) {
+    if (!e) return AGAR_E_INVALID;
+    if (!out) return fail(e, AGAR_E_INVALID, "agar_rollout: out is NULL%s", "");
+    if (n_decisions < 0 || n_frames < 0) return fail(e, AGAR_E_INVALID, "agar_rollout: negative n_decisions or n_frames%s", "");
+    if (out->action && actions_dev)
+        return fail(e, AGAR_E_INVALID, "agar_rollout: out->action records the random driver; it must be NULL with caller actions%s", "");
+    if ((uintptr_t)out->obs % 4 || (uintptr_t)actions_dev % 4)
+        return fail(e, AGAR_E_INVALID, "agar_rollout: out->obs and actions_dev must be 4-byte aligned%s", "");
+    e->P.traj = *out;
+    const int flags = KF_OBS_BEFORE | KF_OBS_AFTER | (actions_dev ? 0 : KF_RANDOM_ACTIONS);
+    const int rc = launch_main(e, actions_dev, out->obs, n_frames, n_decisions, flags, decision_base, stream, true);
+    e->P.traj = AgarTrajectory{};
+    return rc;
 }
 extern "C" int agar_get(AgarEnv* e, AgarField which, void* out_dev, void* stream) {
     AgarEnv* env = e;

@@ -59,6 +59,9 @@ struct DevParams {
     unsigned int* export_count;  /* device counter of CTAs that have exported                                          */
     volatile uint32_t* host_flag;
     uint32_t flag_value;
+    /* agar_rollout: the per-decision outputs the recording kernels (k_main_rec, k_simple_rec) store; set for that launch
+     * only.  traj.obs is not read here: the row buffer travels as the kernel's obs argument. */
+    AgarTrajectory traj;
 };
 
 /* flags of k_main */
@@ -266,6 +269,27 @@ DEV void philox(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
         k1 += 0xBB67AE85u;
     }
     out[0] = c0, out[1] = c1, out[2] = c2, out[3] = c3;
+}
+/* the random-action driver's action of decision `dec` for agent k: 4 uniforms of Philox(dec, 7, env id, k) */
+DEV void random_action(const DevParams& P, uint32_t dec, uint32_t env_id, uint32_t k, float act[4]) {
+    uint32_t w[4];
+    philox(dec, 7u, env_id, k, (uint32_t)P.seed, (uint32_t)(P.seed >> 32), w);
+    for (int i = 0; i < 4; ++i) act[i] = (float)(w[i] >> 8) * (1.0f / 16777216.0f);
+}
+/* agar_rollout: what agar_get(REWARD / DONE / VALID / NEED_ACTION) would return now, into trajectory slot i */
+DEV void record_turn(const DevParams& P, size_t i, double last_reward, int exp_done, int exp_valid, int need_action) {
+    const AgarTrajectory& T = P.traj;
+    if (T.reward) T.reward[i] = (float)last_reward;
+    if (T.done) T.done[i] = (uint8_t)exp_done;
+    if (T.valid) T.valid[i] = (uint8_t)exp_valid;
+    if (T.need_action) T.need_action[i] = (uint8_t)need_action;
+}
+/* agar_rollout with the random driver: decision d's action of agent k into trajectory slot i, whether or not k acts */
+DEV void record_action(const DevParams& P, size_t i, uint32_t dec, uint32_t env_id, uint32_t k) {
+    if (!P.traj.action) return;
+    float a[4];
+    random_action(P, dec, env_id, k, a);
+    for (int j = 0; j < 4; ++j) P.traj.action[i * 4 + j] = a[j];
 }
 /* the draw_* functions are called by lane 0 only (they advance the serial in the record) */
 template <int W>

@@ -6,6 +6,7 @@ missing or no CUDA device is present every constructor raises."""
 import ctypes
 import hashlib
 import os
+from collections import namedtuple
 
 import numpy as np
 
@@ -122,6 +123,46 @@ def check_checkpoint(ck, cfg, layout, n_envs, seed, first_env_id):
     for name, mine in (("n_envs", n_envs), ("seed", seed), ("first_env_id", first_env_id)):
         if int(ck[name]) != int(mine):
             raise CheckpointError("checkpoint %s is %d, the handle's is %d" % (name, int(ck[name]), int(mine)))
+
+
+TRAJECTORY_FIELDS = ("obs", "action", "reward", "done", "valid", "need_action")
+
+
+class _CTrajectory(ctypes.Structure):
+    """AgarTrajectory of include/agar_b200.h: one nullable device pointer per field"""
+    _fields_ = [(f, ctypes.c_void_p) for f in TRAJECTORY_FIELDS]
+
+
+class Trajectory(namedtuple("Trajectory", TRAJECTORY_FIELDS + ("n_frames", "frame_skip"))):
+    """A recorded rollout (AgarBatch.rollout): device tensors, A = max(n_agents, 1), D decisions.
+
+    obs [D+1, E, A, L] float32, action [D, E, A, 4] float32, reward [D+1, E, A] float32, done / valid / need_action
+    [D+1, E, A] uint8.  Row d < D holds what decision d observed (and, for action, what it did); row D the trailing
+    observation.  The turn fields are what agar_get returns right after that observation.  Observation rows of skipping or
+    dead agents are not written: they keep what the tensor held (zeros in a fresh allocation).  A field that is None is not
+    recorded.  n_frames: frames per decision of the rollout that filled it (None before one has); frame_skip: the config's."""
+    __slots__ = ()
+
+    @staticmethod
+    def shapes(n_decisions, n_envs, n_agents, state_len):
+        """{field: (shape, dtype name)} of a D-decision trajectory (no device needed)"""
+        D, E, A, L = int(n_decisions), int(n_envs), max(int(n_agents), 1), int(state_len)
+        turn = ((D + 1, E, A), "uint8")
+        return {"obs": ((D + 1, E, A, L), "float32"), "action": ((D, E, A, 4), "float32"),
+                "reward": ((D + 1, E, A), "float32"), "done": turn, "valid": turn, "need_action": turn}
+
+    @classmethod
+    def allocate(cls, batch, n_decisions, fields=TRAJECTORY_FIELDS):
+        """Zeroed tensors for the named fields on the batch's device, None for the others: reusable through
+        AgarBatch.rollout(out=...), for instance inside a CUDA graph."""
+        unknown = set(fields) - set(TRAJECTORY_FIELDS)
+        if unknown:
+            raise ValueError("unknown trajectory fields %s (known: %s)" % (sorted(unknown), ", ".join(TRAJECTORY_FIELDS)))
+        torch = batch.torch
+        sh = cls.shapes(n_decisions, batch.n_envs, batch.layout.n_agents, batch.layout.state_len)
+        t = {f: torch.zeros(sh[f][0], dtype=getattr(torch, sh[f][1]), device=batch.device) if f in fields else None
+             for f in TRAJECTORY_FIELDS}
+        return cls(n_frames=None, frame_skip=int(batch.cfg.frame_skip), **t)
 
 
 _GET_DTYPES = {lay.GET_REWARD: "float32", lay.GET_DONE: "uint8", lay.GET_VALID: "uint8", lay.GET_NEED_ACTION: "uint8",
@@ -247,6 +288,34 @@ class AgarBatch(object):
         self._check(self.lib.agar_rollout_random(self.h, int(n_decisions), int(n_frames), int(decision_base),
                                                  self._ptr(out), self._stream()))
         return out
+
+    def rollout(self, n_decisions, n_frames=None, decision_base=0, actions=None, out=None):
+        """agar_rollout: n_decisions x (observe -> act -> n_frames frames) and a trailing observation in one launch, every
+        decision recorded.  actions: [D, E, A, 4] caller actions (decision d takes row d), or None for the random driver of
+        rollout_random (whose actions are then recorded).  out: a Trajectory to fill (Trajectory.allocate; None fields are not
+        recorded; out.action must be None with caller actions), or None for a new one.  Returns the Trajectory, whose
+        action is the caller's tensor when actions are given.  The records end as after rollout_random(D, n_frames,
+        decision_base) + observe."""
+        n_frames = self.cfg.frame_skip + 1 if n_frames is None else int(n_frames)
+        D = int(n_decisions)
+        act = None
+        if actions is not None:
+            act = self.torch.as_tensor(actions, dtype=self.torch.float32, device=self.device)
+            shape = (D, self.n_envs, max(self.layout.n_agents, 1), 4)
+            act = (act if tuple(act.shape) == shape else act.reshape(shape)).contiguous()
+        if out is None:
+            out = Trajectory.allocate(self, D, [f for f in TRAJECTORY_FIELDS if not (f == "action" and act is not None)])
+        sh = Trajectory.shapes(D, self.n_envs, self.layout.n_agents, self.layout.state_len)
+        for f in TRAJECTORY_FIELDS:
+            t = getattr(out, f)
+            if t is not None and not (self.torch.is_tensor(t) and tuple(t.shape) == sh[f][0] and t.device == self.device
+                                      and t.dtype == getattr(self.torch, sh[f][1]) and t.is_contiguous()):
+                raise ValueError("out.%s must be a contiguous %s tensor %s on %s" % (f, sh[f][1], sh[f][0], self.device))
+        c = _CTrajectory(*[getattr(out, f).data_ptr() if getattr(out, f) is not None else None for f in TRAJECTORY_FIELDS])
+        fn = self._lazy("agar_rollout", [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_uint32, ctypes.c_void_p,
+                                         ctypes.POINTER(_CTrajectory), ctypes.c_void_p])
+        self._check(fn(self.h, D, n_frames, int(decision_base), self._ptr(act), ctypes.byref(c), self._stream()))
+        return out._replace(action=act if act is not None else out.action, n_frames=n_frames)
 
     def get(self, which):
         per_env = which in (lay.GET_OVERFLOW, lay.GET_EVENT_HASH)

@@ -28,6 +28,20 @@ def _bind(lib):
     return lib
 
 
+def trajectory_transitions(traj):
+    """(obs_t, action, reward, obs_tp1, done, valid) of every transition in a recorded rollout (env.Trajectory): decision d's
+    observation and action, then the reward, observation, done and valid read after decision d + 1's observation -- the
+    alignment of the per-tick loops (step_observe, then add_batch).  Contiguous views, no copies.  It holds when every decision
+    is one bot turn (n_frames == frame_skip + 1); any other trajectory is refused."""
+    missing = [f for f in ("obs", "action", "reward", "done", "valid") if getattr(traj, f) is None]
+    if missing:
+        raise ValueError("add_trajectory needs the %s fields recorded" % ", ".join(missing))
+    if traj.n_frames != traj.frame_skip + 1:
+        raise ValueError("add_trajectory needs one bot turn per decision (n_frames == frame_skip + 1 == %d); this trajectory "
+                         "has n_frames = %s" % (traj.frame_skip + 1, traj.n_frames))
+    return traj.obs[:-1], traj.action, traj.reward[1:], traj.obs[1:], traj.done[1:], traj.valid[1:]
+
+
 class GpuReplayBuffer(object):
     """ReplayBuffer(size) / PrioritizedReplayBuffer(size, alpha, beta) on one GPU."""
 
@@ -101,6 +115,11 @@ class GpuReplayBuffer(object):
         valid = None if valid is None else valid.reshape(n).contiguous().to(t.uint8)
         self._check(self.lib.agar_replay_add_batch(self.h, self._p(obs_t), self._p(action), self._p(reward), self._p(obs_tp1),
                                                    self._p(done), self._p(valid), n, self._stream()))
+
+    def add_trajectory(self, traj):
+        """Every transition of a recorded rollout (AgarBatch.rollout) in one add_batch of D x E x A transitions, in
+        (decision, env, agent) order: see trajectory_transitions for the alignment and what is refused."""
+        self.add_batch(*trajectory_transitions(traj))
 
     def _outs(self, batch):
         t = self.torch

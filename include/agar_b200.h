@@ -286,6 +286,38 @@ int agar_step_observe(AgarEnv* env, const float* actions_dev, int n_frames, floa
 int agar_rollout_random(AgarEnv* env, int n_decisions, int n_frames, uint32_t decision_base, float* obs_dev,
                         void* stream);
 
+/* ---- recorded rollouts: every decision's observation, action, reward and turn flags, one launch ----
+ * Device pointers on the handle's device; each one is nullable (NULL = that field is not recorded).  D = n_decisions,
+ * E = n_envs, A = n_agents, L = state_len; arrays are row-major in the order the brackets give. */
+typedef struct AgarTrajectory {
+    float* obs;           /* [D+1][E][A][L]  row d < D: the observation handed off at decision d; row D: the trailing one  */
+    float* action;        /* [D][E][A][4]    the random driver's action of decision d (must be NULL with caller actions)   */
+    float* reward;        /* [D+1][E][A]     what agar_get(AGAR_GET_REWARD) returns right after decision d's observation */
+    uint8_t* done;        /* [D+1][E][A]     ... AGAR_GET_DONE                                                             */
+    uint8_t* valid;       /* [D+1][E][A]     ... AGAR_GET_VALID                                                            */
+    uint8_t* need_action; /* [D+1][E][A]     ... AGAR_GET_NEED_ACTION                                                      */
+} AgarTrajectory;
+
+/* n_decisions x (observe -> act -> n_frames frames), then a trailing observation, recorded into `out`.
+ *   - Launch: one kernel launch on `stream` (agar_launch_count).  It never synchronises the host and allocates nothing, so a
+ *     CUDA graph can capture it.
+ *   - Actions: actions_dev float[D][E][A][4] (decision d's actions are row d, read as agar_step reads its rows), or NULL for
+ *     the random driver of agar_rollout_random.
+ *   - End state: the env records afterwards are bit for bit those after agar_rollout_random(D, n_frames, decision_base)
+ *     followed by agar_observe; with caller actions, those after D x (agar_observe, agar_step(actions_dev row d,
+ *     n_frames)) followed by agar_observe.
+ *   - Observation rows: row (d, e, a) is written exactly when agar_observe at that moment would write it; rows of skipping
+ *     or dead agents are left untouched, as agar_observe leaves them.  reward / done / valid / need_action are written for
+ *     every (d, e, a) slot.
+ *   - Random actions: action[d][e][a] = the 4 uniforms of Philox(counter = (decision_base + d, 7, first_env_id + e, a),
+ *     key = seed) that agar_rollout_random computes, written for every slot whether or not the agent acted at decision d.
+ *   - Indices are computed in 64 bits: a trajectory may exceed 4 GiB.
+ *   - Refused with AGAR_E_INVALID (reason in agar_last_error): a NULL `out`; a negative n_decisions or n_frames; out->action
+ *     together with caller actions; an out->obs or actions_dev pointer that is not 4-byte aligned.
+ * The records are unchanged in format (AGAR_ABI_VERSION 1): snapshots and checkpoints work across the call. */
+int agar_rollout(AgarEnv* env, int n_decisions, int n_frames, uint32_t decision_base, const float* actions_dev,
+                 const AgarTrajectory* out, void* stream);
+
 int agar_get(AgarEnv* env, AgarField which, void* out_dev, void* stream);
 
 /* lanes of a warp that cooperate on one env (1, 2, 4, 8, 16, 32; multi-cell configs: 4..32).  A tuning knob:

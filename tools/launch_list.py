@@ -12,8 +12,10 @@ sides of the observer-warp wave rule, the default widths at 65 536 and 1 048 576
 at the CTA sizes of k_main<32, true, 1024 / 768> (the wave cost model keeping and shrinking the CTA), configs[2] at 4, 8 and
 16 lanes, configs[3], the G = 42 single-cell config and AGAR_GENERAL_KERNEL=1 (k_main<32, false>).  Each case creates its
 handle (k_init) and runs observe, step, step_observe and rollout_random at 1, 3, 4 and 8 frames, with and without an
-observation buffer, step_host with pinned and with pageable buffers, reset, reset_bots, snapshot and restore.  The trace
-goes to a temporary directory."""
+observation buffer, step_host with pinned and with pageable buffers, reset, reset_bots, snapshot and restore.  Then a second
+handle of each case (case name + " | agar_rollout", so that the lines above stay comparable with builds that lack the call)
+runs agar_rollout with the random driver and with caller actions at the same frame counts.  The trace goes to a temporary
+directory."""
 import json
 import os
 import re
@@ -26,7 +28,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 import aigar_b200.layout as lay  # noqa: E402
-from aigar_b200.env import AgarBatch  # noqa: E402
+from aigar_b200.env import AgarBatch, Trajectory  # noqa: E402
 
 C2 = dict(num_nn=1, num_greedy=1, virus=True, split=True, eject=True)
 C3 = dict(num_nn=8, num_greedy=8, virus=True, split=True, eject=True)
@@ -66,6 +68,13 @@ def run_ops(b):
     b.restore(b.snapshot())
 
 
+def run_rollout_ops(b):
+    for nf in FRAMES:
+        b.rollout(2, nf, 0, out=Trajectory.allocate(b, 2))
+        traj = Trajectory.allocate(b, 2, [f for f in Trajectory._fields[:6] if f != "action"])
+        b.rollout(2, nf, 0, actions=torch.zeros((2,) + tuple(b.actions.shape), device=b.device), out=traj)
+
+
 def kernel_launches(prof, tmp):
     path = os.path.join(tmp, "trace.json")
     prof.export_chrome_trace(path)
@@ -80,23 +89,24 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("launch_list.py lists GPU kernel launches: it needs a CUDA device")
     with tempfile.TemporaryDirectory() as tmp:
-        for name, kw, n, w, general in CASES:
-            if general:
-                os.environ["AGAR_GENERAL_KERNEL"] = "1"
-            try:
-                with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
-                    b = AgarBatch(lay.derive_config(**kw), n, seed=1, tile_width=w)
-                    run_ops(b)
-                    torch.cuda.synchronize()
-            finally:
-                os.environ.pop("AGAR_GENERAL_KERNEL", None)
-            for k in kernel_launches(prof, tmp):
-                print(json.dumps(dict(case=name, **k)))
-            print(json.dumps({"case": name, "tile_width": b.tile_width, "agar_launch_count": b.launch_count,
-                              "agar_observer_launch_count": b.observer_launch_count}))
-            b.close()
-            del b
-            torch.cuda.empty_cache()
+        for case, kw, n, w, general in CASES:
+            for name, ops in ((case, run_ops), (case + " | agar_rollout", run_rollout_ops)):
+                if general:
+                    os.environ["AGAR_GENERAL_KERNEL"] = "1"
+                try:
+                    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+                        b = AgarBatch(lay.derive_config(**kw), n, seed=1, tile_width=w)
+                        ops(b)
+                        torch.cuda.synchronize()
+                finally:
+                    os.environ.pop("AGAR_GENERAL_KERNEL", None)
+                for k in kernel_launches(prof, tmp):
+                    print(json.dumps(dict(case=name, **k)))
+                print(json.dumps({"case": name, "tile_width": b.tile_width, "agar_launch_count": b.launch_count,
+                                  "agar_observer_launch_count": b.observer_launch_count}))
+                b.close()
+                del b
+                torch.cuda.empty_cache()
 
 
 if __name__ == "__main__":
