@@ -19,7 +19,7 @@ struct ReplayDev {
     float *obs_t, *obs_tp1, *action, *reward;
     uint8_t* done;
     double *sum, *mn;    /* segment trees, 2 * itcap each (node 1 = root) */
-    int32_t* counters;   /* [0] next_idx  [1] size  [2] n_valid of the last add */
+    int32_t* counters;   /* [0] next_idx  [1] size  [2] n_valid of the last add  [3] error flags  [4] verdict of the last load */
     double* max_priority;
     int32_t* pos;        /* scratch: ring position per candidate of the last add (-1 = not stored) */
     int cap, itcap, L, AL, prioritized;
@@ -31,6 +31,7 @@ struct AgarReplay {
     int64_t launches;
     char err[256];
 };
+constexpr size_t RP_COUNTER_BYTES = 32; /* int32 counters[8]; [5..7] unused */
 static char g_rp_err[256] = "";
 
 static int rp_fail(AgarReplay* rp, int code, const char* msg) {
@@ -332,6 +333,174 @@ static int rp_fix_paths(AgarReplay* rp, const int32_t* idx_dev, int n, cudaStrea
     return AGAR_OK;
 }
 
+/* ---- state snapshots (agar_replay_save / agar_replay_load; bank layout in agar_replay.h) */
+constexpr int RP_SECTIONS = 6; /* obs_t, obs_tp1, action, reward, done, leaf */
+constexpr int RP_LEAF = 5;
+struct RpStateLayout {
+    int64_t off[RP_SECTIONS + 1]; /* section s spans bytes [off[s], off[s + 1]) of the bank; off[RP_SECTIONS] = bank bytes */
+    int64_t row[RP_SECTIONS];     /* bytes per ring slot (0 for the leaves of a uniform buffer: an empty section) */
+};
+static RpStateLayout rp_state_layout(const ReplayDev& d) {
+    const int64_t row[RP_SECTIONS] = {4ll * d.L, 4ll * d.L, 4ll * d.AL, 4, 1, d.prioritized ? 8 : 0};
+    RpStateLayout s;
+    int64_t at = 256; /* the header */
+    for (int i = 0; i < RP_SECTIONS; ++i) {
+        s.row[i] = row[i];
+        s.off[i] = at;
+        at = (at + (int64_t)d.cap * row[i] + 255) & ~(int64_t)255;
+    }
+    s.off[RP_SECTIONS] = at;
+    return s;
+}
+__device__ uint8_t* rp_ring(const ReplayDev& d, int s) {
+    return s == 0 ? (uint8_t*)d.obs_t : s == 1 ? (uint8_t*)d.obs_tp1 : s == 2 ? (uint8_t*)d.action : s == 3 ? (uint8_t*)d.reward : d.done;
+}
+union RpWord {
+    uint4 v;
+    uint8_t b[16];
+};
+/* 16-byte word i of a ring allocation whose first `live` bytes are live; bytes past `live` read as zero (and are not read:
+ * the allocation need not extend to a whole word) */
+__device__ uint4 rp_fetch(const uint8_t* a, int64_t i, int64_t live) {
+    const int64_t o = i * 16;
+    if (o + 16 <= live) return *(const uint4*)(a + o);
+    RpWord w;
+    w.v = make_uint4(0, 0, 0, 0);
+    for (int k = 0; o + k < live; ++k) w.b[k] = a[o + k];
+    return w.v;
+}
+__device__ void rp_put(uint8_t* a, int64_t i, int64_t live, uint4 v) {
+    const int64_t o = i * 16;
+    if (o + 16 <= live) {
+        *(uint4*)(a + o) = v;
+        return;
+    }
+    RpWord w;
+    w.v = v;
+    for (int k = 0; o + k < live; ++k) a[o + k] = w.b[k];
+}
+__device__ bool rp_leaf_bad(double v, int64_t k, int64_t size) {
+    return k >= size ? __double_as_longlong(v) != 0 : !(v >= 0.0); /* +0.0 past size; below it neither NaN nor negative */
+}
+/* Load, step 1: the verdict (counters[4], zeroed by the host's memset) is set when the bank fails any check listed at
+ * agar_replay_load.  Thread 0 checks the header, the grid the leaves. */
+__global__ void __launch_bounds__(256) k_rp_validate(ReplayDev d, RpStateLayout s, const uint8_t* __restrict__ bank) {
+    const AgarReplayStateHeader* h = (const AgarReplayStateHeader*)bank;
+    const int64_t size = h->size;
+    bool bad = false;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        const double mp = h->max_priority;
+        bad = h->capacity != d.cap || h->state_len != d.L || h->action_len != d.AL || h->prioritized != (d.prioritized != 0) ||
+              h->alpha_bits != (uint64_t)__double_as_longlong(d.alpha) || h->beta_bits != (uint64_t)__double_as_longlong(d.beta) ||
+              h->next_idx < 0 || h->next_idx >= d.cap || size < 0 || size > d.cap || (size < d.cap && h->next_idx != size) ||
+              !(mp >= 1.0 && mp <= 1.7e308);
+    }
+    if (d.prioritized) {
+        const double2* leaf = (const double2*)(bank + s.off[RP_LEAF]);
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; 2 * i < d.cap; i += (int64_t)gridDim.x * blockDim.x) {
+            const double2 v = leaf[i];
+            bad |= rp_leaf_bad(v.x, 2 * i, size) || (2 * i + 1 < d.cap && rp_leaf_bad(v.y, 2 * i + 1, size));
+        }
+    }
+    if (bad) {
+        d.counters[4] = 1;
+        atomicOr(&d.counters[3], AGAR_RP_ERR_STATE);
+    }
+}
+/* Save (load = 0): bank <- buffer, zeros for ring rows and leaves at index >= size and for padding.  Load, step 2: buffer <-
+ * bank if the verdict is good, ring rows below the bank's size and every leaf (sum / min: the leaf below size, 0 / +inf at
+ * and above it).  blockIdx.y is the section; the grid strides over its 16-byte words with RP_COPY_U loads in flight. */
+constexpr int RP_COPY_U = 4;
+__global__ void __launch_bounds__(256) k_rp_state(ReplayDev d, RpStateLayout s, uint8_t* bank, int load) {
+    if (load && d.counters[4] != 0) return;
+    const AgarReplayStateHeader* hb = (const AgarReplayStateHeader*)bank;
+    const int64_t size = load ? hb->size : d.counters[1];
+    const int sec = blockIdx.y;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x, t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t nw = (s.off[sec + 1] - s.off[sec]) / 16;
+    uint4* b = (uint4*)(bank + s.off[sec]);
+    if (sec == 0 && t0 == 0) {
+        if (load) {
+            d.counters[0] = (int32_t)hb->next_idx;
+            d.counters[1] = (int32_t)size;
+            *d.max_priority = hb->max_priority;
+        } else {
+            union {
+                AgarReplayStateHeader h;
+                uint4 w[16];
+            } u;
+            for (int k = 0; k < 16; ++k) u.w[k] = make_uint4(0, 0, 0, 0);
+            u.h.capacity = d.cap, u.h.state_len = d.L, u.h.action_len = d.AL, u.h.prioritized = d.prioritized != 0;
+            u.h.alpha_bits = (uint64_t)__double_as_longlong(d.alpha), u.h.beta_bits = (uint64_t)__double_as_longlong(d.beta);
+            u.h.next_idx = d.counters[0], u.h.size = size, u.h.max_priority = *d.max_priority;
+            for (int k = 0; k < 16; ++k) ((uint4*)bank)[k] = u.w[k];
+        }
+    }
+    if (sec == RP_LEAF) {
+        double2* leaf = (double2*)b;
+        for (int64_t i = t0; i < nw; i += stride) {
+            const int64_t k = 2 * i;
+            if (load) {
+                const double2 v = leaf[i];
+                if (k < d.cap) d.sum[d.itcap + k] = k < size ? v.x : 0.0, d.mn[d.itcap + k] = k < size ? v.x : INFINITY;
+                if (k + 1 < d.cap) d.sum[d.itcap + k + 1] = k + 1 < size ? v.y : 0.0, d.mn[d.itcap + k + 1] = k + 1 < size ? v.y : INFINITY;
+            } else {
+                leaf[i] = make_double2(k < size ? d.sum[d.itcap + k] : 0.0, k + 1 < size ? d.sum[d.itcap + k + 1] : 0.0);
+            }
+        }
+        return;
+    }
+    uint8_t* a = rp_ring(d, sec);
+    const int64_t live = size * s.row[sec];
+    for (int64_t base = t0; base < nw; base += RP_COPY_U * stride) {
+        uint4 v[RP_COPY_U];
+#pragma unroll
+        for (int u = 0; u < RP_COPY_U; ++u) {
+            const int64_t i = base + u * stride;
+            if (i < nw) v[u] = load ? b[i] : rp_fetch(a, i, live);
+        }
+#pragma unroll
+        for (int u = 0; u < RP_COPY_U; ++u) {
+            const int64_t i = base + u * stride;
+            if (i < nw) {
+                if (load)
+                    rp_put(a, i, live, v[u]);
+                else
+                    b[i] = v[u];
+            }
+        }
+    }
+}
+
+/* Load, step 3: both trees from their leaves, RP_REBUILD_LEVELS levels per launch.  CTA b owns the subtree above nodes
+ * [first + b 2^RP_REBUILD_LEVELS, first + (b + 1) 2^RP_REBUILD_LEVELS) of the starting level, with a barrier between levels: 2
+ * launches for 2^20 slots where the per-level kernel k_rp_level takes 20, whose launch gaps made a restore of a 1 GB bank 15 %
+ * slower (DESIGN §9).  Same op as k_rp_level per node, so the same nodes bit for bit. */
+constexpr int RP_REBUILD_LEVELS = 11;
+__global__ void __launch_bounds__(1024) k_rp_rebuild(ReplayDev d, int first, int levels) {
+    for (int lv = 1; lv <= levels; ++lv) {
+        const int width = first >> lv, per = (1 << RP_REBUILD_LEVELS) >> lv;
+        for (int i = threadIdx.x; i < per && blockIdx.x * per + i < width; i += blockDim.x) {
+            const int node = width + blockIdx.x * per + i;
+            d.sum[node] = d.sum[2 * node] + d.sum[2 * node + 1];
+            const double a = d.mn[2 * node], b = d.mn[2 * node + 1];
+            d.mn[node] = b < a ? b : a;
+        }
+        __syncthreads();
+    }
+}
+static int rp_rebuild(AgarReplay* rp, cudaStream_t s) {
+    for (int first = rp->d.itcap; first > 1;) {
+        int levels = 0;
+        while (levels < RP_REBUILD_LEVELS && (first >> levels) > 1) ++levels;
+        k_rp_rebuild<<<first > (1 << RP_REBUILD_LEVELS) ? first >> RP_REBUILD_LEVELS : 1, 1024, 0, s>>>(rp->d, first, levels);
+        rp->launches += 1;
+        first >>= levels;
+    }
+    RCU(cudaGetLastError());
+    return AGAR_OK;
+}
+
 extern "C" int agar_replay_create(int capacity, int state_len, int action_len, int prioritized, double alpha, double beta,
                                   int device, AgarReplay** out) {
     AgarReplay* rp = nullptr;
@@ -348,7 +517,7 @@ extern "C" int agar_replay_create(int capacity, int state_len, int action_len, i
     if (cudaMalloc(&d.obs_t, cap * state_len * 4) != cudaSuccess || cudaMalloc(&d.obs_tp1, cap * state_len * 4) != cudaSuccess ||
         cudaMalloc(&d.action, cap * action_len * 4) != cudaSuccess || cudaMalloc(&d.reward, cap * 4) != cudaSuccess ||
         cudaMalloc(&d.done, cap) != cudaSuccess || cudaMalloc(&d.sum, (size_t)2 * d.itcap * 8) != cudaSuccess ||
-        cudaMalloc(&d.mn, (size_t)2 * d.itcap * 8) != cudaSuccess || cudaMalloc(&d.counters, 16) != cudaSuccess ||
+        cudaMalloc(&d.mn, (size_t)2 * d.itcap * 8) != cudaSuccess || cudaMalloc(&d.counters, RP_COUNTER_BYTES) != cudaSuccess ||
         cudaMalloc(&d.max_priority, 8) != cudaSuccess) {
         cudaGetLastError();
         free(rp);
@@ -448,4 +617,65 @@ extern "C" int agar_replay_update_priorities(AgarReplay* rp, const int32_t* idx_
     RCU(cudaGetLastError());
     rp->launches += 2;
     return rp_fix_paths(rp, idx_dev, batch, s);
+}
+
+extern "C" int64_t agar_replay_state_bytes(const AgarReplay* rp) { return rp ? rp_state_layout(rp->d).off[RP_SECTIONS] : AGAR_E_INVALID; }
+/* a bank must be 16-byte aligned (the copy moves 16-byte words) and must not overlap any allocation of the buffer */
+static int rp_bank_check(AgarReplay* rp, const void* bank, const char* what) {
+    char msg[160];
+    const ReplayDev& d = rp->d;
+    const char* why = nullptr;
+    const uintptr_t b0 = (uintptr_t)bank, b1 = b0 + (uintptr_t)rp_state_layout(d).off[RP_SECTIONS];
+    const size_t cap = (size_t)d.cap;
+    const struct {
+        const void* p;
+        size_t n;
+    } own[] = {{d.obs_t, cap * d.L * 4},         {d.obs_tp1, cap * d.L * 4},         {d.action, cap * d.AL * 4},
+               {d.reward, cap * 4},              {d.done, cap},                      {d.sum, (size_t)2 * d.itcap * 8},
+               {d.mn, (size_t)2 * d.itcap * 8}, {d.counters, RP_COUNTER_BYTES},   {d.max_priority, 8},
+               {d.pos, (size_t)rp->pos_cap * 4}};
+    if (!bank)
+        why = "bank is NULL";
+    else if (b0 % 16)
+        why = "bank is not 16-byte aligned";
+    for (const auto& o : own)
+        if (!why && o.p && b0 < (uintptr_t)o.p + o.n && (uintptr_t)o.p < b1) why = "bank overlaps the buffer's own allocations";
+    if (!why) return AGAR_OK;
+    snprintf(msg, sizeof msg, "%s: %s", what, why);
+    return rp_fail(rp, AGAR_E_INVALID, msg);
+}
+static dim3 rp_state_grid(const RpStateLayout& s) {
+    int64_t most = 0;
+    for (int i = 0; i < RP_SECTIONS; ++i) most = s.off[i + 1] - s.off[i] > most ? s.off[i + 1] - s.off[i] : most;
+    const int64_t blocks = (most / 16 + 256 * RP_COPY_U - 1) / (256 * RP_COPY_U);
+    return dim3((unsigned)(blocks < 1 ? 1 : blocks > 1024 ? 1024 : blocks), RP_SECTIONS);
+}
+extern "C" int agar_replay_save(AgarReplay* rp, void* bank_dev, void* stream) {
+    if (!rp) return AGAR_E_INVALID;
+    const int rc = rp_bank_check(rp, bank_dev, "agar_replay_save");
+    if (rc != AGAR_OK) return rc;
+    RCU(cudaSetDevice(rp->device));
+    const RpStateLayout s = rp_state_layout(rp->d);
+    k_rp_state<<<rp_state_grid(s), 256, 0, (cudaStream_t)stream>>>(rp->d, s, (uint8_t*)bank_dev, 0);
+    RCU(cudaGetLastError());
+    rp->launches += 1;
+    return AGAR_OK;
+}
+/* validate, then install (a refused bank installs nothing), then rebuild the trees from their leaves: a rebuild after a refusal
+ * recomputes the same nodes from the same leaves, so the buffer stays as it was without a host synchronisation */
+extern "C" int agar_replay_load(AgarReplay* rp, const void* bank_dev, void* stream) {
+    if (!rp) return AGAR_E_INVALID;
+    const int rc = rp_bank_check(rp, bank_dev, "agar_replay_load");
+    if (rc != AGAR_OK) return rc;
+    RCU(cudaSetDevice(rp->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const RpStateLayout lay = rp_state_layout(rp->d);
+    const int64_t pairs = rp->d.prioritized ? ((int64_t)rp->d.cap + 1) / 2 : 1;
+    const int vblocks = (int)((pairs + 255) / 256 > 1024 ? 1024 : (pairs + 255) / 256);
+    RCU(cudaMemsetAsync(rp->d.counters + 4, 0, 4, s));
+    k_rp_validate<<<vblocks, 256, 0, s>>>(rp->d, lay, (const uint8_t*)bank_dev);
+    k_rp_state<<<rp_state_grid(lay), 256, 0, s>>>(rp->d, lay, (uint8_t*)bank_dev, 1);
+    RCU(cudaGetLastError());
+    rp->launches += 2;
+    return rp->d.prioritized ? rp_rebuild(rp, s) : AGAR_OK;
 }

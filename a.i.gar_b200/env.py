@@ -64,6 +64,13 @@ def load_library():
     return lib
 
 
+def bind_lazy(lib, name, argtypes, restype=ctypes.c_int):
+    """A C function bound on first use (not in EXPORTS: older builds load for A/B runs)."""
+    fn = getattr(lib, name)
+    fn.argtypes, fn.restype = argtypes, restype
+    return fn
+
+
 class AgarError(RuntimeError):
     pass
 
@@ -80,26 +87,44 @@ def _struct_bytes(s):
     return np.frombuffer(bytes(s), dtype=np.uint8).copy()
 
 
+def save_npz_checkpoint(path, fmt, payload, **fields):
+    """Write a checkpoint .npz (no pickled objects): a format tag, the fields, and `payload` (a uint8 host array, stored under
+    that name) with its SHA-256."""
+    arr = np.ascontiguousarray(fields[payload], dtype=np.uint8)
+    fields[payload] = arr
+    with open(path, "wb") as f:  # a file object: numpy would otherwise append ".npz" to the name
+        np.savez(f, format=np.array(fmt), sha256=np.array(hashlib.sha256(arr.tobytes()).hexdigest()), **fields)
+
+
+def load_npz_checkpoint(path, fmt, keys, kind):
+    """The fields `keys` of a checkpoint .npz, read without pickles.  Raises CheckpointError for a file that lacks one of
+    them (naming it a `kind` checkpoint) or has another format tag."""
+    with np.load(path, allow_pickle=False) as z:
+        missing = [k for k in keys if k not in z.files]
+        if missing:
+            raise CheckpointError("%s: not a %s checkpoint (missing %s)" % (path, kind, ", ".join(missing)))
+        ck = {k: z[k] for k in keys}
+    if str(ck["format"]) != fmt:
+        raise CheckpointError("%s: format %r, expected %r" % (path, str(ck["format"]), fmt))
+    return ck
+
+
+def check_npz_digest(path, ck, payload):
+    if hashlib.sha256(np.ascontiguousarray(ck[payload]).tobytes()).hexdigest() != str(ck["sha256"]):
+        raise CheckpointError("%s: sha256 of the %s does not match the stored digest" % (path, payload))
+
+
 def write_checkpoint(path, cfg, layout, n_envs, seed, first_env_id, records):
     """Write a batch checkpoint (.npz, no pickled objects).  records: uint8 [n_envs, record_bytes] host array."""
-    records = np.ascontiguousarray(records, dtype=np.uint8)
-    with open(path, "wb") as f:  # a file object: numpy would otherwise append ".npz" to the name
-        np.savez(f, format=np.array(CHECKPOINT_FORMAT), abi_version=np.int64(lay.ABI_VERSION),
-                 config=_struct_bytes(cfg), layout=_struct_bytes(layout), n_envs=np.int64(n_envs),
-                 seed=np.uint64(seed), first_env_id=np.uint64(first_env_id), records=records,
-                 sha256=np.array(hashlib.sha256(records.tobytes()).hexdigest()))
+    save_npz_checkpoint(path, CHECKPOINT_FORMAT, "records", abi_version=np.int64(lay.ABI_VERSION),
+                        config=_struct_bytes(cfg), layout=_struct_bytes(layout), n_envs=np.int64(n_envs),
+                        seed=np.uint64(seed), first_env_id=np.uint64(first_env_id), records=records)
 
 
 def read_checkpoint(path):
     """Parse a checkpoint file without a device: a dict of its fields.  Raises CheckpointError for a file that is not a
     checkpoint of this format and ABI version, whose records are not [n_envs, record_bytes] uint8, or whose digest differs."""
-    with np.load(path, allow_pickle=False) as z:
-        missing = [k for k in _CHECKPOINT_KEYS if k not in z.files]
-        if missing:
-            raise CheckpointError("%s: not a records checkpoint (missing %s)" % (path, ", ".join(missing)))
-        ck = {k: z[k] for k in _CHECKPOINT_KEYS}
-    if str(ck["format"]) != CHECKPOINT_FORMAT:
-        raise CheckpointError("%s: format %r, expected %r" % (path, str(ck["format"]), CHECKPOINT_FORMAT))
+    ck = load_npz_checkpoint(path, CHECKPOINT_FORMAT, _CHECKPOINT_KEYS, "records")
     if int(ck["abi_version"]) != lay.ABI_VERSION:
         raise CheckpointError("%s: abi_version %d, this library has %d" % (path, int(ck["abi_version"]), lay.ABI_VERSION))
     for name, struct in (("config", lay.AgarConfig), ("layout", lay.AgarLayout)):
@@ -109,8 +134,7 @@ def read_checkpoint(path):
     if rec.dtype != np.uint8 or rec.ndim != 2 or rec.shape != (int(ck["n_envs"]), rb):
         raise CheckpointError("%s: records of shape %s / %s do not match n_envs and the layout's record_bytes"
                               % (path, rec.shape, rec.dtype))
-    if hashlib.sha256(np.ascontiguousarray(rec).tobytes()).hexdigest() != str(ck["sha256"]):
-        raise CheckpointError("%s: sha256 of the records does not match the stored digest" % path)
+    check_npz_digest(path, ck, "records")
     return ck
 
 
@@ -241,10 +265,7 @@ class AgarBatch(object):
         return int(fn(self.h))
 
     def _lazy(self, name, argtypes, restype=ctypes.c_int):
-        """A C function bound on first use (not in EXPORTS: older builds load for A/B runs)."""
-        fn = getattr(self.lib, name)
-        fn.argtypes, fn.restype = argtypes, restype
-        return fn
+        return bind_lazy(self.lib, name, argtypes, restype)
 
     def _ptr(self, t):
         return ctypes.c_void_p(t.data_ptr()) if t is not None else ctypes.c_void_p()

@@ -3,7 +3,47 @@ ReplayBuffer / PrioritizedReplayBuffer for batches of transitions that stay on t
 (uniforms in [0, 1)) exactly where the reference calls random.randint / random.random."""
 import ctypes
 
+import numpy as np
+
 from . import env as _env
+
+CheckpointError = _env.CheckpointError
+ERR_STATE = 8  # AGAR_RP_ERR_STATE: a bank refused by agar_replay_load
+
+REPLAY_CHECKPOINT_FORMAT = "agar_b200.replay.v1"
+_REPLAY_KEYS = ("format", "capacity", "state_len", "action_len", "prioritized", "alpha", "beta", "bank", "sha256")
+
+
+def write_replay_checkpoint(path, capacity, state_len, action_len, prioritized, alpha, beta, bank):
+    """Write a replay-buffer checkpoint (.npz, no pickled objects).  bank: the uint8 host bytes of agar_replay_save."""
+    _env.save_npz_checkpoint(path, REPLAY_CHECKPOINT_FORMAT, "bank", capacity=np.int64(capacity), state_len=np.int64(state_len),
+                             action_len=np.int64(action_len), prioritized=np.bool_(prioritized), alpha=np.float64(alpha),
+                             beta=np.float64(beta), bank=np.ravel(bank))
+
+
+def read_replay_checkpoint(path):
+    """Parse a replay checkpoint without a device: a dict of its fields.  Raises CheckpointError for a file that is not one of
+    this format, whose bank is not 1-D uint8, or whose digest differs."""
+    ck = _env.load_npz_checkpoint(path, REPLAY_CHECKPOINT_FORMAT, _REPLAY_KEYS, "replay")
+    if ck["bank"].dtype != np.uint8 or ck["bank"].ndim != 1:
+        raise CheckpointError("%s: bank of shape %s / %s is not 1-D uint8" % (path, ck["bank"].shape, ck["bank"].dtype))
+    _env.check_npz_digest(path, ck, "bank")
+    return ck
+
+
+def check_replay_checkpoint(ck, capacity, state_len, action_len, prioritized, alpha, beta, state_bytes):
+    """Raise CheckpointError naming the first field of a parsed replay checkpoint that differs from a buffer's
+    (state_bytes: the buffer's bank size)."""
+    for name, mine in (("capacity", capacity), ("state_len", state_len), ("action_len", action_len)):
+        if int(ck[name]) != int(mine):
+            raise CheckpointError("checkpoint %s is %d, the buffer's is %d" % (name, int(ck[name]), int(mine)))
+    if bool(ck["prioritized"]) != bool(prioritized):
+        raise CheckpointError("checkpoint prioritized is %s, the buffer's is %s" % (bool(ck["prioritized"]), bool(prioritized)))
+    for name, mine in (("alpha", alpha), ("beta", beta)):  # compared bit for bit, as the device compares them
+        if np.float64(ck[name]).tobytes() != np.float64(mine).tobytes():
+            raise CheckpointError("checkpoint %s is %r, the buffer's is %r" % (name, float(ck[name]), float(mine)))
+    if ck["bank"].size != int(state_bytes):
+        raise CheckpointError("checkpoint bank has %d bytes, the buffer's has %d" % (ck["bank"].size, int(state_bytes)))
 
 
 def _bind(lib):
@@ -53,6 +93,7 @@ class GpuReplayBuffer(object):
         self.lib = _bind(_env.load_library())
         self.device = torch.device("cuda", device)
         self.size_max, self.state_len, self.action_len, self.prioritized = size, state_len, action_len, bool(prioritized)
+        self.alpha, self.beta = float(alpha), float(beta)
         self.h = ctypes.c_void_p()
         rc = self.lib.agar_replay_create(size, state_len, action_len, int(prioritized), alpha, beta, self.device.index,
                                          ctypes.byref(self.h))
@@ -89,7 +130,8 @@ class GpuReplayBuffer(object):
 
     @property
     def error_flags(self):
-        """Sticky AGAR_RP_ERR_* bits (1 sampled a too-small buffer, 2 index out of range, 4 priority <= 0)."""
+        """Sticky AGAR_RP_ERR_* bits (1 sampled a too-small buffer, 2 index out of range, 4 priority <= 0, 8 a state bank
+        refused on restore)."""
         return int(self.lib.agar_replay_error_flags(self.h, self._stream()))
 
     def raise_on_error(self):
@@ -97,7 +139,7 @@ class GpuReplayBuffer(object):
         f = self.error_flags
         if f:
             raise _env.AgarError("replay buffer error flags %d (1 = sampled from a buffer that is too small, 2 = index out of "
-                                 "range, 4 = priority <= 0)" % f)
+                                 "range, 4 = priority <= 0, 8 = a state bank refused on restore)" % f)
 
     @property
     def launch_count(self):
@@ -156,3 +198,62 @@ class GpuReplayBuffer(object):
         idx = t.as_tensor(idx, device=self.device).to(t.int32).contiguous()
         pr = t.as_tensor(priorities, dtype=t.float64, device=self.device).contiguous()
         self._check(self.lib.agar_replay_update_priorities(self.h, self._p(idx), self._p(pr), int(idx.numel()), self._stream()))
+
+    # ---- state snapshots (agar_replay_save / agar_replay_load; bank layout in include/agar_replay.h)
+    @property
+    def state_bytes(self):
+        """bytes of one bank of this buffer"""
+        n = _env.bind_lazy(self.lib, "agar_replay_state_bytes", [ctypes.c_void_p], ctypes.c_int64)(self.h)
+        if n < 0:
+            self._check(int(n))
+        return int(n)
+
+    def _bank(self, bank):
+        t = self.torch
+        n = self.state_bytes
+        if not (t.is_tensor(bank) and bank.dtype == t.uint8 and bank.device == self.device and bank.dim() == 1 and
+                bank.numel() == n and bank.is_contiguous()):
+            raise ValueError("a replay bank is a contiguous 1-D uint8 tensor of %d bytes on %s" % (n, self.device))
+        return bank
+
+    def snapshot(self, out=None):
+        """The buffer's whole state (ring, next index, size, max priority, tree leaves) as a 1-D uint8 device tensor of
+        state_bytes.  Canonical: two buffers with the same observable state give equal banks.  out: a bank to reuse."""
+        out = self._bank(self.torch.empty(self.state_bytes, dtype=self.torch.uint8, device=self.device) if out is None else out)
+        fn = _env.bind_lazy(self.lib, "agar_replay_save", [ctypes.c_void_p] * 3)
+        self._check(fn(self.h, self._p(out), self._stream()))
+        return out
+
+    def restore(self, bank):
+        """Install a bank of a buffer created with the same size, state_len, action_len, prioritized, alpha and beta; a clone is
+        other.restore(buf.snapshot()).  The device checks the bank first: a refused one leaves this buffer unchanged and sets
+        error flag 8.  No host synchronisation: a CUDA graph can capture it."""
+        fn = _env.bind_lazy(self.lib, "agar_replay_load", [ctypes.c_void_p] * 3)
+        self._check(fn(self.h, self._p(self._bank(bank)), self._stream()))
+
+    def _fields(self):
+        return (self.size_max, self.state_len, self.action_len, self.prioritized, self.alpha, self.beta)
+
+    def save_checkpoint(self, path):
+        """Write the buffer's bank with what a later load must match (size, state_len, action_len, prioritized, alpha, beta)."""
+        write_replay_checkpoint(path, *self._fields(), bank=self.snapshot().cpu().numpy())
+
+    def load_checkpoint(self, path):
+        """Restore from a checkpoint of a buffer with the same parameters.  A file that differs in one of them, whose digest
+        is wrong or whose bank the device refuses raises CheckpointError and leaves the buffer as it was."""
+        ck = read_replay_checkpoint(path)
+        check_replay_checkpoint(ck, *self._fields(), state_bytes=self.state_bytes)
+        bank = self.torch.from_numpy(ck["bank"]).to(self.device)
+        self.restore(bank)
+        # banks are canonical, so an installed bank saves back unchanged; the sticky flag may have been set earlier
+        if not self.torch.equal(self.snapshot(), bank):
+            raise CheckpointError("%s: a bank that fails the device-side checks; nothing was loaded" % path)
+
+    @classmethod
+    def from_checkpoint(cls, path, device=0):
+        """A new buffer with a checkpoint's parameters, loaded from it."""
+        ck = read_replay_checkpoint(path)
+        rp = cls(int(ck["capacity"]), int(ck["state_len"]), int(ck["action_len"]), bool(ck["prioritized"]), float(ck["alpha"]),
+                 float(ck["beta"]), device=device)
+        rp.load_checkpoint(path)
+        return rp

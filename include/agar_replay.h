@@ -51,11 +51,58 @@ int agar_replay_update_priorities(AgarReplay* rp, const int32_t* idx_dev, const 
 /* Sticky error bits raised ON THE DEVICE since create (synchronises `stream`).  Where the reference raises — sampling an empty
  * buffer (random.randint(0, -1), replay_buffer.py:66; the prioritized path recurses without end for len < 2, :116) — or asserts
  * (0 <= idx < len(storage), priority > 0, :203-204), the kernels skip the offending element (index 0 / weight 0 is returned,
- * trees are left untouched) and set a bit here instead of hanging or corrupting memory. */
-enum { AGAR_RP_ERR_EMPTY = 1, AGAR_RP_ERR_INDEX = 2, AGAR_RP_ERR_PRIORITY = 4 };
+ * trees are left untouched) and set a bit here instead of hanging or corrupting memory.  AGAR_RP_ERR_STATE: a bank refused by
+ * agar_replay_load (below). */
+enum { AGAR_RP_ERR_EMPTY = 1, AGAR_RP_ERR_INDEX = 2, AGAR_RP_ERR_PRIORITY = 4, AGAR_RP_ERR_STATE = 8 };
 int agar_replay_error_flags(AgarReplay* rp, void* stream);
 /* number of kernels launched so far */
 int64_t agar_replay_launch_count(const AgarReplay* rp);
+
+/* ---- state snapshots: the whole observable state of a buffer in one caller-owned device bank (checkpoint, resume, clone).
+ *
+ * Bank layout (every offset 64-bit; each section starts on a 256-byte boundary, the bank is padded to one):
+ *   [0, 256)   AgarReplayStateHeader below, zero-padded
+ *   obs_t      float [cap][state_len]
+ *   obs_tp1    float [cap][state_len]
+ *   action     float [cap][action_len]
+ *   reward     float [cap]
+ *   done       uint8 [cap]
+ *   leaf       double [cap]   prioritized buffers only: the common leaf of the sum and min trees
+ * The trees' internal nodes are not stored: a node is op(left child, right child), so a load installs the leaves and
+ * rebuilds both trees.  Below `size` the sum and min leaves are equal; at and above it they are 0 and +inf.
+ *
+ * Banks are canonical: a save writes zeros for every ring row and leaf at index >= size and for all padding, so two buffers
+ * with the same observable state give byte-identical banks.
+ *
+ * Not state, and left as they are by a load: the sticky error flags, the n_valid of the last add and the add scratch.
+ * A load copies into the buffer's existing allocations, so a CUDA graph that captured this buffer's kernels sees the restored
+ * contents on its next replay. */
+typedef struct AgarReplayStateHeader {
+    int64_t capacity, state_len, action_len, prioritized; /* prioritized: 0 or 1 */
+    uint64_t alpha_bits, beta_bits;                       /* the float64 bits of alpha and beta */
+    int64_t next_idx, size;
+    double max_priority;
+} AgarReplayStateHeader;
+
+/* bytes of one bank of this buffer (< 0: an AGAR_E_* code) */
+int64_t agar_replay_state_bytes(const AgarReplay* rp);
+/* Write the buffer's state into bank_dev (agar_replay_state_bytes bytes, 16-byte aligned, on the buffer's device, not
+ * overlapping any of its allocations).  One kernel launch on `stream`; no host synchronisation, no allocation. */
+int agar_replay_save(AgarReplay* rp, void* bank_dev, void* stream);
+/* Install a bank written by agar_replay_save of a buffer created with the same capacity, state_len, action_len, prioritized,
+ * alpha and beta.  Enqueued on `stream` without host synchronisation or allocation: a 4-byte memset of the verdict word, a
+ * validation kernel, an install kernel that copies only if the verdict is good, and for prioritized buffers the rebuild of
+ * both trees from their leaves, 11 tree levels per launch: ceil(log2(capacity rounded up to a power of two) / 11) launches
+ * (1 up to 2048 slots, 2 up to 4M).  So 2 launches, plus the rebuild's.
+ *
+ * The device refuses the bank, sets AGAR_RP_ERR_STATE and leaves the buffer unchanged bit for bit when: a header shape field
+ * (capacity, state_len, action_len, prioritized, alpha or beta bits) differs from the buffer's; next_idx is outside [0, cap)
+ * or size outside [0, cap]; size < cap and next_idx != size; max_priority is NaN or outside [1, 1.7e308]; or, for a
+ * prioritized buffer, a leaf at index >= size is not +0.0 or a leaf below size is NaN or negative (0 and +inf are reachable
+ * leaves below size: agar_pow underflows and overflows for alpha >= 1).
+ * The host refuses (AGAR_E_INVALID) a NULL bank, a bank that is not 16-byte aligned or one that overlaps the buffer's own
+ * allocations; agar_replay_save does the same. */
+int agar_replay_load(AgarReplay* rp, const void* bank_dev, void* stream);
 
 #ifdef __cplusplus
 }
